@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- SIPP native prover benchmark (BASELINE.json metric: pairings aggregated per second at n = 2^k).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--n PAIRS] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--n PAIRS] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one complete `sipp_prove_native` of n random BN254 pairs (seeded synthetic inputs): Z, then log2(n)
 rounds of (Z_L, Z_R multi-pairings, Poseidon challenge, G1/G2 folds).  N = 1 runs BASELINE configs[1]
@@ -17,6 +17,15 @@ rounds of (Z_L, Z_R multi-pairings, Poseidon challenge, G1/G2 folds).  N = 1 run
 
 `--impl reference` times the CPU restatement of the reference prover (oracle/, faithful structure: one full
 pairing per pair) with all host threads on the same config.
+
+`--dump-outputs DIR` writes the proofs of the last timed step as DIR/<name>.npy, so that two builds can be compared
+output for output (the inputs are seeded: the same arguments give the same inputs).  Each proof element is an Fq12 of
+12 coefficients of 8 little-endian u32 limbs, stored as float64 limb values (exact):
+  proof.npy                  [2 log2(n) + 1, 12, 8]  the headline proof (seed 2; `--impl reference`: of the pairs it times)
+  proof_n2p16.npy, ...       the BASELINE large configurations of the default line, when they run
+  batch_proofs.npy           [instances, 2 log2(n) + 1, 12, 8]  batched instances (--workload batch, or the default
+  batch_instances.npy        line's config-5 step) and their instance indices; beyond 64 MB in all, a fixed seeded
+                             sample of the instances
 """
 import argparse
 import json
@@ -133,8 +142,10 @@ def run_reference(args):
         times = []
         for _ in range(args.steps):
             t0 = time.perf_counter()
-            o.sipp_prove(A, B, o.FAITHFUL, cores)
+            proof = o.sipp_prove(A, B, o.FAITHFUL, cores)
             times.append(time.perf_counter() - t0)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {}, (proof, len(proof) // 384, 0))
         per_step = sum(times) / len(times)
         value = 1.0 / per_step
         print(json.dumps({"impl": "reference", "metric": "SIPP native prove throughput, batched independent instances (instances per second)",
@@ -159,8 +170,10 @@ def run_reference(args):
     times = []
     for _ in range(args.steps):
         t0 = time.perf_counter()
-        o.sipp_prove(As, Bs, o.FAITHFUL, cores)
+        proof = o.sipp_prove(As, Bs, o.FAITHFUL, cores)
         times.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"proof": proof})
     per_step = sum(times) / len(times)
     value = sample_n / per_step
     t0 = time.perf_counter()
@@ -252,7 +265,7 @@ def measure_batch(count_total, n, world, rank, local_rank, W, K, barrier, all_ma
         a, b = A[64 * n * j:64 * n * (j + 1)], B[128 * n * j:128 * n * (j + 1)]
         assert proofs[j * plen * 384:(j + 1) * plen * 384] == b"".join(sipp_b200.sipp_prove_native(a, b)), "batch instance %d differs" % j
     return {"count": count, "t_res": t_res, "t_e2e": t_e2e, "stats": st, "h2d": total * 192, "d2h": count * plen * 384,
-            "sample": (A[:64 * n], B[:128 * n], proofs[:plen * 384])}
+            "sample": (A[:64 * n], B[:128 * n], proofs[:plen * 384]), "proofs": (proofs, plen, lo)}
 
 
 def run_batch(args, world, rank, local_rank, W, K):
@@ -294,6 +307,8 @@ def run_batch(args, world, rank, local_rank, W, K):
         if world > 1:
             dist.destroy_process_group()
         return 0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {}, m["proofs"])
     st = m["stats"]
     mill_ach = st["miller_pairs"] * FQMUL_PER_MILLER * IMAD_PER_FQMUL / max(st["miller_ms"] * 1e-3, 1e-12)
     line = {"metric": "SIPP native prove throughput, batched independent instances (instances per second)", "value": count_total * K / m["t_res"],
@@ -393,7 +408,7 @@ def measure_large(k, seed, world, rank, local_rank, barrier, all_max, flush):
         assert ok, "n = 2^%d proof differs from the oracle digest" % k
     return {"n": n, "seed": seed, "n_gpus": world, "prove_s": dt, "pairs_per_s": n / dt, "timed": "one prove through host buffers (H2D of every "
             "rank's shard and D2H of the proof inside), after %s" % ("one warm-up prove" if k <= 16 else "the n = 2^16 run as warm-up"),
-            "h2d_bytes": n * 192, "d2h_bytes": 384 * (2 * k + 1), "sha256_proof": digest,
+            "h2d_bytes": n * 192, "d2h_bytes": 384 * (2 * k + 1), "sha256_proof": digest, "proof": b"".join(proof),
             "parity": ("bit-exact: sha256(proof) equals the oracle's digest (tests/golden/sipp_large.json)" if ok else "no golden digest for this size"),
             "rank0_kernel_ms": {"miller": st["miller_ms"], "reduce_final_exp": st["reduce_fe_ms"], "fold": st["fold_ms"], "other": st["other_ms"]},
             "host_transcript_exposed_ms": st["transcript_ms"], "miller_pairs_rank0": int(st["miller_pairs"]),
@@ -404,6 +419,35 @@ def measure_large(k, seed, world, rank, local_rank, barrier, all_max, flush):
 def ctypes_ptr(t):
     import ctypes
     return ctypes.cast(t.data_ptr(), ctypes.c_char_p)
+
+
+DUMP_BYTES_MAX = 64 << 20
+
+
+def fq12_limbs(raw, plen):
+    """proof bytes (384-byte Fq12 elements, plen per proof) -> float64 [proofs, plen, 12, 8] of the u32 limbs (all < 2^32: exact)"""
+    import numpy as np
+    return np.frombuffer(raw, dtype="<u4").astype(np.float64).reshape(-1, plen, 12, 8)
+
+
+def dump_outputs(directory, proofs, batch=None):
+    """--dump-outputs: `proofs` maps names to single proofs (bytes); `batch` = (bytes of consecutive proofs, elements per proof,
+    index of the first instance).  The batch gets what the single proofs leave of the budget, as a fixed seeded sample of
+    its instances if it does not fit."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    used = 0
+    for name, raw in proofs.items():
+        a = fq12_limbs(raw, len(raw) // 384)[0]
+        np.save(os.path.join(directory, name + ".npy"), a)
+        used += a.nbytes
+    if batch is not None:
+        raw, plen, first = batch
+        a = fq12_limbs(raw, plen)
+        keep = (DUMP_BYTES_MAX - used - 4096) // (a[0].nbytes + 8)    # 8 bytes for the index; 4096 for the .npy headers
+        idx = np.arange(len(a)) if keep >= len(a) else np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))
+        np.save(os.path.join(directory, "batch_proofs.npy"), a[idx])
+        np.save(os.path.join(directory, "batch_instances.npy"), (idx + first).astype(np.float64))
 
 
 def main():
@@ -423,7 +467,10 @@ def main():
     ap.add_argument("--instance-n", type=int, default=128)
     ap.add_argument("--batch-instances", type=int, default=4096, help="config-5 summary added to the default line (0 = skip)")
     ap.add_argument("--large", default="16,20", help="log2 sizes of the BASELINE large configurations added to the default line ('' = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the proofs of the last timed step to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -555,10 +602,12 @@ def main():
 
     # ---- the other BASELINE configurations beside the headline (every rank takes part) ----
     large = []
+    large_proofs = {}
     if not args.quick and not args.n:
         for k in [int(x) for x in args.large.split(",") if x]:
             r = measure_large(k, {16: 3, 20: 4}.get(k, 7), world, rank, local_rank, barrier, all_max, l2_flush)
             if r is not None:
+                large_proofs["proof_n2p%d" % k] = r.pop("proof")
                 r["miller_frac_of_imad_peak_rank0"] = r["miller_loops_per_s_rank0"] * FQMUL_PER_MILLER * IMAD_PER_FQMUL / imad_peak
                 large.append(r)
     bm = None
@@ -675,6 +724,8 @@ def main():
                                      "rank0_miller_ms": bst["miller_ms"], "rank0_final_exp_ms": bst["reduce_fe_ms"], "rank0_fold_ms": bst["fold_ms"],
                                      "miller_frac_of_imad_peak": bst["miller_pairs"] * FQMUL_PER_MILLER * IMAD_PER_FQMUL
                                      / max(bst["miller_ms"] * 1e-3, 1e-12) / imad_peak}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"proof": b"".join(proof_res), **large_proofs}, bm["proofs"] if bm is not None else None)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
