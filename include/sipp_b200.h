@@ -87,6 +87,8 @@ int sipp_device_count(void);          /* 0 when no usable GPU: callers must trea
                                          product of its diagonal and the first log2(blocks) rounds are one matrix fold each.  10..24 = the
                                          budget is 2^value loops whatever n.  0 = the first rounds run on the points */
 #define SIPP_OPT_MATRIX_BLOCK_R 16    /* blocks per look-ahead stage: 4, 8 (default), 16 or 32 (capped so that the stage ends where the tail begins) */
+#define SIPP_OPT_PRODUCT_CHUNK_PAIRS 18 /* batched independent products (sipp_inner_product_batch and friends) only: at most this many pairs per
+                                         line-table chunk; 0 = as many as the 16 GB line-table budget holds [default] */
 int sipp_set_option(int option, int value);
 int sipp_get_option(int option);
 
@@ -184,6 +186,26 @@ int sipp_fr_inverse(const uint8_t x[32], uint8_t out[32]);
 /* Z_L.pow(x) * Z * Z_R.pow(inv_x)                              verifier_native.rs:59-61 */
 int sipp_gt_fold(const uint8_t zl[384], const uint8_t z[384], const uint8_t zr[384], const uint8_t x[32],
                  const uint8_t x_inv[32], uint8_t out[384]);
+
+/* ---- batched independent products: many inner products of unequal lengths (and many pairings) in one call ---------------- */
+/* count independent products, CSR segments: out[j] = prod_{offsets[j] <= i < offsets[j+1]} e(A_i, B_i)  (inner_product,
+ * prover_native.rs:15-23, per segment).  offsets: count + 1 HOST entries, offsets[0] = 0, non-decreasing, offsets[count] = a_len.
+ * An empty segment gives Fq12::one().  out: count x 384 B, boundary format.  Points validated as for sipp_inner_product.
+ * Every out[j] is byte-identical to sipp_inner_product on its segment (GT products are exact: the grouping of the multiplications
+ * does not change the bits), under either SIPP_OPT_FE_NORMALISATION.
+ *   - a_len != b_len: SIPP_ERR_LENGTH; a NULL pointer (count > 0) or bad offsets: SIPP_ERR_ARG -- both before the device is touched.
+ *   - count == 0: returns what sipp_init(0) would (SIPP_ERR_CUDA without a device) and writes nothing.
+ *   - a coordinate >= p, or with SIPP_OPT_VALIDATE_POINTS a point off the curve or a G2 point outside the subgroup, fails the whole
+ *     call with SIPP_ERR_ENCODING and writes nothing.  Identity points (all-zero bytes) contribute the factor 1.
+ *   - Always the split pipeline (lines + 6-lane accumulation); SIPP_OPT_PIPELINE is not read.  SIPP_OPT_FE_ENGINE,
+ *     SIPP_OPT_WIDE_LINES_MAX, SIPP_OPT_BATCH_KPG_MAX (pairs per accumulator group, at most) and SIPP_OPT_PRODUCT_CHUNK_PAIRS apply.
+ *   - sipp_stats.miller_pairs grows by a_len. */
+int sipp_inner_product_batch(const uint8_t *A, size_t a_len, const uint8_t *B, size_t b_len, const size_t *offsets, size_t count,
+                             uint8_t *out);
+/* same, A / B / out in DEVICE memory (boundary format); offsets stay on the host */
+int sipp_inner_product_batch_device(const void *dA, const void *dB, size_t n, const size_t *offsets, size_t count, void *d_out);
+/* out[j] = pairing(a_j, b_j)  (verifier_native.rs:80) for j < count: the batch above with one pair per segment */
+int sipp_pairing_batch(const uint8_t *a, const uint8_t *b, size_t count, uint8_t *out);
 
 /* ---- Fiat-Shamir transcript (host; Poseidon over Goldilocks)  transcript_native.rs:14-66 ---------------- */
 typedef struct { uint64_t state[4]; } sipp_transcript;
@@ -307,6 +329,11 @@ int sipp_microbench(int which, int iters, double *ops_per_s, double *ms);
  * multiply-add of a partial round, in = lo, hi, top, p7, m00; 2: out[0] = in[0]^7, out[1] = in[0]^7 + in[1]; 3, 4: pieces of the IFMA path, see transcript.cc); -1 without AVX-512 / IFMA */
 /* the pairing-matrix stage policy (host logic only): blocks of the first stage (which = 0) or of a later stage (which = 1) at n points; 0 = none */
 long sipp_test_stage_blocks(int which, size_t n);
+/* the plan of sipp_inner_product_batch (host logic only): the accumulator groups of `count` segments (offsets as there) with
+ * SIPP_OPT_BATCH_KPG_MAX = kpg_max and SIPP_OPT_PRODUCT_CHUNK_PAIRS = chunk_pairs.  Writes 4 words per group -- first pair, pairs,
+ * segment, chunk -- to `out` when out_cap >= 4 x groups, the pairs per group at most to *kpg_out (may be NULL); returns the number
+ * of groups or a negative sipp_status */
+long sipp_test_product_plan(const size_t *offsets, size_t count, int kpg_max, size_t chunk_pairs, size_t *out, size_t out_cap, int *kpg_out);
 long sipp_test_poseidon_chain(uint64_t seed, long count);
 int sipp_test_poseidon_scalar(int which, const uint64_t *in, uint64_t *out);
 /* the derived tables of the host Poseidon (sipp::PoseidonFastTables, poseidon_fast.h), for tools/probe/poseidon_lab.cc */

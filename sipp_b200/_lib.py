@@ -12,6 +12,7 @@ LIB_PATH = os.environ.get("SIPP_LIB") or os.path.join(_HERE, "libsipp_b200.so") 
 OK, ERR_CUDA, ERR_ARG, ERR_LENGTH, ERR_ZERO_CHALLENGE, ERR_SHORT_PROOF, ERR_ENCODING, ERR_VERIFY, ERR_COMM = 0, -1, -2, -3, -4, -5, -6, -7, -8
 OPT_FE_NORMALISATION, OPT_FQ12_ORDER, OPT_PROFILE, OPT_PIPELINE, OPT_WIDE_LINES_MAX, OPT_FE_ENGINE, OPT_WIDE_FOLD_MAX, OPT_WIDE_ACCUM_MAX = 1, 2, 3, 4, 5, 6, 7, 8
 OPT_BATCH_KPG_MAX, OPT_FOLD_STRAUS, OPT_BATCH_STREAMS, OPT_BATCH_QLINES, OPT_VALIDATE_POINTS, OPT_MATRIX_TAIL, OPT_MATRIX_BLOCK_N, OPT_MATRIX_BLOCK_R, OPT_MATRIX_FIRST = 9, 10, 11, 12, 13, 14, 15, 16, 17
+OPT_PRODUCT_CHUNK_PAIRS = 18
 
 
 class SippError(RuntimeError):
@@ -79,6 +80,12 @@ def load():
     lib.sipp_inner_product.argtypes = [u8p, u8p, sz, u8p]
     lib.sipp_fr_inverse.argtypes = [u8p, u8p]
     lib.sipp_gt_fold.argtypes = [u8p, u8p, u8p, u8p, u8p, u8p]
+    szp = ctypes.POINTER(ctypes.c_size_t)
+    lib.sipp_inner_product_batch.argtypes = [u8p, sz, u8p, sz, szp, sz, u8p]
+    lib.sipp_inner_product_batch_device.argtypes = [vp, vp, sz, szp, sz, vp]
+    lib.sipp_pairing_batch.argtypes = [u8p, u8p, sz, u8p]
+    lib.sipp_test_product_plan.argtypes = [szp, sz, i, sz, szp, sz, ctypes.POINTER(ctypes.c_int)]
+    lib.sipp_test_product_plan.restype = ctypes.c_long
     lib.sipp_transcript_new.argtypes = [ctypes.POINTER(TranscriptState)]
     lib.sipp_transcript_new.restype = None
     lib.sipp_transcript_append.argtypes = [ctypes.POINTER(TranscriptState), ctypes.POINTER(ctypes.c_uint64), sz]

@@ -117,6 +117,51 @@ def pairing(a: bytes, b: bytes) -> bytes:
     return out.raw
 
 
+def _offsets(lengths: Sequence[int], n: int):
+    """segment sizes -> the count + 1 CSR offsets of sipp_inner_product_batch"""
+    offs = [0]
+    for length in lengths:
+        if length < 0:
+            raise ValueError("negative segment length %d" % length)
+        offs.append(offs[-1] + int(length))
+    if offs[-1] != n:
+        raise ValueError("the segment lengths add up to %d, not to the %d pairs" % (offs[-1], n))
+    return (ctypes.c_size_t * len(offs))(*offs)
+
+
+def inner_product_batch(A: Points, B: Points, lengths: Sequence[int]) -> List[bytes]:
+    """[inner_product(A[o[j]:o[j+1]], B[o[j]:o[j+1]]) for j < len(lengths)] in one call (sipp_inner_product_batch), o = the running
+    sums of `lengths` starting at 0: segment j holds the next lengths[j] pairs, an empty segment gives Fq12::one()"""
+    a, b = _flat(A, G1_BYTES), _flat(B, G2_BYTES)
+    n = len(a) // G1_BYTES
+    assert n == len(b) // G2_BYTES, "assert_eq!(A.len(), B.len())"  # prover_native.rs:16
+    offs = _offsets(lengths, n)
+    count = len(offs) - 1
+    _lib.require_gpu_once()
+    out = ctypes.create_string_buffer(max(1, FQ12_BYTES * count))
+    _lib.check(_lib.load().sipp_inner_product_batch(a, n, b, n, offs, count, out))
+    return _split(out.raw[:FQ12_BYTES * count], FQ12_BYTES)
+
+
+def pairing_batch(a: Points, b: Points) -> List[bytes]:
+    """[pairing(a_j, b_j) for j] in one call (sipp_pairing_batch; verifier_native.rs:80 per pair)"""
+    pa, pb = _flat(a, G1_BYTES), _flat(b, G2_BYTES)
+    count = len(pa) // G1_BYTES
+    assert count == len(pb) // G2_BYTES, "assert_eq!(A.len(), B.len())"
+    _lib.require_gpu_once()
+    out = ctypes.create_string_buffer(max(1, FQ12_BYTES * count))
+    _lib.check(_lib.load().sipp_pairing_batch(pa, pb, count, out))
+    return _split(out.raw[:FQ12_BYTES * count], FQ12_BYTES)
+
+
+def inner_product_batch_device(dA: int, dB: int, n: int, lengths: Sequence[int], d_out: int) -> None:
+    """inner_product_batch on DEVICE buffers (integer pointers, e.g. tensor.data_ptr()): dA n x 64 B, dB n x 128 B, d_out
+    len(lengths) x 384 B, boundary format (sipp_inner_product_batch_device)"""
+    offs = _offsets(lengths, n)
+    _lib.require_gpu_once()
+    _lib.check(_lib.load().sipp_inner_product_batch_device(dA, dB, n, offs, len(offs) - 1, d_out))
+
+
 def sipp_prove_native(A: Points, B: Points) -> List[bytes]:
     """prover_native.rs:26-80; returns the proof as a list of 2 log2(n) + 1 Fq12 byte strings."""
     a, b = _flat(A, G1_BYTES), _flat(B, G2_BYTES)

@@ -13,18 +13,11 @@
 //
 // Replaces the per-pair `pairing` calls + serial product of /root/reference/src/prover_native.rs:17-22 (and :48-49).
 #define SIPP_CURVE_FQ2_CALLS 1
+#include "accum.cuh"
 #include "coop.cuh"
 #include "device_common.cuh"
 
 namespace sipp {
-
-#define SIPP_LINE_WORDS 80                               // 5 Fq2
-#define SIPP_PAIR_LINE_WORDS (SIPP_LINES_PER_PAIR * SIPP_LINE_WORDS)
-#ifndef SIPP_ACCUM_THREADS
-#define SIPP_ACCUM_THREADS 128
-#endif
-#define SIPP_GROUPS_PER_WARP 5
-#define SIPP_ACCUM_GROUPS (SIPP_ACCUM_THREADS / 32 * SIPP_GROUPS_PER_WARP)
 
 // ------------------------------------------------------------------------------------------------ L: line generation
 // A chunk covers pairs [c0, c0 + mc) of EVERY product of the job; lines layout [prod][mc][91][80 words].
@@ -166,37 +159,8 @@ __global__ void __launch_bounds__(128) k_eval_lines_mat(const uint32_t* __restri
 }
 
 // ------------------------------------------------------------------------------------------------ A: accumulation
-__device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
-    unsigned s = (unsigned)__cvta_generic_to_shared(smem);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(s), "l"(gmem));
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;"); }
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
-
-__device__ __forceinline__ Fq2 lane_one(int k) { return k == 0 ? fq2_one() : fq2_zero(); }
-
-// tree product over the groups of a block; result in group 0.  sh: [groups][96 words]
-__device__ __noinline__ Fq2 block_product_coop(const Lane6& L, Fq2 f, uint32_t* sh, int group, int ngroups) {
-    const int k = L.k < 6 ? L.k : 0;
-    int n = ngroups;
-    while (n > 1) {
-        int half = (n + 1) >> 1;
-        __syncthreads();
-        if (L.k < 6 && group >= half && group < n) store_fq2_words(sh + group * 96 + k * 16, f);
-        __syncthreads();
-        bool take = group + half < n;
-        Fq2 other = take ? load_fq2_words(sh + (group + half) * 96 + k * 16) : lane_one(k);
-        f = coop_mul(L, f, other);
-        n = half;
-    }
-    return f;
-}
-
 // grid = (blocks, nprod).  Group gid of product `prod` folds pairs [gid * kpg, (gid + 1) * kpg) of that product.
 // lines: chunk-local, pair index = prod_local_base + j.
-#ifndef SIPP_ACCUM_MINBLOCKS
-#define SIPP_ACCUM_MINBLOCKS 2
-#endif
 __global__ void __launch_bounds__(SIPP_ACCUM_THREADS, SIPP_ACCUM_MINBLOCKS) k_accum(const uint32_t* __restrict__ lines, size_t m_chunk, int nprod_in_chunk, int kpg,
                                                             uint32_t* __restrict__ partials, int partial_stride_prod, int block_offset, int segmented) {
     __shared__ __align__(16) uint32_t stage[SIPP_ACCUM_GROUPS][2][SIPP_LINE_WORDS];

@@ -87,6 +87,18 @@ int launch_test_poseidon(uint64_t* states, size_t count, cudaStream_t s);
 int launch_gt_fold_batch(const uint32_t* proofs, size_t stride, int slot_l, int slot_r, const uint64_t* challenges, uint32_t* z, size_t count,
                          cudaStream_t s);
 
+// batched independent products (k_products.cu, host driver products.cu).  An accumulator group folds pairs [first, first + pairs)
+// of the flat pair list, all of one segment and one chunk; a task multiplies work[src .. src + n) into work[dst] (Fq12 slots of 96 words).
+struct ProductGroup {
+    uint32_t first, pairs;
+};
+struct ProductTask {
+    uint32_t src, n, dst, pad;
+};
+#define SIPP_PRODUCT_SPAN 40  // Fq12 per task: 2 for each of the 20 six-lane groups of a block
+int launch_accum_plan(const uint32_t* lines, const ProductGroup* plan, size_t g0, size_t ngroups, size_t c0, int kpg, uint32_t* partials, cudaStream_t s);
+int launch_seg_product(const ProductTask* tasks, size_t ntasks, uint32_t* work, cudaStream_t s);
+
 // BLS input producers (k_bls.cu): group 1 = G1 (16 words per point), 2 = G2 (32 words)
 size_t window_table_bytes(int group);
 int launch_window_table(int group, const uint32_t* base, uint32_t* table, cudaStream_t s);

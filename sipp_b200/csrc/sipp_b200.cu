@@ -36,6 +36,7 @@ int g_opt_matrix_n = 32;       // pairing matrix of single points (k_mat.cu) onc
 int g_opt_matrix_first = 1;     // the first matrix is built from the inputs, under the host's absorb chain; 10..24: log2 of its Miller-loop budget
 int g_opt_matrix_block_n = 256, g_opt_matrix_block_r = 8;  // look-ahead stages: from at most this many points, that many blocks
 int g_opt_validate = 1;        // every prove / verify entry point checks its points: on the curve, B_i in the order-r subgroup
+int g_opt_product_chunk = 0;    // batched independent products (products.cu): pairs per line-table chunk, at most; 0 = by the budget
 
 struct TimedSpan {
     cudaEvent_t a, b;
@@ -629,6 +630,7 @@ int sipp_set_option(int option, int value) {
         case SIPP_OPT_BATCH_STREAMS: g_opt_batch_streams = value < 0 ? 0 : value; return SIPP_OK;
         case SIPP_OPT_BATCH_QLINES: g_opt_batch_qlines = value ? 1 : 0; return SIPP_OK;
         case SIPP_OPT_VALIDATE_POINTS: g_opt_validate = value ? 1 : 0; return SIPP_OK;
+        case SIPP_OPT_PRODUCT_CHUNK_PAIRS: g_opt_product_chunk = value < 0 ? 0 : value; return SIPP_OK;
         case SIPP_OPT_MATRIX_TAIL:
             if (value < 0 || value > 64 || (value & (value - 1))) return fail(SIPP_ERR_ARG, "SIPP_OPT_MATRIX_TAIL: 0 or a power of two <= 64");
             g_opt_matrix_n = value;
@@ -659,6 +661,7 @@ int sipp_get_option(int option) {
         case SIPP_OPT_BATCH_STREAMS: return g_opt_batch_streams;
         case SIPP_OPT_BATCH_QLINES: return g_opt_batch_qlines;
         case SIPP_OPT_VALIDATE_POINTS: return g_opt_validate;
+        case SIPP_OPT_PRODUCT_CHUNK_PAIRS: return g_opt_product_chunk;
         case SIPP_OPT_MATRIX_TAIL: return g_opt_matrix_n;
         case SIPP_OPT_MATRIX_FIRST: return g_opt_matrix_first;
         case SIPP_OPT_MATRIX_BLOCK_N: return g_opt_matrix_block_n;
