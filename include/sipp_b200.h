@@ -103,7 +103,10 @@ size_t sipp_ctx_len(const sipp_ctx *ctx);                     /* current n */
 int sipp_ctx_inner_product(sipp_ctx *ctx, uint8_t out[384]);
 /* Z_L = inner_product(A2, B1), Z_R = inner_product(A1, B2)     prover_native.rs:46-49 */
 int sipp_ctx_cross_products(sipp_ctx *ctx, uint8_t zl[384], uint8_t zr[384]);
-/* A <- A1 + x A2, B <- B1 + x^-1 B2, n <- n/2                   prover_native.rs:60-74 */
+/* A <- A1 + x A2, B <- B1 + x^-1 B2, n <- n/2                   prover_native.rs:60-74
+ * Fold scalars (here and in sipp_gt_fold): little-endian, checked on the host before anything else, in this order: x >= r or
+ * x_inv >= r -> SIPP_ERR_ENCODING; x == 0 -> SIPP_ERR_ZERO_CHALLENGE; x x_inv != 1 (mod r) -> SIPP_ERR_ENCODING ("x_inv is not the
+ * inverse of x").  A refused fold leaves the context as it was (n, points, stage in progress). */
 int sipp_ctx_fold(sipp_ctx *ctx, const uint8_t x[32], const uint8_t x_inv[32]);
 /* Opt-in for a host that keeps its own transcript: with stages on, sipp_ctx_inner_product / _cross_products / _fold may run on
  * pairing-matrix stages (SIPP_OPT_MATRIX_*: same Z, Z_L, Z_R bit for bit, several times shorter rounds) exactly as the library's
@@ -183,7 +186,8 @@ int sipp_pairing(const uint8_t a[64], const uint8_t b[128], uint8_t out[384]);
 int sipp_inner_product(const uint8_t *A, const uint8_t *B, size_t n, uint8_t out[384]);
 /* x.inverse() in Fr                                            prover_native.rs:58 */
 int sipp_fr_inverse(const uint8_t x[32], uint8_t out[32]);
-/* Z_L.pow(x) * Z * Z_R.pow(inv_x)                              verifier_native.rs:59-61 */
+/* Z_L.pow(x) * Z * Z_R.pow(inv_x)                              verifier_native.rs:59-61
+ * x, x_inv: the fold-scalar checks of sipp_ctx_fold, made before the device is touched */
 int sipp_gt_fold(const uint8_t zl[384], const uint8_t z[384], const uint8_t zr[384], const uint8_t x[32],
                  const uint8_t x_inv[32], uint8_t out[384]);
 
@@ -313,6 +317,16 @@ int sipp_test_fq12_op(int op, const uint8_t *a, const uint8_t *b, uint8_t *out, 
  * (G2, x^-1) sub-scalars in non-adjacent form.  Writes the raw plan as 32-bit words: 6 components (2 for G1, then 4 for
  * G2) of {plus[5], minus[5], neg}, then g1_bits, g2_bits; returns the number of words written or a negative status. */
 int sipp_test_fold_plan(const uint8_t x[32], const uint8_t x_inv[32], uint32_t *out_words, size_t out_cap);
+/* the same recoding by the device code of the batched prover's transcript (glv::plan_build with the __device__ tables of
+ * k_tr_round), one thread per pair, on `count` pairs (x, x_inv: count x 32 B).  Writes count plans of 68 words in the layout of
+ * sipp_test_fold_plan; returns the number of pairs the recoding refused, or a negative status.  The scalars are not checked. */
+int sipp_test_fold_plan_device(const uint8_t *x, const uint8_t *x_inv, size_t count, uint32_t *out_words);
+/* one launch of a batched fold kernel over `count` instances of n points each (n even): instance j owns A, B [j n, (j + 1) n) and is
+ * folded with xs[j], x_invs[j] (32 B each, the checks of sipp_ctx_fold), h = n / 2.  kernel: 0 k_fold_batch, 1 k_fold_wide_batch,
+ * 2 k_fold_straus.  Points are decoded and checked as by sipp_ctx_create; A_out (count x h x 64 B), B_out (count x h x 128 B)
+ * receive the first h points of every instance. */
+int sipp_test_fold_batch(const uint8_t *A, const uint8_t *B, size_t n, size_t count, const uint8_t *xs, const uint8_t *x_invs, int kernel,
+                         uint8_t *A_out, uint8_t *B_out);
 /* which: 0 mad.lo.u32 chains, 1 mad.wide.u32 chains, 2 lo/hi carry chains, 3 fq_mul PTX, 4 fq_mul portable.
  * returns operations per second (IMAD instructions for 0-2, Fq multiplications for 3-4) in *ops_per_s */
 /* device transcript (k_transcript.cu): `count` independent Poseidon permutations, 12 x u64 each, in place */

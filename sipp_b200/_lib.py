@@ -116,6 +116,8 @@ def load():
     lib.sipp_test_transcript_round_device.argtypes = [ctypes.POINTER(ctypes.c_uint64), u8p, i, sz, u8p, ctypes.POINTER(ctypes.c_uint32)]
     lib.sipp_test_fold_plan.argtypes = [u8p, u8p, ctypes.POINTER(ctypes.c_uint32), sz]
     u32p = ctypes.POINTER(ctypes.c_uint32)
+    lib.sipp_test_fold_plan_device.argtypes = [u8p, u8p, sz, u32p]
+    lib.sipp_test_fold_batch.argtypes = [u8p, u8p, sz, sz, u8p, u8p, i, u8p, u8p]
     lib.sipp_statement_u32_len.argtypes = [sz]
     lib.sipp_statement_u32_len.restype = sz
     lib.sipp_statement_to_u32.argtypes = [u8p, u8p, sz, u8p, u8p, u8p, u8p, u32p, sz]

@@ -118,6 +118,12 @@ __device__ __forceinline__ uint64_t tr_append_fq12_lanes(uint64_t s, int l, cons
     });
 }
 
+// the lattice tables of the device recoding (glv_consts.h as __device__ constants)
+__device__ __forceinline__ glv::Tables device_glv_tables() {
+    return glv::Tables{&SIPP_GLV_G1_BASIS[0][0][0], &SIPP_GLV_G1_RECIP[0][0], SIPP_GLV_G1_RECIP_SIGN,
+                       &SIPP_GLS_G2_BASIS[0][0][0], &SIPP_GLS_G2_RECIP[0][0], SIPP_GLS_G2_RECIP_SIGN};
+}
+
 __device__ __forceinline__ void load_rc_shared(uint64_t* rc) {
     for (int i = threadIdx.x; i < 360; i += blockDim.x) rc[i] = c_rc[i];
     __syncthreads();
@@ -203,11 +209,23 @@ __global__ void __launch_bounds__(SIPP_TR_THREADS) k_tr_round(uint64_t* __restri
     if (rc_inv) {
         atomicOr(flags, 1);
     } else {
-        const glv::Tables t = {&SIPP_GLV_G1_BASIS[0][0][0], &SIPP_GLV_G1_RECIP[0][0], SIPP_GLV_G1_RECIP_SIGN,
-                               &SIPP_GLS_G2_BASIS[0][0][0], &SIPP_GLS_G2_RECIP[0][0], SIPP_GLS_G2_RECIP_SIGN};
-        if (glv::plan_build(v, vi, t, &plan)) atomicOr(flags, 2);
+        if (glv::plan_build(v, vi, device_glv_tables(), &plan)) atomicOr(flags, 2);
     }
     plans[inst] = plan;
+}
+
+// test hook: the recoding k_tr_round runs, on given pairs (xs, xinvs: 4 u64 each), one thread per pair; fails counts the pairs
+// plan_build refused
+__global__ void __launch_bounds__(64) k_test_plan_build(const uint64_t* __restrict__ xs, const uint64_t* __restrict__ xinvs, size_t count,
+                                                         FoldPlan* __restrict__ plans, int* __restrict__ fails) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= count) return;
+    uint64_t kx[4], ki[4];
+    for (int w = 0; w < 4; w++) { kx[w] = xs[4 * i + w]; ki[w] = xinvs[4 * i + w]; }
+    FoldPlan plan;
+    for (int w = 0; w < (int)(sizeof(FoldPlan) / 4); w++) ((uint32_t*)&plan)[w] = 0;
+    if (glv::plan_build(kx, ki, device_glv_tables(), &plan)) atomicAdd(fails, 1);
+    plans[i] = plan;
 }
 
 // test hook: `count` independent permutations, 16 lanes each
@@ -244,6 +262,10 @@ int launch_tr_round(uint64_t* states, const uint32_t* proofs, size_t np, int slo
     int e = load_rc();
     if (e) return e;
     k_tr_round<<<(unsigned)((count * 16 + SIPP_TR_THREADS - 1) / SIPP_TR_THREADS), SIPP_TR_THREADS, 0, s>>>(states, proofs, np, slot_z, slot_l, slot_r, order, count, plans, challenges, flags);
+    return (int)cudaGetLastError();
+}
+int launch_test_plan_build(const uint64_t* xs, const uint64_t* xinvs, size_t count, FoldPlan* plans, int* fails, cudaStream_t s) {
+    k_test_plan_build<<<(unsigned)((count + 63) / 64), 64, 0, s>>>(xs, xinvs, count, plans, fails);
     return (int)cudaGetLastError();
 }
 int launch_test_poseidon(uint64_t* states, size_t count, cudaStream_t s) {

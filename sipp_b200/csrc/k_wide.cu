@@ -243,10 +243,10 @@ __global__ void __launch_bounds__(SIPP_WIDE_THREADS) k_fold_wide_batch(uint32_t*
                                                                       const FoldPlan* __restrict__ plans, unsigned g2_blocks) {
     __shared__ __align__(16) uint32_t smem[SIPP_WIDE_GROUPS * SIPP_LP_SLOTS * 8];
     __shared__ __align__(16) uint32_t xch[SIPP_WIDE_GROUPS * 48];  // one Jacobian point per group (G2: 48 words, G1: 24)
-    // the two groups of a warp must run the same digit schedule: they take two elements of the SAME instance (h >= 2: h is even
-    // and element pairs start at even indices), or the same element twice when an instance has a single element left (h == 1)
+    // the two groups of a warp must run the same digit schedule: they take two elements of the SAME instance (h even: element pairs
+    // start at even indices), or the same element twice when h is odd (h == 1 in the lock-step prover, whose h is a power of two)
     const size_t total = count * h;
-    const int epw = h >= 2 ? 2 : 1;
+    const int epw = (h & 1) ? 1 : 2;
     const int warp = threadIdx.x >> 5, group = threadIdx.x / SIPP_LP_LANES, lane = threadIdx.x % SIPP_LP_LANES, gi = group & 1;
     uint32_t* slots = smem + group * (SIPP_LP_SLOTS * 8);
     DevMachine mach;
@@ -344,7 +344,7 @@ __global__ void __launch_bounds__(SIPP_WIDE_THREADS) k_fold_wide_batch(uint32_t*
 
 
 int launch_fold_wide_batch(uint32_t* A, uint32_t* B, size_t h, size_t stride, size_t count, const FoldPlan* plans, cudaStream_t s) {
-    const size_t total = count * h, epw = h >= 2 ? 2 : 1;
+    const size_t total = count * h, epw = (h & 1) ? 1 : 2;
     const unsigned g2_blocks = (unsigned)((total + epw - 1) / epw), g1_blocks = (unsigned)((total + 2 * epw - 1) / (2 * epw));
     k_fold_wide_batch<<<g2_blocks + g1_blocks, SIPP_WIDE_THREADS, 0, s>>>(A, B, h, stride, count, plans, g2_blocks);
     return (int)cudaGetLastError();

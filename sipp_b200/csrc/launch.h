@@ -84,6 +84,7 @@ int launch_tr_absorb_pairs(const uint32_t* bytesA, const uint32_t* bytesB, size_
 int launch_tr_round(uint64_t* states, const uint32_t* proofs, size_t np, int slot_z, int slot_l, int slot_r, int order, size_t count, FoldPlan* plans,
                     uint64_t* challenges, int* flags, cudaStream_t s);
 int launch_test_poseidon(uint64_t* states, size_t count, cudaStream_t s);
+int launch_test_plan_build(const uint64_t* xs, const uint64_t* xinvs, size_t count, FoldPlan* plans, int* fails, cudaStream_t s);
 int launch_gt_fold_batch(const uint32_t* proofs, size_t stride, int slot_l, int slot_r, const uint64_t* challenges, uint32_t* z, size_t count,
                          cudaStream_t s);
 

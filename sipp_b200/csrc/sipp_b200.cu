@@ -107,6 +107,23 @@ Scalar256 scalar_from_bytes(const uint8_t* b) {
     return s;
 }
 
+// The scalars of one fold (prover_native.rs:58-69, verifier_native.rs:46-61): x and x_inv canonical (< r), x != 0, x x_inv = 1 (mod r).
+// The kernels only see the recodings, which would reduce a scalar >= r silently; a wrong inverse would fold B by whatever it is given
+// and, on the pairing-matrix route, give other Z_L / Z_R than the point route.  Host only: one Fr product, no device work.
+int check_fold_scalars(const uint8_t* x, const uint8_t* x_inv) {
+    const uint64_t R[4] = {0x43e1f593f0000001ull, 0x2833e84879b97091ull, 0xb85045b68181585dull, 0x30644e72e131a029ull};
+    const uint64_t R2[4] = {0x1bb8e645ae216da7ull, 0x53fe3ab1e35c59e3ull, 0x8c49833d53bb8085ull, 0x0216d0b17f4e44a5ull};  // 2^512 mod r
+    uint64_t a[4], b[4], t[4];
+    memcpy(a, x, 32);
+    memcpy(b, x_inv, 32);
+    if (glv::fr_geq(a, R) || glv::fr_geq(b, R)) return fail(SIPP_ERR_ENCODING, "fold scalar out of range (must be < r)");
+    if (!(a[0] | a[1] | a[2] | a[3])) return fail(SIPP_ERR_ZERO_CHALLENGE, "challenge is zero: x.inverse().unwrap() panics in the reference");
+    glv::fr_mont_mul(t, a, b);   // x x_inv / 2^256
+    glv::fr_mont_mul(t, t, R2);  // x x_inv
+    if (t[0] != 1 || (t[1] | t[2] | t[3])) return fail(SIPP_ERR_ENCODING, "x_inv is not the inverse of x");
+    return SIPP_OK;
+}
+
 // Device memory pool: contexts and staging buffers are created per prove call; cudaMalloc / cudaFree cost hundreds of
 // microseconds each and cudaFree synchronises the device, so freed blocks are kept and reused (grow-only, released in
 // sipp_shutdown).  One host thread per process by contract, so no locking.
@@ -821,6 +838,7 @@ int sipp_ctx_cross_products(sipp_ctx* c, uint8_t zl[384], uint8_t zr[384]) {
 
 int sipp_ctx_fold(sipp_ctx* c, const uint8_t x[32], const uint8_t x_inv[32]) {
     if (!c || !x || !x_inv) return fail(SIPP_ERR_ARG, "null argument");
+    if (int rc = check_fold_scalars(x, x_inv)) return rc;  // before any stage dispatch or device work: a refusal changes nothing
     if (c->n < 2) return fail(SIPP_ERR_ARG, "fold needs n >= 2");
     if (c->pending_validation) CK(cudaStreamWaitEvent(g_stream, c->validated, 0));  // the deferred check reads the points folded here
     if (c->mt.n) return mat_fold(c, c->mt, x, x_inv);  // :60-74 on the matrix of the stage in progress
@@ -929,9 +947,11 @@ int sipp_pairing(const uint8_t a[64], const uint8_t b[128], uint8_t out[384]) { 
 
 int sipp_gt_fold(const uint8_t zl[384], const uint8_t z[384], const uint8_t zr[384], const uint8_t x[32], const uint8_t x_inv[32],
                  uint8_t out[384]) {
-    int rc = ensure_init();
-    if (rc) return rc;
     if (!zl || !z || !zr || !x || !x_inv || !out) return fail(SIPP_ERR_ARG, "null argument");
+    int rc = check_fold_scalars(x, x_inv);  // raw 256-bit exponents: x and x + r differ on an Fq12 outside GT
+    if (rc) return rc;
+    rc = ensure_init();
+    if (rc) return rc;
     rc = scratch_reserve(1);
     if (rc) return rc;
     uint32_t* d_in;
@@ -1179,6 +1199,69 @@ int sipp_test_fold_plan(const uint8_t x[32], const uint8_t x_inv[32], uint32_t* 
     if (fold_plan_build(x, x_inv, &plan)) return fail(SIPP_ERR_ENCODING, "fold scalar out of range (must be < r)");
     memcpy(out_words, &plan, sizeof plan);
     return (int)(sizeof(FoldPlan) / 4);
+}
+
+int sipp_test_fold_plan_device(const uint8_t* x, const uint8_t* x_inv, size_t count, uint32_t* out_words) {
+    if (!x || !x_inv || !out_words || count == 0) return fail(SIPP_ERR_ARG, "bad argument");
+    int rc = ensure_init();
+    if (rc) return rc;
+    uint64_t *dx = nullptr, *dxi = nullptr;
+    FoldPlan* dplans = nullptr;
+    int* dfails = nullptr;
+    int fails = 0;
+    cudaError_t e = cudaMalloc(&dx, count * 32);
+    if (e == cudaSuccess) e = cudaMalloc(&dxi, count * 32);
+    if (e == cudaSuccess) e = cudaMalloc(&dplans, count * sizeof(FoldPlan));
+    if (e == cudaSuccess) e = cudaMalloc(&dfails, sizeof(int));
+    if (e == cudaSuccess) e = cudaMemcpyAsync(dx, x, count * 32, cudaMemcpyHostToDevice, g_stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(dxi, x_inv, count * 32, cudaMemcpyHostToDevice, g_stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(dfails, 0, sizeof(int), g_stream);
+    if (e == cudaSuccess) e = (cudaError_t)launch_test_plan_build(dx, dxi, count, dplans, dfails, g_stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out_words, dplans, count * sizeof(FoldPlan), cudaMemcpyDeviceToHost, g_stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&fails, dfails, sizeof(int), cudaMemcpyDeviceToHost, g_stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(g_stream);
+    g_stats.launches++;
+    cudaFree(dx); cudaFree(dxi); cudaFree(dplans); cudaFree(dfails);
+    if (e != cudaSuccess) return cuda_fail(e, "sipp_test_fold_plan_device");
+    return fails;
+}
+
+int sipp_test_fold_batch(const uint8_t* A, const uint8_t* B, size_t n, size_t count, const uint8_t* xs, const uint8_t* x_invs, int kernel,
+                         uint8_t* A_out, uint8_t* B_out) {
+    if (!A || !B || !xs || !x_invs || !A_out || !B_out || count == 0 || n < 2 || n % 2 || kernel < 0 || kernel > 2)
+        return fail(SIPP_ERR_ARG, "bad argument");
+    std::vector<FoldPlan> plans(count);
+    for (size_t j = 0; j < count; j++) {
+        int rc = check_fold_scalars(xs + 32 * j, x_invs + 32 * j);
+        if (rc) return rc;
+        if (fold_plan_build(xs + 32 * j, x_invs + 32 * j, &plans[j])) return fail(SIPP_ERR_ENCODING, "fold scalar out of range (must be < r)");
+    }
+    sipp_ctx* c;
+    int rc = ctx_create_ex(A, B, n * count, &c, false);  // decode + point checks as sipp_ctx_create
+    if (rc) return rc;
+    const size_t h = n / 2, total = n * count;
+    FoldPlan* dplans = nullptr;
+    cudaError_t e = pool_alloc((void**)&dplans, count * sizeof(FoldPlan));
+    if (e == cudaSuccess) e = cudaMemcpyAsync(dplans, plans.data(), count * sizeof(FoldPlan), cudaMemcpyHostToDevice, g_stream);
+    if (e == cudaSuccess) {
+        Span sp(2, g_stream);
+        e = (cudaError_t)(kernel == 0   ? launch_fold_batch(c->dA, c->dB, h, n, count, dplans, g_stream)
+                          : kernel == 1 ? launch_fold_wide_batch(c->dA, c->dB, h, n, count, dplans, g_stream)
+                                        : launch_fold_straus(c->dA, c->dB, h, n, count, dplans, g_stream));
+        g_stats.launches++;
+    }
+    std::vector<uint8_t> a(total * 64), b(total * 128);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(g_stream);  // the plans were staged from pageable memory
+    pool_free(dplans);
+    if (e != cudaSuccess) { sipp_ctx_destroy(c); return cuda_fail(e, "sipp_test_fold_batch"); }
+    rc = sipp_ctx_read(c, a.data(), b.data());
+    sipp_ctx_destroy(c);
+    if (rc) return rc;
+    for (size_t j = 0; j < count; j++) {
+        memcpy(A_out + 64 * h * j, &a[64 * n * j], 64 * h);
+        memcpy(B_out + 128 * h * j, &b[128 * n * j], 128 * h);
+    }
+    return SIPP_OK;
 }
 
 int sipp_microbench(int which, int iters, double* ops_per_s, double* ms_out) {
