@@ -87,7 +87,8 @@ int sipp_device_count(void);          /* 0 when no usable GPU: callers must trea
                                          product of its diagonal and the first log2(blocks) rounds are one matrix fold each.  10..24 = the
                                          budget is 2^value loops whatever n.  0 = the first rounds run on the points */
 #define SIPP_OPT_MATRIX_BLOCK_R 16    /* blocks per look-ahead stage: 4, 8 (default), 16 or 32 (capped so that the stage ends where the tail begins) */
-#define SIPP_OPT_PRODUCT_CHUNK_PAIRS 18 /* batched independent products (sipp_inner_product_batch and friends) only: at most this many pairs per
+#define SIPP_OPT_PRODUCT_CHUNK_PAIRS 18 /* batched independent products (sipp_inner_product_batch and friends) and the ragged batched prover
+                                         (sipp_prove_native_batch_ragged, every round's products) only: at most this many pairs per
                                          line-table chunk; 0 = as many as the 16 GB line-table budget holds [default] */
 int sipp_set_option(int option, int value);
 int sipp_get_option(int option);
@@ -268,6 +269,32 @@ int sipp_verify_native_batch(const uint8_t *A, const uint8_t *B, size_t n, size_
 /* same with DEVICE buffers in boundary format (inputs resident in HBM, proofs left in HBM) */
 int sipp_prove_native_batch_device(const void *dA, const void *dB, size_t n, size_t count, void *d_proofs);
 
+/* ---- batched instances of different sizes: `count` independent proofs in lock-step, each with its own n ------------------- */
+/* count independent proofs of instances of different sizes, in lock-step.  Instance j = pairs [offsets[j], offsets[j+1]) of A and B;
+ * n_j = offsets[j+1] - offsets[j] must be a non-zero power of two.  offsets: count + 1 HOST entries, offsets[0] = 0, offsets[count] = a_len.
+ * proofs: sum_j sipp_proof_len(n_j) x 384 B.  Instance j's proof starts at byte 384 * sum_{k<j} sipp_proof_len(n_k), in the returned
+ * (reversed) order.  Every proof is byte-identical to sipp_prove_native on that instance's pairs (prover_native.rs:26-80).
+ *   - a_len != b_len: SIPP_ERR_LENGTH.  SIPP_ERR_ARG: a NULL pointer, count == 0, offsets[0] != 0, decreasing offsets,
+ *     offsets[count] != a_len, a segment of length 0 or not a power of two, more than 2^32 - 1 pairs.  All of these are returned
+ *     before the device is touched; valid arguments without a device give SIPP_ERR_CUDA.
+ *   - a coordinate >= p, or with SIPP_OPT_VALIDATE_POINTS a point off the curve or a G2 point outside the subgroup, fails the whole
+ *     call with SIPP_ERR_ENCODING, a zero challenge with SIPP_ERR_ZERO_CHALLENGE; in both cases nothing is written to `proofs`.
+ *   - n_j = 1 gives the proof [Z] = [pairing(A_i, B_i)].
+ *   - Rounds run together: round 0 computes Z of every instance, round r >= 1 the instances with log2 n_j >= r.  The products use
+ *     the path of sipp_inner_product_batch.  Options read: SIPP_OPT_FE_NORMALISATION, SIPP_OPT_FQ12_ORDER, SIPP_OPT_WIDE_LINES_MAX,
+ *     SIPP_OPT_FE_ENGINE, SIPP_OPT_WIDE_FOLD_MAX, SIPP_OPT_BATCH_KPG_MAX, SIPP_OPT_FOLD_STRAUS, SIPP_OPT_VALIDATE_POINTS and
+ *     SIPP_OPT_PRODUCT_CHUNK_PAIRS.  Not read: SIPP_OPT_PIPELINE, SIPP_OPT_BATCH_STREAMS, SIPP_OPT_BATCH_QLINES and the matrix
+ *     stages (SIPP_OPT_MATRIX_*).
+ *   - The registration of A and B in every instance's transcript is a chain of 8 n_j Poseidon permutations on the device, and the
+ *     longest instance bounds it (about 9.4 us per permutation on the device against 0.61 us on the host): an instance far larger
+ *     than the rest is better proved on its own with sipp_prove_native.
+ *   - sipp_stats.miller_pairs grows by sum_j (3 n_j - 2), fold_points by sum_j (n_j - 1).
+ * Until a ragged verifier exists, verify with sipp_verify_native_batch once per size. */
+int sipp_prove_native_batch_ragged(const uint8_t *A, size_t a_len, const uint8_t *B, size_t b_len, const size_t *offsets, size_t count,
+                                   uint8_t *proofs);
+/* the same with A, B and proofs in DEVICE memory (boundary format); offsets stay on the host */
+int sipp_prove_native_batch_ragged_device(const void *dA, const void *dB, size_t n, const size_t *offsets, size_t count, void *d_proofs);
+
 /* ---- input producers of the BLS-aggregation demo (bin/bls_aggregation.rs:95-117; SURVEY 8f row 3) ---------------------------- */
 /* Scalars are 32-byte little-endian integers < r.  The `_device` forms take DEVICE pointers in the same formats.
  * `map_to_g2_without_cofactor_mul(u).mul_by_cofactor()` (:100-104) is not provided: it lives in the un-vendored starky-bn254
@@ -348,6 +375,11 @@ long sipp_test_stage_blocks(int which, size_t n);
  * segment, chunk -- to `out` when out_cap >= 4 x groups, the pairs per group at most to *kpg_out (may be NULL); returns the number
  * of groups or a negative sipp_status */
 long sipp_test_product_plan(const size_t *offsets, size_t count, int kpg_max, size_t chunk_pairs, size_t *out, size_t out_cap, int *kpg_out);
+/* the schedule of sipp_prove_native_batch_ragged (host logic only) under the current options: 5 words per round r = 0 .. log2 max n_j --
+ * active instances, pairs of its products, fold elements, fold kernel (-1 none, 0 k_fold_batch, 1 k_fold_wide_batch, 2 k_fold_straus,
+ * in their ragged forms) and line-table chunks -- to `out` when out_cap >= 5 x rounds; returns the number of rounds or a negative
+ * sipp_status (the argument checks of sipp_prove_native_batch_ragged) */
+long sipp_test_ragged_schedule(const size_t *offsets, size_t count, long long *out, size_t out_cap);
 long sipp_test_poseidon_chain(uint64_t seed, long count);
 int sipp_test_poseidon_scalar(int which, const uint64_t *in, uint64_t *out);
 /* the derived tables of the host Poseidon (sipp::PoseidonFastTables, poseidon_fast.h), for tools/probe/poseidon_lab.cc */

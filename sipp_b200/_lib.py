@@ -86,6 +86,8 @@ def load():
     lib.sipp_pairing_batch.argtypes = [u8p, u8p, sz, u8p]
     lib.sipp_test_product_plan.argtypes = [szp, sz, i, sz, szp, sz, ctypes.POINTER(ctypes.c_int)]
     lib.sipp_test_product_plan.restype = ctypes.c_long
+    lib.sipp_test_ragged_schedule.argtypes = [szp, sz, ctypes.POINTER(ctypes.c_longlong), sz]
+    lib.sipp_test_ragged_schedule.restype = ctypes.c_long
     lib.sipp_transcript_new.argtypes = [ctypes.POINTER(TranscriptState)]
     lib.sipp_transcript_new.restype = None
     lib.sipp_transcript_append.argtypes = [ctypes.POINTER(TranscriptState), ctypes.POINTER(ctypes.c_uint64), sz]
@@ -111,6 +113,8 @@ def load():
     lib.sipp_test_fq12_op.argtypes = [i, u8p, u8p, u8p, sz]
     lib.sipp_prove_native_batch.argtypes = [u8p, u8p, sz, sz, u8p]
     lib.sipp_prove_native_batch_device.argtypes = [vp, vp, sz, sz, vp]
+    lib.sipp_prove_native_batch_ragged.argtypes = [u8p, sz, u8p, sz, szp, sz, u8p]
+    lib.sipp_prove_native_batch_ragged_device.argtypes = [vp, vp, sz, szp, sz, vp]
     lib.sipp_verify_native_batch.argtypes = [u8p, u8p, sz, sz, u8p, sz, ctypes.POINTER(ctypes.c_int), u8p, u8p, u8p]
     lib.sipp_test_poseidon_device.argtypes = [ctypes.POINTER(ctypes.c_uint64), sz]
     lib.sipp_test_transcript_round_device.argtypes = [ctypes.POINTER(ctypes.c_uint64), u8p, i, sz, u8p, ctypes.POINTER(ctypes.c_uint32)]

@@ -197,6 +197,48 @@ def sipp_prove_native_batch(A: Points, B: Points, n: int) -> List[List[bytes]]:
     return [_split(raw[j * plen * FQ12_BYTES:(j + 1) * plen * FQ12_BYTES], FQ12_BYTES) for j in range(count)]
 
 
+def _ragged_offsets(lengths: Sequence[int], n: int):
+    """instance sizes -> the count + 1 CSR offsets of sipp_prove_native_batch_ragged; every size a non-zero power of two"""
+    for length in lengths:
+        if int(length) <= 0 or int(length) & (int(length) - 1):
+            raise ValueError("instance size %d is not a non-zero power of two" % length)
+    return _offsets(lengths, n)
+
+
+def sipp_prove_native_batch_ragged(A: Points, B: Points, lengths: Sequence[int]) -> List[List[bytes]]:
+    """Independent instances of different sizes, proved in lock-step on the device (sipp_prove_native_batch_ragged): instance j is
+    the next lengths[j] pairs (a power of two) and proofs[j] == sipp_prove_native(A[o[j]:o[j+1]], B[o[j]:o[j+1]]), o = the running
+    sums of `lengths` starting at 0.  A bad point or a zero challenge fails the whole call (SippError) and returns no proof.
+
+    The registration of A and B in each instance's transcript is a device chain of 8 n_j Poseidon permutations, and the longest
+    instance bounds it: an instance far larger than the rest is better proved on its own with sipp_prove_native."""
+    a, b = _flat(A, G1_BYTES), _flat(B, G2_BYTES)
+    n = len(a) // G1_BYTES
+    assert n == len(b) // G2_BYTES, "assert_eq!(A.len(), B.len())"  # prover_native.rs:27
+    offs = _ragged_offsets(lengths, n)
+    count = len(offs) - 1
+    if count == 0:
+        raise ValueError("no instances")
+    _lib.require_gpu_once()
+    lib = _lib.load()
+    plens = [lib.sipp_proof_len(int(length)) for length in lengths]
+    proofs = ctypes.create_string_buffer(FQ12_BYTES * sum(plens))
+    _lib.check(lib.sipp_prove_native_batch_ragged(a, n, b, n, offs, count, proofs))
+    raw, out, pos = proofs.raw, [], 0
+    for plen in plens:
+        out.append(_split(raw[pos:pos + plen * FQ12_BYTES], FQ12_BYTES))
+        pos += plen * FQ12_BYTES
+    return out
+
+
+def sipp_prove_native_batch_ragged_device(dA: int, dB: int, n: int, lengths: Sequence[int], d_proofs: int) -> None:
+    """sipp_prove_native_batch_ragged on DEVICE buffers (integer pointers, e.g. tensor.data_ptr()): dA n x 64 B, dB n x 128 B,
+    d_proofs sum_j (2 log2 lengths[j] + 1) x 384 B, boundary format; instance j's proof follows those of instances 0 .. j - 1"""
+    offs = _ragged_offsets(lengths, n)
+    _lib.require_gpu_once()
+    _lib.check(_lib.load().sipp_prove_native_batch_ragged_device(dA, dB, n, offs, len(offs) - 1, d_proofs))
+
+
 def sipp_verify_native_batch(A: Points, B: Points, n: int, proofs: Sequence[Sequence[bytes]]) -> List[Union[SIPPStatement, VerificationError]]:
     """`count` independent verifications in lock-step (verifier_native.rs:14-85 per instance).  Returns, per instance, the
     SIPPStatement (Ok) or a VerificationError instance (Err) -- a failed instance does not abort the others."""

@@ -5,6 +5,7 @@
 #define SIPP_FQ_CALLS 1
 #include "coop.cuh"
 #include "device_common.cuh"
+#include "fold_map.cuh"
 #include "fold_plan.h"
 #include "fq2h.cuh"
 
@@ -190,19 +191,22 @@ __global__ void __launch_bounds__(SIPP_FOLD_THREADS) k_fold_split(uint32_t* __re
 // Batched instances: the same lane split, but every instance has its own challenge, so the plan is read per element
 // (plans[inst]).  A warp's 32 elements belong to one instance while h >= 32 (uniform digit tests); in the last rounds a warp
 // spans several instances and the digit branches diverge -- those rounds hold 31/127 of an instance's fold work.
-__global__ void __launch_bounds__(SIPP_FOLD_THREADS) k_fold_batch(uint32_t* __restrict__ A, uint32_t* __restrict__ B, size_t h, size_t stride, size_t count,
-                                                                 const FoldPlan* __restrict__ plans, unsigned g2_blocks) {
+// The element mapping is a template parameter (fold_map.cuh): UniformFold for the lock-step batch, RaggedFold for the ragged one.
+template <class Map>
+__device__ __forceinline__ void fold_batch_body(uint32_t* __restrict__ A, uint32_t* __restrict__ B, const Map& map, const FoldPlan* __restrict__ plans,
+                                                unsigned g2_blocks) {
     __shared__ __align__(16) uint32_t xch[3 * 16 * 48];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, el = lane >> 1;
-    const size_t total = count * h;
+    const size_t total = map.total();
     if (blockIdx.x < g2_blocks) {
         // as k_fold_split: 16 elements per block, every Fq2 on a lane pair; pairs of one warp may follow different digit schedules
         // (different instances) -- the pair shuffles of fq2h.cuh name only their own two lanes
         size_t e = (size_t)blockIdx.x * 16 + el;
         const bool valid = e < total;
         if (!valid) e = total - 1;
-        const size_t inst = e / h, i = inst * stride + e % h;
-        const FoldPlan* pl = plans + inst;
+        const FoldElem fe = map.elem(e);
+        const size_t i = fe.i, h = fe.h;
+        const FoldPlan* pl = plans + fe.inst;
         G2A q = endo_apply(load_g2(B, i + h), warp);
         if (pl->g2[warp].neg) q.y = f_neg(q.y);
         Jac<Fq2H> acc = jac_scalar_mul_naf(split_g2(q), pl->g2[warp].plus, pl->g2[warp].minus, pl->g2_bits);
@@ -223,8 +227,9 @@ __global__ void __launch_bounds__(SIPP_FOLD_THREADS) k_fold_batch(uint32_t* __re
         size_t e = (size_t)(blockIdx.x - g2_blocks) * 32 + half * 16 + el;
         const bool valid = e < total;
         if (!valid) e = total - 1;
-        const size_t inst = e / h, i = inst * stride + e % h;
-        const FoldPlan* pl = plans + inst;
+        const FoldElem fe = map.elem(e);
+        const size_t i = fe.i, h = fe.h;
+        const FoldPlan* pl = plans + fe.inst;
         G1A q = endo_apply(load_g1(A, i + h), comp);
         if (pl->g1[comp].neg) q.y = fq_neg(q.y);
         Jac<Fq> acc = jac_scalar_mul_naf_pair(q, pl->g1[comp].plus, pl->g1[comp].minus, pl->g1_bits);
@@ -237,6 +242,14 @@ __global__ void __launch_bounds__(SIPP_FOLD_THREADS) k_fold_batch(uint32_t* __re
         }
     }
 }
+__global__ void __launch_bounds__(SIPP_FOLD_THREADS) k_fold_batch(uint32_t* __restrict__ A, uint32_t* __restrict__ B, size_t h, size_t stride, size_t count,
+                                                                 const FoldPlan* __restrict__ plans, unsigned g2_blocks) {
+    fold_batch_body(A, B, UniformFold{h, stride, count}, plans, g2_blocks);
+}
+__global__ void __launch_bounds__(SIPP_FOLD_THREADS) k_fold_batch_ragged(uint32_t* __restrict__ A, uint32_t* __restrict__ B, const RaggedInst* __restrict__ tab,
+                                                                        unsigned act, size_t elems, const FoldPlan* __restrict__ plans, unsigned g2_blocks) {
+    fold_batch_body(A, B, RaggedFold{tab, act, elems, 0}, plans, g2_blocks);
+}
 
 // ------------------------------------------------------------------------------------------------ K4, throughput form
 // One thread per element, all endomorphism components on ONE accumulator (Straus / Shamir): the 66 (G2) or 128 (G1)
@@ -246,14 +259,16 @@ __global__ void __launch_bounds__(SIPP_FOLD_THREADS) k_fold_batch(uint32_t* __re
 // the GPU: batched instances and the first rounds of a large proof.  plans[inst] as in k_fold_batch (count = 1: one proof).
 #define SIPP_STRAUS_THREADS 64
 
-__global__ void __launch_bounds__(SIPP_STRAUS_THREADS) k_fold_straus(uint32_t* __restrict__ A, uint32_t* __restrict__ B, size_t h, size_t stride, size_t count,
-                                                                   const FoldPlan* __restrict__ plans, unsigned g2_blocks) {
-    const size_t total = count * h;
+template <class Map>
+__device__ __forceinline__ void fold_straus_body(uint32_t* __restrict__ A, uint32_t* __restrict__ B, const Map& map, const FoldPlan* __restrict__ plans,
+                                                 unsigned g2_blocks) {
+    const size_t total = map.total();
     const bool is_g2 = blockIdx.x < g2_blocks;
     size_t e = (size_t)(is_g2 ? blockIdx.x : blockIdx.x - g2_blocks) * SIPP_STRAUS_THREADS + threadIdx.x;
     if (e >= total) return;
-    const size_t inst = e / h, i = inst * stride + e % h;
-    const FoldPlan* pl = plans + inst;
+    const FoldElem fe = map.elem(e);
+    const size_t i = fe.i, h = fe.h;
+    const FoldPlan* pl = plans + fe.inst;
     if (is_g2) {
         G2A tbl[4];
         const G2A p2 = load_g2(B, i + h);
@@ -275,6 +290,14 @@ __global__ void __launch_bounds__(SIPP_STRAUS_THREADS) k_fold_straus(uint32_t* _
         Jac<Fq> acc = straus_naf<Fq, 2>(tbl, pl->g1, pl->g1_bits);
         store_g1(A, i, jac_to_affine(jac_add_affine(acc, load_g1(A, i))));
     }
+}
+__global__ void __launch_bounds__(SIPP_STRAUS_THREADS) k_fold_straus(uint32_t* __restrict__ A, uint32_t* __restrict__ B, size_t h, size_t stride, size_t count,
+                                                                   const FoldPlan* __restrict__ plans, unsigned g2_blocks) {
+    fold_straus_body(A, B, UniformFold{h, stride, count}, plans, g2_blocks);
+}
+__global__ void __launch_bounds__(SIPP_STRAUS_THREADS) k_fold_straus_ragged(uint32_t* __restrict__ A, uint32_t* __restrict__ B, const RaggedInst* __restrict__ tab,
+                                                                          unsigned act, size_t elems, const FoldPlan* __restrict__ plans, unsigned g2_blocks) {
+    fold_straus_body(A, B, RaggedFold{tab, act, elems, 0}, plans, g2_blocks);
 }
 
 // ------------------------------------------------------------------------------------------------ input validation
@@ -338,6 +361,16 @@ int launch_fold_batch(uint32_t* A, uint32_t* B, size_t h, size_t stride, size_t 
     size_t total = count * h;
     unsigned g2_blocks = (unsigned)((total + 15) / 16), g1_blocks = (unsigned)((total + 31) / 32);
     k_fold_batch<<<g2_blocks + g1_blocks, SIPP_FOLD_THREADS, 0, s>>>(A, B, h, stride, count, plans, g2_blocks);
+    return (int)cudaGetLastError();
+}
+int launch_fold_batch_ragged(uint32_t* A, uint32_t* B, const RaggedInst* tab, unsigned act, size_t elems, const FoldPlan* plans, cudaStream_t s) {
+    unsigned g2_blocks = (unsigned)((elems + 15) / 16), g1_blocks = (unsigned)((elems + 31) / 32);
+    k_fold_batch_ragged<<<g2_blocks + g1_blocks, SIPP_FOLD_THREADS, 0, s>>>(A, B, tab, act, elems, plans, g2_blocks);
+    return (int)cudaGetLastError();
+}
+int launch_fold_straus_ragged(uint32_t* A, uint32_t* B, const RaggedInst* tab, unsigned act, size_t elems, const FoldPlan* plans, cudaStream_t s) {
+    unsigned blocks = (unsigned)((elems + SIPP_STRAUS_THREADS - 1) / SIPP_STRAUS_THREADS);
+    k_fold_straus_ragged<<<2 * blocks, SIPP_STRAUS_THREADS, 0, s>>>(A, B, tab, act, elems, plans, blocks);
     return (int)cudaGetLastError();
 }
 int launch_fold_straus(uint32_t* A, uint32_t* B, size_t h, size_t stride, size_t count, const FoldPlan* plans, cudaStream_t s) {

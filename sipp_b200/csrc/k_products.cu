@@ -91,7 +91,54 @@ __global__ void __launch_bounds__(SIPP_ACCUM_THREADS) k_seg_product(const Produc
     if (active_lane && group == 0) store_fq2_words(work + (size_t)t.dst * 96 + k * 16, f);
 }
 
+// ragged batched prover (ragged.cu), rounds >= 1: per active instance (h = current n / 2), gA / gB <- A_hi || A_lo and B_lo || B_hi
+// at pairs [2 estart, 2 estart + 2h), so that Z_L = <A_hi, B_lo> (prover_native.rs:48) and Z_R = <A_lo, B_hi> (:49) are two
+// consecutive segments of the products path.  One thread per 16-byte quarter of a Montgomery point: 4 of A_hi, 4 of A_lo, 8 of
+// B_lo, 8 of B_hi per element.
+#define SIPP_GATHER_QUADS 24
+__global__ void __launch_bounds__(256) k_ragged_gather(const uint32_t* __restrict__ A, const uint32_t* __restrict__ B, const RaggedInst* __restrict__ tab,
+                                                       unsigned act, size_t elems, uint32_t* __restrict__ gA, uint32_t* __restrict__ gB) {
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= elems * SIPP_GATHER_QUADS) return;
+    const size_t e = t / SIPP_GATHER_QUADS;
+    const int q = (int)(t % SIPP_GATHER_QUADS);
+    unsigned lo = 0, hi = act - 1;  // last instance whose elements start at or before e
+    while (lo < hi) {
+        const unsigned mid = (lo + hi + 1) >> 1;
+        if ((size_t)tab[mid].estart <= e) lo = mid; else hi = mid - 1;
+    }
+    const RaggedInst r = tab[lo];
+    const size_t i = e - r.estart, src_lo = (size_t)r.base + i, src_hi = src_lo + r.h;
+    const size_t dst_l = 2 * (size_t)r.estart + i, dst_r = dst_l + r.h;  // Z_L segment, Z_R segment
+    const uint4* sA = reinterpret_cast<const uint4*>(A);
+    const uint4* sB = reinterpret_cast<const uint4*>(B);
+    uint4* dA = reinterpret_cast<uint4*>(gA);
+    uint4* dB = reinterpret_cast<uint4*>(gB);
+    if (q < 4) dA[4 * dst_l + q] = sA[4 * src_hi + q];
+    else if (q < 8) dA[4 * dst_r + q - 4] = sA[4 * src_lo + q - 4];
+    else if (q < 16) dB[8 * dst_l + q - 8] = sB[8 * src_lo + q - 8];
+    else dB[8 * dst_r + q - 16] = sB[8 * src_hi + q - 16];
+}
+
+// proofs[dst[j]] <- res[j]: the products of a round into the proof slots of their instances, 24 quarters of an Fq12 per thread row
+__global__ void __launch_bounds__(256) k_scatter_fq12(const uint32_t* __restrict__ res, const uint64_t* __restrict__ dst, size_t count,
+                                                      uint32_t* __restrict__ proofs) {
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= count * 24) return;
+    const size_t j = t / 24, q = t % 24;
+    reinterpret_cast<uint4*>(proofs)[24 * dst[j] + q] = reinterpret_cast<const uint4*>(res)[24 * j + q];
+}
+
 // ------------------------------------------------------------------------------------------------ launch wrappers
+int launch_ragged_gather(const uint32_t* A, const uint32_t* B, const RaggedInst* tab, unsigned act, size_t elems, uint32_t* gA, uint32_t* gB, cudaStream_t s) {
+    const size_t threads = elems * SIPP_GATHER_QUADS;
+    k_ragged_gather<<<(unsigned)((threads + 255) / 256), 256, 0, s>>>(A, B, tab, act, elems, gA, gB);
+    return (int)cudaGetLastError();
+}
+int launch_scatter_fq12(const uint32_t* res, const uint64_t* dst, size_t count, uint32_t* proofs, cudaStream_t s) {
+    k_scatter_fq12<<<(unsigned)((count * 24 + 255) / 256), 256, 0, s>>>(res, dst, count, proofs);
+    return (int)cudaGetLastError();
+}
 int launch_accum_plan(const uint32_t* lines, const ProductGroup* plan, size_t g0, size_t ngroups, size_t c0, int kpg, uint32_t* partials, cudaStream_t s) {
     const size_t blocks = (ngroups + SIPP_ACCUM_GROUPS - 1) / SIPP_ACCUM_GROUPS;
     k_accum_plan<<<(unsigned)blocks, SIPP_ACCUM_THREADS, 0, s>>>(lines, plan, g0, ngroups, c0, kpg, partials);

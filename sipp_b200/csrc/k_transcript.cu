@@ -131,6 +131,18 @@ __device__ __forceinline__ void load_rc_shared(uint64_t* rc) {
 
 }  // namespace
 
+// register n pairs (prover_native.rs:36-39) on a lane group, from Transcript::new (transcript_native.rs:19-23)
+__device__ __forceinline__ uint64_t absorb_pairs_lanes(const uint32_t* a, const uint32_t* b, size_t n, int l, const uint64_t* rc) {
+    uint64_t s = 0;
+    for (size_t i = 0; i < n; i++) {
+        const uint32_t* pa = a + 16 * i;
+        const uint32_t* pb = b + 32 * i;
+        s = tr_append_lanes(s, l, rc, 16, [&](int k) -> uint64_t { return pa[k]; });  // append_g1  :42-46
+        s = tr_append_lanes(s, l, rc, 32, [&](int k) -> uint64_t { return pb[k]; });  // append_g2  :48-54
+    }
+    return s;
+}
+
 #define SIPP_TR_THREADS 32  // two instances per block: the chains are latency-bound, spread them over the SMs
 
 // 16 lanes per instance: register A and B (prover_native.rs:36-39), 8 permutations per pair
@@ -142,15 +154,22 @@ __global__ void __launch_bounds__(SIPP_TR_THREADS) k_tr_absorb_pairs(const uint3
     size_t inst = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 4;
     const bool have = inst < count;
     if (!have) inst = count - 1;  // shadow: the shuffles need every lane of the warp
-    uint64_t s = 0;  // Transcript::new  transcript_native.rs:19-23
-    const uint32_t* a = bytesA + inst * n * 16;
-    const uint32_t* b = bytesB + inst * n * 32;
-    for (size_t i = 0; i < n; i++) {
-        const uint32_t* pa = a + 16 * i;
-        const uint32_t* pb = b + 32 * i;
-        s = tr_append_lanes(s, l, rc, 16, [&](int k) -> uint64_t { return pa[k]; });  // append_g1  :42-46
-        s = tr_append_lanes(s, l, rc, 32, [&](int k) -> uint64_t { return pb[k]; });  // append_g2  :48-54
-    }
+    const uint64_t s = absorb_pairs_lanes(bytesA + inst * n * 16, bytesB + inst * n * 32, n, l, rc);
+    if (have && l < 4) states[4 * inst + l] = s;
+}
+
+// ragged batch: instance k absorbs pairs [tab[k].base, tab[k].base + 2 tab[k].h) (round 1's table: n_k = 2h).  The chain of an
+// instance is 8 n_k permutations, so the longest instance bounds the launch.
+__global__ void __launch_bounds__(SIPP_TR_THREADS) k_tr_absorb_pairs_ragged(const uint32_t* __restrict__ bytesA, const uint32_t* __restrict__ bytesB,
+                                                                            const RaggedInst* __restrict__ tab, unsigned act, uint64_t* __restrict__ states) {
+    __shared__ uint64_t rc[360];
+    load_rc_shared(rc);
+    const int l = threadIdx.x & 15;
+    size_t inst = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 4;
+    const bool have = inst < act;
+    if (!have) inst = act - 1;
+    const RaggedInst r = tab[inst];
+    const uint64_t s = absorb_pairs_lanes(bytesA + (size_t)r.base * 16, bytesB + (size_t)r.base * 32, 2 * (size_t)r.h, l, rc);
     if (have && l < 4) states[4 * inst + l] = s;
 }
 
@@ -158,17 +177,11 @@ __global__ void __launch_bounds__(SIPP_TR_THREADS) k_tr_absorb_pairs(const uint3
 // inverts it and recodes it.  proofs: [count][np][96 words] boundary bytes; slots index the Fq12 inside an instance's proof
 // (slot_z < 0: skip).  flags[0] |= 1 on a zero challenge (x.inverse().unwrap() panics in the reference), |= 2 on a recoding
 // failure.
-__global__ void __launch_bounds__(SIPP_TR_THREADS) k_tr_round(uint64_t* __restrict__ states, const uint32_t* __restrict__ proofs, size_t np, int slot_z, int slot_l,
-                                                              int slot_r, int order, size_t count, FoldPlan* __restrict__ plans, uint64_t* __restrict__ challenges,
-                                                              int* __restrict__ flags) {
-    __shared__ uint64_t rc[360];
-    load_rc_shared(rc);
-    const int l = threadIdx.x & 15;
-    size_t inst = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 4;
-    const bool have = inst < count;
-    if (!have) inst = count - 1;
+// the round of instance `inst` (pf: its proof) on a lane group
+__device__ __forceinline__ void tr_round_lanes(uint64_t* __restrict__ states, const uint32_t* pf, int slot_z, int slot_l, int slot_r, int order, size_t inst,
+                                               bool have, int l, const uint64_t* rc, FoldPlan* __restrict__ plans, uint64_t* __restrict__ challenges,
+                                               int* __restrict__ flags) {
     uint64_t s = states[4 * inst + (l & 3)];
-    const uint32_t* pf = proofs + inst * np * 96;
     if (slot_z >= 0) s = tr_append_fq12_lanes(s, l, rc, pf + (size_t)slot_z * 96, order);  // prover_native.rs:42-43
     s = tr_append_fq12_lanes(s, l, rc, pf + (size_t)slot_l * 96, order);                    // :52-53
     s = tr_append_fq12_lanes(s, l, rc, pf + (size_t)slot_r * 96, order);                    // :54-55
@@ -212,6 +225,34 @@ __global__ void __launch_bounds__(SIPP_TR_THREADS) k_tr_round(uint64_t* __restri
         if (glv::plan_build(v, vi, device_glv_tables(), &plan)) atomicOr(flags, 2);
     }
     plans[inst] = plan;
+}
+__global__ void __launch_bounds__(SIPP_TR_THREADS) k_tr_round(uint64_t* __restrict__ states, const uint32_t* __restrict__ proofs, size_t np, int slot_z, int slot_l,
+                                                              int slot_r, int order, size_t count, FoldPlan* __restrict__ plans, uint64_t* __restrict__ challenges,
+                                                              int* __restrict__ flags) {
+    __shared__ uint64_t rc[360];
+    load_rc_shared(rc);
+    const int l = threadIdx.x & 15;
+    size_t inst = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 4;
+    const bool have = inst < count;
+    if (!have) inst = count - 1;
+    tr_round_lanes(states, proofs + inst * np * 96, slot_z, slot_l, slot_r, order, inst, have, l, rc, plans, challenges, flags);
+}
+
+// ragged batch, round `round` >= 1 of the active instances k < act: instance k's proof is pt[k] (its own np), its slots those of
+// batch.cu (Z at np - 1, absorbed in round 1 only; Z_L at np - 2 round, Z_R at np - 1 - 2 round)
+__global__ void __launch_bounds__(SIPP_TR_THREADS) k_tr_round_ragged(uint64_t* __restrict__ states, const uint32_t* __restrict__ proofs,
+                                                                     const RaggedProof* __restrict__ pt, int round, int order, unsigned act,
+                                                                     FoldPlan* __restrict__ plans, int* __restrict__ flags) {
+    __shared__ uint64_t rc[360];
+    load_rc_shared(rc);
+    const int l = threadIdx.x & 15;
+    size_t inst = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 4;
+    const bool have = inst < act;
+    if (!have) inst = act - 1;
+    const RaggedProof p = pt[inst];
+    const int np = (int)p.np;
+    tr_round_lanes(states, proofs + p.first * 96, round == 1 ? np - 1 : -1, np - 2 * round, np - 1 - 2 * round, order, inst, have, l, rc, plans, nullptr,
+                   flags);
 }
 
 // test hook: the recoding k_tr_round runs, on given pairs (xs, xinvs: 4 u64 each), one thread per pair; fails counts the pairs
@@ -262,6 +303,20 @@ int launch_tr_round(uint64_t* states, const uint32_t* proofs, size_t np, int slo
     int e = load_rc();
     if (e) return e;
     k_tr_round<<<(unsigned)((count * 16 + SIPP_TR_THREADS - 1) / SIPP_TR_THREADS), SIPP_TR_THREADS, 0, s>>>(states, proofs, np, slot_z, slot_l, slot_r, order, count, plans, challenges, flags);
+    return (int)cudaGetLastError();
+}
+int launch_tr_absorb_pairs_ragged(const uint32_t* bytesA, const uint32_t* bytesB, const RaggedInst* tab, unsigned act, uint64_t* states, cudaStream_t s) {
+    int e = load_rc();
+    if (e) return e;
+    k_tr_absorb_pairs_ragged<<<(unsigned)(((size_t)act * 16 + SIPP_TR_THREADS - 1) / SIPP_TR_THREADS), SIPP_TR_THREADS, 0, s>>>(bytesA, bytesB, tab, act, states);
+    return (int)cudaGetLastError();
+}
+int launch_tr_round_ragged(uint64_t* states, const uint32_t* proofs, const RaggedProof* pt, int round, int order, unsigned act, FoldPlan* plans, int* flags,
+                           cudaStream_t s) {
+    int e = load_rc();
+    if (e) return e;
+    k_tr_round_ragged<<<(unsigned)(((size_t)act * 16 + SIPP_TR_THREADS - 1) / SIPP_TR_THREADS), SIPP_TR_THREADS, 0, s>>>(states, proofs, pt, round, order, act, plans,
+                                                                                                                        flags);
     return (int)cudaGetLastError();
 }
 int launch_test_plan_build(const uint64_t* xs, const uint64_t* xinvs, size_t count, FoldPlan* plans, int* fails, cudaStream_t s) {

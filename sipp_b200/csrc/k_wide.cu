@@ -6,6 +6,7 @@
 // Replaces the per-pair `pairing` calls of /root/reference/src/prover_native.rs:17-22, :48-49 (G2 arithmetic part).
 #include "engine.cuh"
 #include "device_common.cuh"
+#include "fold_map.cuh"
 
 namespace sipp {
 
@@ -238,26 +239,25 @@ __global__ void __launch_bounds__(SIPP_WIDE_THREADS) k_fold_wide(uint32_t* __res
     }
 }
 
-// batched instances: the plan is read per instance (plans[inst]); otherwise as k_fold_wide
-__global__ void __launch_bounds__(SIPP_WIDE_THREADS) k_fold_wide_batch(uint32_t* __restrict__ A, uint32_t* __restrict__ B, size_t h, size_t stride, size_t count,
-                                                                      const FoldPlan* __restrict__ plans, unsigned g2_blocks) {
+// batched instances: the plan is read per instance (plans[inst]); otherwise as k_fold_wide.  The element mapping is a template
+// parameter (fold_map.cuh): UniformFold for the lock-step batch, RaggedFold for the ragged one.
+template <class Map>
+__device__ __forceinline__ void fold_wide_batch_body(uint32_t* __restrict__ A, uint32_t* __restrict__ B, const Map& map, const FoldPlan* __restrict__ plans,
+                                                     unsigned g2_blocks) {
     __shared__ __align__(16) uint32_t smem[SIPP_WIDE_GROUPS * SIPP_LP_SLOTS * 8];
     __shared__ __align__(16) uint32_t xch[SIPP_WIDE_GROUPS * 48];  // one Jacobian point per group (G2: 48 words, G1: 24)
-    // the two groups of a warp must run the same digit schedule: they take two elements of the SAME instance (h even: element pairs
-    // start at even indices), or the same element twice when h is odd (h == 1 in the lock-step prover, whose h is a power of two)
-    const size_t total = count * h;
-    const int epw = (h & 1) ? 1 : 2;
+    // the two groups of a warp must run the same digit schedule: a unit is two elements of the SAME instance (h even: element pairs
+    // start at even indices), or one element taken twice when h is odd (the second group is a shadow that stores nothing)
     const int warp = threadIdx.x >> 5, group = threadIdx.x / SIPP_LP_LANES, lane = threadIdx.x % SIPP_LP_LANES, gi = group & 1;
     uint32_t* slots = smem + group * (SIPP_LP_SLOTS * 8);
     DevMachine mach;
     mach.slots = slots; mach.out = nullptr; mach.lane = lane; mach.store = false; mach.ident = false;
     if (blockIdx.x < g2_blocks) {
         const int comp = warp;                       // 4 warps = 4 GLS components, 2 elements per block
-        size_t E = (size_t)blockIdx.x * epw + (gi % epw);
-        const bool valid = E < total && gi < epw;
-        if (E >= total) E = total - 1;
-        const size_t inst = E / h, e = inst * stride + E % h;
-        const FoldPlan& plan = plans[inst];
+        bool valid;
+        const FoldElem fe = map.unit((size_t)blockIdx.x, gi, valid);
+        const size_t e = fe.i, h = fe.h;
+        const FoldPlan& plan = plans[fe.inst];
         const FoldDigits d = fold_digits(plan.g2[comp], plan.g2_bits);
         bool ident = false;
         if (lane == 0) {
@@ -299,11 +299,10 @@ __global__ void __launch_bounds__(SIPP_WIDE_THREADS) k_fold_wide_batch(uint32_t*
         }
     } else {
         const int comp = warp & 1, pair = warp >> 1;  // warps (0,1) and (2,3): the two GLV components of 2 x 2 elements
-        size_t E = (size_t)(blockIdx.x - g2_blocks) * (2 * epw) + pair * epw + (gi % epw);
-        const bool valid = E < total && gi < epw;
-        if (E >= total) E = total - 1;
-        const size_t inst = E / h, e = inst * stride + E % h;
-        const FoldPlan& plan = plans[inst];
+        bool valid;
+        const FoldElem fe = map.unit((size_t)(blockIdx.x - g2_blocks) * 2 + pair, gi, valid);
+        const size_t e = fe.i, h = fe.h;
+        const FoldPlan& plan = plans[fe.inst];
         const FoldDigits d = fold_digits(plan.g1[comp], plan.g1_bits);
         bool ident = false;
         if (lane == 0) {
@@ -341,8 +340,22 @@ __global__ void __launch_bounds__(SIPP_WIDE_THREADS) k_fold_wide_batch(uint32_t*
         }
     }
 }
+__global__ void __launch_bounds__(SIPP_WIDE_THREADS) k_fold_wide_batch(uint32_t* __restrict__ A, uint32_t* __restrict__ B, size_t h, size_t stride, size_t count,
+                                                                      const FoldPlan* __restrict__ plans, unsigned g2_blocks) {
+    fold_wide_batch_body(A, B, UniformFold{h, stride, count}, plans, g2_blocks);
+}
+__global__ void __launch_bounds__(SIPP_WIDE_THREADS) k_fold_wide_batch_ragged(uint32_t* __restrict__ A, uint32_t* __restrict__ B, const RaggedInst* __restrict__ tab,
+                                                                             unsigned act, size_t elems, size_t units, const FoldPlan* __restrict__ plans,
+                                                                             unsigned g2_blocks) {
+    fold_wide_batch_body(A, B, RaggedFold{tab, act, elems, units}, plans, g2_blocks);
+}
 
-
+int launch_fold_wide_batch_ragged(uint32_t* A, uint32_t* B, const RaggedInst* tab, unsigned act, size_t elems, size_t units, const FoldPlan* plans,
+                                  cudaStream_t s) {
+    const unsigned g2_blocks = (unsigned)units, g1_blocks = (unsigned)((units + 1) / 2);
+    k_fold_wide_batch_ragged<<<g2_blocks + g1_blocks, SIPP_WIDE_THREADS, 0, s>>>(A, B, tab, act, elems, units, plans, g2_blocks);
+    return (int)cudaGetLastError();
+}
 int launch_fold_wide_batch(uint32_t* A, uint32_t* B, size_t h, size_t stride, size_t count, const FoldPlan* plans, cudaStream_t s) {
     const size_t total = count * h, epw = (h & 1) ? 1 : 2;
     const unsigned g2_blocks = (unsigned)((total + epw - 1) / epw), g1_blocks = (unsigned)((total + 2 * epw - 1) / (2 * epw));

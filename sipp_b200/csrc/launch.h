@@ -100,6 +100,29 @@ struct ProductTask {
 int launch_accum_plan(const uint32_t* lines, const ProductGroup* plan, size_t g0, size_t ngroups, size_t c0, int kpg, uint32_t* partials, cudaStream_t s);
 int launch_seg_product(const ProductTask* tasks, size_t ntasks, uint32_t* work, cudaStream_t s);
 
+// ragged batched prover (host driver ragged.cu).  One entry per active instance of a round, in the round's order: its points are
+// [base, base + 2h) of the flat arrays, its fold elements [estart, estart + h) of the round, its wide-fold units start at ustart
+// (h / 2 units of two elements, or one unit when h = 1).  Round 1's table also gives the absorb: pairs [base, base + 2h).
+struct RaggedInst {
+    uint32_t estart, ustart, h, base;
+};
+// proof of an instance: Fq12 slots [first, first + np) of the flat proof buffer
+struct RaggedProof {
+    uint64_t first;
+    uint32_t np, pad;
+};
+int launch_fold_batch_ragged(uint32_t* A, uint32_t* B, const RaggedInst* tab, unsigned act, size_t elems, const FoldPlan* plans, cudaStream_t s);
+int launch_fold_wide_batch_ragged(uint32_t* A, uint32_t* B, const RaggedInst* tab, unsigned act, size_t elems, size_t units, const FoldPlan* plans,
+                                  cudaStream_t s);
+int launch_fold_straus_ragged(uint32_t* A, uint32_t* B, const RaggedInst* tab, unsigned act, size_t elems, const FoldPlan* plans, cudaStream_t s);
+int launch_tr_absorb_pairs_ragged(const uint32_t* bytesA, const uint32_t* bytesB, const RaggedInst* tab, unsigned act, uint64_t* states, cudaStream_t s);
+int launch_tr_round_ragged(uint64_t* states, const uint32_t* proofs, const RaggedProof* pt, int round, int order, unsigned act, FoldPlan* plans, int* flags,
+                           cudaStream_t s);
+// gA / gB <- per active instance A_hi || A_lo and B_lo || B_hi at pairs [2 estart, 2 estart + 2h): Z_L and Z_R as two segments
+int launch_ragged_gather(const uint32_t* A, const uint32_t* B, const RaggedInst* tab, unsigned act, size_t elems, uint32_t* gA, uint32_t* gB, cudaStream_t s);
+// proofs[dst[j]] <- res[j] (Fq12 slots of 96 words)
+int launch_scatter_fq12(const uint32_t* res, const uint64_t* dst, size_t count, uint32_t* proofs, cudaStream_t s);
+
 // BLS input producers (k_bls.cu): group 1 = G1 (16 words per point), 2 = G2 (32 words)
 size_t window_table_bytes(int group);
 int launch_window_table(int group, const uint32_t* base, uint32_t* table, cudaStream_t s);

@@ -12,23 +12,16 @@
 //   final exp.       k_fe_batch_eng / k_fe_batch, one per segment, boundary bytes
 #include <vector>
 
-#include "host_state.h"
+#include "products.h"
 
 using namespace sipp;
 using namespace sipp_host;
 
 namespace {
+void product_tasks(ProductPlan& p, size_t count);
+}  // namespace
 
-// line-table budget of one call: the same as a batched proof's (batch.cu)
-const size_t kProductLinesCap = (size_t)16 << 30;
-
-struct ProductPlan {
-    int kpg = 1;
-    size_t chunk_pairs = 0;                 // pairs per chunk (the last one may be shorter)
-    std::vector<ProductGroup> groups;       // in pair order: segment by segment, chunk by chunk
-    std::vector<size_t> seg_first_group;    // count + 1 entries: the groups of segment j are [seg_first_group[j], seg_first_group[j + 1])
-    std::vector<size_t> chunk_first_group;  // chunks + 1 entries
-};
+namespace sipp_host {
 
 // offsets already checked (products_args)
 int product_plan(const size_t* offsets, size_t count, int kpg_max, size_t chunk_pairs, ProductPlan& p) {
@@ -72,12 +65,58 @@ int product_plan(const size_t* offsets, size_t count, int kpg_max, size_t chunk_
     }
     p.seg_first_group[count] = p.groups.size();
     p.chunk_first_group.push_back(p.groups.size());
+    product_tasks(p, count);
     return SIPP_OK;
 }
 
-// passes of k_seg_product over the work array [group partials | intermediate runs | one product per segment]; returns the slot
+int products_launch(const uint32_t* dA, const uint32_t* dB, size_t n, size_t count, const ProductPlan& plan, const ProductGroup* dgroups,
+                    const ProductTask* dtasks, uint32_t* work, uint32_t* res, cudaStream_t s) {
+    {
+        Span sp(0, s);
+        MillerJob job;
+        job.a_off[0] = job.b_off[0] = job.a_off[1] = job.b_off[1] = 0;
+        job.m = n;
+        for (size_t c = 0; c < plan.chunks(); c++) {
+            const size_t c0 = c * plan.chunk_pairs, cur = n - c0 < plan.chunk_pairs ? n - c0 : plan.chunk_pairs;
+            const size_t g0 = plan.chunk_first_group[c], ng = plan.chunk_first_group[c + 1] - g0;
+            uint32_t* lines = lines_buffer();
+            // 16 lanes per pair for a launch that cannot fill the GPU, one thread per pair otherwise (as ctx_products_to_device)
+            const bool wide = cur <= (size_t)g_opt_wide_max;
+            int le = wide ? launch_lines_wide(dA, dB, job, 1, c0, cur, lines, s) : launch_lines(dA, dB, job, 1, c0, cur, lines, s);
+            if (le) return cuda_fail((cudaError_t)le, "k_lines");
+            le = launch_accum_plan(lines, dgroups, g0, ng, c0, plan.kpg, work, s);
+            if (le) return cuda_fail((cudaError_t)le, "k_accum_plan");
+            g_stats.launches += 2;
+            g_stats.miller_launches++;
+        }
+    }
+    g_stats.miller_pairs += n;
+    {
+        Span sp(1, s);
+        for (size_t k = 0; k + 1 < plan.pass_first.size(); k++) {
+            int le = launch_seg_product(dtasks + plan.pass_first[k], plan.pass_first[k + 1] - plan.pass_first[k], work, s);
+            if (le) return cuda_fail((cudaError_t)le, "k_seg_product");
+            g_stats.launches++;
+        }
+        // one 32-lane machine per product while they all fit the GPU at once, 6-lane groups beyond (as batch_products)
+        const uint32_t* seg = work + plan.seg0 * 96;
+        int le = (g_opt_fe_engine && count <= (size_t)g_sm_count * 12) ? launch_fe_batch_eng(seg, count, 1, 1, res, 96, 0, 0, g_opt_fe_norm, s)
+                                                                       : launch_fe_batch(seg, count, 1, 1, res, 96, 0, 0, g_opt_fe_norm, s);
+        if (le) return cuda_fail((cudaError_t)le, "k_fe_batch");
+        g_stats.launches++;
+    }
+    return SIPP_OK;
+}
+
+}  // namespace sipp_host
+
+namespace {
+
+// passes of k_seg_product over the work array [group partials | intermediate runs | one product per segment]; p.seg0 = the slot
 // of segment 0's product (the `count` products are consecutive)
-size_t product_tasks(const ProductPlan& p, size_t count, std::vector<ProductTask>& tasks, std::vector<size_t>& pass_first) {
+void product_tasks(ProductPlan& p, size_t count) {
+    std::vector<ProductTask>& tasks = p.tasks;
+    std::vector<size_t>& pass_first = p.pass_first;
     std::vector<size_t> start(count), len(count);
     size_t longest = 0;
     for (size_t j = 0; j < count; j++) {
@@ -109,7 +148,7 @@ size_t product_tasks(const ProductPlan& p, size_t count, std::vector<ProductTask
     pass_first.push_back(tasks.size());
     for (size_t j = 0; j < count; j++) tasks.push_back(ProductTask{(uint32_t)start[j], (uint32_t)len[j], (uint32_t)(next + j), 0});
     pass_first.push_back(tasks.size());
-    return next;
+    p.seg0 = next;
 }
 
 int products_args(const void* A, size_t a_len, const void* B, size_t b_len, const size_t* offsets, size_t count, const void* out) {
@@ -130,10 +169,8 @@ int products_run(const uint32_t* bytesA, const uint32_t* bytesB, size_t n, const
     ProductPlan plan;
     int rc = product_plan(offsets, count, g_opt_batch_kpg_max, (size_t)g_opt_product_chunk, plan);
     if (rc) return rc;
-    std::vector<ProductTask> tasks;
-    std::vector<size_t> pass_first;
-    const size_t seg0 = product_tasks(plan, count, tasks, pass_first);
-    const size_t slots = seg0 + count;
+    const std::vector<ProductTask>& tasks = plan.tasks;
+    const size_t slots = plan.work_slots(count);
     uint32_t *dA = nullptr, *dB = nullptr, *work = nullptr, *res = nullptr;
     ProductGroup* dgroups = nullptr;
     ProductTask* dtasks = nullptr;
@@ -166,45 +203,12 @@ int products_run(const uint32_t* bytesA, const uint32_t* bytesB, size_t n, const
                 g_stats.launches++;
             }
         }
-        const size_t chunks = plan.chunk_first_group.size() - 1;
-        if (chunks) {
+        if (plan.chunks()) {
             const int lr = lines_reserve((n < plan.chunk_pairs ? n : plan.chunk_pairs) * lines_bytes_per_pair());
             if (lr) return lr;
         }
-        {
-            Span sp(0, s);
-            MillerJob job;
-            job.a_off[0] = job.b_off[0] = job.a_off[1] = job.b_off[1] = 0;
-            job.m = n;
-            for (size_t c = 0; c < chunks; c++) {
-                const size_t c0 = c * plan.chunk_pairs, cur = n - c0 < plan.chunk_pairs ? n - c0 : plan.chunk_pairs;
-                const size_t g0 = plan.chunk_first_group[c], ng = plan.chunk_first_group[c + 1] - g0;
-                uint32_t* lines = lines_buffer();
-                // 16 lanes per pair for a launch that cannot fill the GPU, one thread per pair otherwise (as ctx_products_to_device)
-                const bool wide = cur <= (size_t)g_opt_wide_max;
-                int le = wide ? launch_lines_wide(dA, dB, job, 1, c0, cur, lines, s) : launch_lines(dA, dB, job, 1, c0, cur, lines, s);
-                if (le) return cuda_fail((cudaError_t)le, "k_lines");
-                le = launch_accum_plan(lines, dgroups, g0, ng, c0, plan.kpg, work, s);
-                if (le) return cuda_fail((cudaError_t)le, "k_accum_plan");
-                g_stats.launches += 2;
-                g_stats.miller_launches++;
-            }
-        }
-        g_stats.miller_pairs += n;
-        {
-            Span sp(1, s);
-            for (size_t k = 0; k + 1 < pass_first.size(); k++) {
-                int le = launch_seg_product(dtasks + pass_first[k], pass_first[k + 1] - pass_first[k], work, s);
-                if (le) return cuda_fail((cudaError_t)le, "k_seg_product");
-                g_stats.launches++;
-            }
-            // one 32-lane machine per product while they all fit the GPU at once, 6-lane groups beyond (as batch_products)
-            const uint32_t* seg = work + seg0 * 96;
-            int le = (g_opt_fe_engine && count <= (size_t)g_sm_count * 12) ? launch_fe_batch_eng(seg, count, 1, 1, res, 96, 0, 0, g_opt_fe_norm, s)
-                                                                           : launch_fe_batch(seg, count, 1, 1, res, 96, 0, 0, g_opt_fe_norm, s);
-            if (le) return cuda_fail((cudaError_t)le, "k_fe_batch");
-            g_stats.launches++;
-        }
+        const int pr = products_launch(dA, dB, n, count, plan, dgroups, dtasks, work, res, s);
+        if (pr) return pr;
         int flag = 0;
         CK(cudaMemcpyAsync(&flag, flags, sizeof(int), cudaMemcpyDeviceToHost, s));
         CK(cudaStreamSynchronize(s));

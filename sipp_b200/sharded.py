@@ -33,6 +33,20 @@ def shard_instances(count: int, rank: int, world: int):
     return lo, lo + base + (1 if rank < extra else 0)
 
 
+def shard_instances_ragged(lengths, rank: int, world: int):
+    """Ragged batches (sipp_prove_native_batch_ragged): rank g proves the contiguous slice [lo, hi) of the instances.  The slices
+    are balanced by the pairs of the products, sum_j (3 n_j - 2), not by instance count: slice g ends at the instance boundary
+    whose running cost is nearest to (g + 1) / world of the total (the first such boundary on a tie)."""
+    prefix = [0]
+    for n in lengths:
+        prefix.append(prefix[-1] + 3 * int(n) - 2)
+
+    def cut(g):
+        target = prefix[-1] * g
+        return min(range(len(prefix)), key=lambda j: (abs(prefix[j] * world - target), j))
+    return cut(rank), cut(rank + 1)
+
+
 def comm_init_nccl(rank: int, world: int, broadcast_bytes) -> None:
     """NCCL communicator inside the library.  `broadcast_bytes(b: Optional[bytes]) -> bytes` ships rank 0's 128-byte unique id
     to every rank over the host's own channel (e.g. `comm_init_torch` below)."""
