@@ -289,11 +289,40 @@ int sipp_prove_native_batch_device(const void *dA, const void *dB, size_t n, siz
  *     longest instance bounds it (about 9.4 us per permutation on the device against 0.61 us on the host): an instance far larger
  *     than the rest is better proved on its own with sipp_prove_native.
  *   - sipp_stats.miller_pairs grows by sum_j (3 n_j - 2), fold_points by sum_j (n_j - 1).
- * Until a ragged verifier exists, verify with sipp_verify_native_batch once per size. */
+ * sipp_verify_native_batch_ragged checks such proofs in one call. */
 int sipp_prove_native_batch_ragged(const uint8_t *A, size_t a_len, const uint8_t *B, size_t b_len, const size_t *offsets, size_t count,
                                    uint8_t *proofs);
 /* the same with A, B and proofs in DEVICE memory (boundary format); offsets stay on the host */
 int sipp_prove_native_batch_ragged_device(const void *dA, const void *dB, size_t n, const size_t *offsets, size_t count, void *d_proofs);
+/* count independent verifications of instances of different sizes, in lock-step (verifier_native.rs:14-85 per instance).  A, B,
+ * offsets: as for sipp_prove_native_batch_ragged, with the same checks in the same order.  proof_offsets: count + 1 HOST entries in
+ * Fq12 units, proof_offsets[0] = 0, never decreasing: proof j is the Fq12 elements [proof_offsets[j], proof_offsets[j+1]) of
+ * `proofs` (384 B each), read from its end like the reference's pop() -- its last element is Z, and only its last sipp_proof_len(n_j)
+ * elements are read, so a longer proof is accepted as by sipp_verify_native.  The running sums of sipp_proof_len(n_j) give exactly
+ * the layout sipp_prove_native_batch_ragged writes.
+ *   results[j] = SIPP_OK for Ok(statement), SIPP_ERR_VERIFY for Err("Verification failed"), SIPP_ERR_ENCODING for a coordinate >= p
+ *   among the elements read: what sipp_verify_native returns on instance j's pairs and proof slice.  One failed instance does not
+ *   affect the others.  For every instance with SIPP_OK or SIPP_ERR_VERIFY, final_A + 64 j, final_B + 128 j and final_Z + 384 j
+ *   (when non-NULL) receive its statement members, byte-identical to sipp_verify_native's, in the caller's order.
+ *   - The return value reports whether the batch ran, not whether the proofs verified.  a_len != b_len: SIPP_ERR_LENGTH.
+ *     SIPP_ERR_ARG: a NULL A, B, offsets, proofs, proof_offsets or results, count == 0, bad offsets (as above), proof_offsets[0] != 0
+ *     or decreasing proof_offsets.  A proof shorter than sipp_proof_len(n_j): SIPP_ERR_SHORT_PROOF (verifier_native.rs:31,40,42).
+ *     All of these are returned before the device is touched; valid arguments without a device give SIPP_ERR_CUDA.
+ *   - a coordinate >= p in A or B, or with SIPP_OPT_VALIDATE_POINTS a point off the curve or a G2 point outside the subgroup, fails
+ *     the whole call with SIPP_ERR_ENCODING, a zero challenge with SIPP_ERR_ZERO_CHALLENGE; in both cases nothing is written to
+ *     `results` or the finals.
+ *   - n_j = 1 gives results[j] = SIPP_OK exactly when pairing(A_i, B_i) == Z.
+ *   - The transcripts are replayed first; then the folds of every round run back to back, and every GT update Z_L^x, Z_R^(1/x) of
+ *     every instance is one independent power in a single launch beside them.  Options read: SIPP_OPT_FE_NORMALISATION,
+ *     SIPP_OPT_FQ12_ORDER, SIPP_OPT_WIDE_LINES_MAX, SIPP_OPT_FE_ENGINE, SIPP_OPT_WIDE_FOLD_MAX, SIPP_OPT_BATCH_KPG_MAX,
+ *     SIPP_OPT_FOLD_STRAUS, SIPP_OPT_VALIDATE_POINTS and SIPP_OPT_PRODUCT_CHUNK_PAIRS.  Not read: SIPP_OPT_PIPELINE,
+ *     SIPP_OPT_BATCH_STREAMS, SIPP_OPT_BATCH_QLINES and the matrix stages (SIPP_OPT_MATRIX_*).
+ *   - As for the prover, the registration of A and B is a device chain of 8 n_j Poseidon permutations per instance, and the longest
+ *     instance bounds the call: an instance far larger than the rest is better verified on its own with sipp_verify_native.
+ *   - sipp_stats.fold_points grows by sum_j (n_j - 1), miller_pairs by count (the final pairings). */
+int sipp_verify_native_batch_ragged(const uint8_t *A, size_t a_len, const uint8_t *B, size_t b_len, const size_t *offsets, size_t count,
+                                    const uint8_t *proofs, const size_t *proof_offsets, int *results, uint8_t *final_A, uint8_t *final_B,
+                                    uint8_t *final_Z);
 
 /* ---- input producers of the BLS-aggregation demo (bin/bls_aggregation.rs:95-117; SURVEY 8f row 3) ---------------------------- */
 /* Scalars are 32-byte little-endian integers < r.  The `_device` forms take DEVICE pointers in the same formats.

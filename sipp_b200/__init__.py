@@ -7,5 +7,6 @@ Poseidon transcript, which the reference also keeps on the host.
 from .api import (ProverContext, SIPPStatement, Transcript, VerificationError, combine_partials, fr_inverse,  # noqa: F401
                   g1_generator_mul_batch, g1_neg_generator, g2_mul_batch, g2_sum, inner_product, inner_product_batch, inner_product_batch_device,
                   pairing, pairing_batch, seeded_inputs, set_option, sipp_prove_native, sipp_prove_native_batch,
-                  sipp_prove_native_batch_ragged, sipp_prove_native_batch_ragged_device, sipp_verify_native, sipp_verify_native_batch, stats)
+                  sipp_prove_native_batch_ragged, sipp_prove_native_batch_ragged_device, sipp_verify_native, sipp_verify_native_batch,
+                  sipp_verify_native_batch_ragged, stats)
 from ._lib import SippError  # noqa: F401

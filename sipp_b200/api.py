@@ -268,6 +268,50 @@ def sipp_verify_native_batch(A: Points, B: Points, n: int, proofs: Sequence[Sequ
     return out
 
 
+def sipp_verify_native_batch_ragged(A: Points, B: Points, lengths: Sequence[int],
+                                    proofs: Sequence[Sequence[bytes]]) -> List[Union[SIPPStatement, VerificationError, SippError]]:
+    """Independent verifications of instances of different sizes in lock-step (sipp_verify_native_batch_ragged): instance j is the
+    next lengths[j] pairs (a power of two) with proof proofs[j] (a list of Fq12 byte strings or one buffer, read from its end), as
+    sipp_prove_native_batch_ragged returns them.  Returns, per instance, what sipp_verify_native gives on it: the SIPPStatement (Ok),
+    a VerificationError instance (Err), or a SippError instance with code ERR_ENCODING for a proof with a coordinate >= p -- a
+    failed instance does not abort the others.  A bad point, a zero challenge or a short proof fails the whole call (SippError).
+
+    As for the prover, the registration of A and B is a device chain of 8 n_j Poseidon permutations per instance and the longest
+    instance bounds it: an instance far larger than the rest is better verified on its own with sipp_verify_native."""
+    a, b = _flat(A, G1_BYTES), _flat(B, G2_BYTES)
+    n = len(a) // G1_BYTES
+    assert n == len(b) // G2_BYTES, "assert_eq!(A.len(), B.len())"
+    offs = _ragged_offsets(lengths, n)
+    count = len(offs) - 1
+    if count == 0:
+        raise ValueError("no instances")
+    if len(proofs) != count:
+        raise ValueError("%d instances but %d proofs" % (count, len(proofs)))
+    flat = [_flat(p, FQ12_BYTES) for p in proofs]
+    poffs = [0]
+    for p in flat:
+        poffs.append(poffs[-1] + len(p) // FQ12_BYTES)
+    _lib.require_gpu_once()
+    res = (ctypes.c_int * count)()
+    fa, fb, fz = (ctypes.create_string_buffer(s * count) for s in (G1_BYTES, G2_BYTES, FQ12_BYTES))
+    _lib.check(_lib.load().sipp_verify_native_batch_ragged(a, n, b, n, offs, count, b"".join(flat), (ctypes.c_size_t * len(poffs))(*poffs), res,
+                                                           fa, fb, fz))
+    out = []
+    for j in range(count):
+        if res[j] == _lib.OK:
+            out.append(SIPPStatement(A=_split(a[G1_BYTES * offs[j]:G1_BYTES * offs[j + 1]], G1_BYTES),
+                                     B=_split(b[G2_BYTES * offs[j]:G2_BYTES * offs[j + 1]], G2_BYTES), Z=flat[j][-FQ12_BYTES:],
+                                     final_A=fa.raw[G1_BYTES * j:G1_BYTES * (j + 1)], final_B=fb.raw[G2_BYTES * j:G2_BYTES * (j + 1)],
+                                     final_Z=fz.raw[FQ12_BYTES * j:FQ12_BYTES * (j + 1)]))
+        elif res[j] == _lib.ERR_VERIFY:
+            out.append(VerificationError("Verification failed"))
+        elif res[j] == _lib.ERR_ENCODING:
+            out.append(SippError(_lib.ERR_ENCODING, "instance %d: proof coordinate >= p" % j))
+        else:
+            out.append(SippError(res[j], "instance %d: unexpected result" % j))
+    return out
+
+
 def sipp_verify_native(A: Points, B: Points, proof: Sequence[bytes]) -> SIPPStatement:
     """verifier_native.rs:14-85; returns the SIPPStatement or raises VerificationError."""
     a, b = _flat(A, G1_BYTES), _flat(B, G2_BYTES)

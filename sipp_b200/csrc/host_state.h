@@ -51,6 +51,7 @@ namespace sipp_host {
 extern int g_device;             // CUDA device of this process, -1 before sipp_init
 extern int g_sm_count;
 extern cudaStream_t g_stream;    // the library's non-blocking stream
+extern cudaStream_t g_fold_stream;  // its side stream (created on first use, sipp_b200.cu)
 #define SIPP_FIRST_STAGE_LOG2_LOOPS 18
 size_t mat_first_budget(size_t n);
 extern int g_opt_pipeline, g_opt_fe_norm, g_opt_fq12_order, g_opt_profile, g_opt_fold_straus, g_opt_batch_kpg_max, g_opt_batch_streams, g_opt_batch_qlines, g_opt_wide_max, g_opt_wide_fold_max, g_opt_fe_engine, g_opt_validate, g_opt_matrix_n, g_opt_matrix_first, g_opt_matrix_block_n, g_opt_matrix_block_r, g_opt_product_chunk;

@@ -290,11 +290,22 @@ __global__ void __launch_bounds__(SIPP_ACCUM_THREADS, 3) k_fe_batch(const uint32
     }
 }
 
+// acc <- acc^(2^254) base^e on a 6-lane group (acc = 1: base^e): generic square-and-multiply over the 254 bits of e (4 u64,
+// little-endian) -- proof elements need not lie in the cyclotomic subgroup, and the reference's `pow` does not assume it -- with
+// the multiplication computed at every bit and selected (groups of one warp hold different exponents).  The accumulator is the
+// caller's: returning it by value costs k_gt_fold_batch 64 bytes of stack frame.
+__device__ __forceinline__ void coop_pow254(const Lane6& L, const Fq2& base, const uint64_t* e, Fq2& acc) {
+#pragma unroll 1
+    for (int i = 253; i >= 0; i--) {
+        acc = coop_sqr(L, acc);
+        const Fq2 m = coop_mul(L, acc, base);
+        acc = select_fq2(((e[i >> 6] >> (i & 63)) & 1ull) != 0, m, acc);
+    }
+}
+
 // Batched verifier GT update (verifier_native.rs:59-61): Z <- Z_L^x * Z * Z_R^(x^-1) for every instance, 6 lanes per power
-// (two groups per instance, both in the same block).  Generic square-and-multiply over the 254 bits of the exponent -- proof
-// elements need not lie in the cyclotomic subgroup, and the reference's `pow` does not assume it -- with the multiplication
-// computed at every bit and selected (groups of one warp hold different exponents).  proofs: [count][stride][96] boundary
-// bytes; challenges: [count][8] u64 = x || x^-1; z: [count][96] boundary bytes, updated in place.
+// (two groups per instance, both in the same block; coop_pow254).  proofs: [count][stride][96] boundary bytes; challenges:
+// [count][8] u64 = x || x^-1; z: [count][96] boundary bytes, updated in place.
 __global__ void __launch_bounds__(SIPP_ACCUM_THREADS) k_gt_fold_batch(const uint32_t* __restrict__ proofs, size_t stride, int slot_l, int slot_r,
                                                                     const uint64_t* __restrict__ challenges, uint32_t* __restrict__ z, size_t count) {
     __shared__ __align__(16) uint32_t xch[SIPP_ACCUM_GROUPS * 96];
@@ -310,14 +321,8 @@ __global__ void __launch_bounds__(SIPP_ACCUM_THREADS) k_gt_fold_batch(const uint
     const int which = (int)(g & 1);
     const int slot = (k & 1) * 3 + (k >> 1);
     const Fq2 base = fq2_decode(proofs + (inst * stride + (size_t)(which ? slot_r : slot_l)) * 96 + 16 * slot);
-    const uint64_t* e = challenges + 8 * inst + 4 * which;
     Fq2 acc = lane_one(k);
-#pragma unroll 1
-    for (int i = 253; i >= 0; i--) {
-        acc = coop_sqr(L, acc);
-        const Fq2 m = coop_mul(L, acc, base);
-        acc = select_fq2(((e[i >> 6] >> (i & 63)) & 1ull) != 0, m, acc);
-    }
+    coop_pow254(L, base, challenges + 8 * inst + 4 * which, acc);
     if (have && which == 1) store_fq2_words(xch + group * 96 + k * 16, acc);
     __syncthreads();
     // group of Z_L (even g; its partner g + 1 is the next group of the same block: 20 groups per block)
@@ -325,6 +330,46 @@ __global__ void __launch_bounds__(SIPP_ACCUM_THREADS) k_gt_fold_batch(const uint
     const Fq2 zc = fq2_decode(z + inst * 96 + 16 * slot);
     const Fq2 r = coop_mul(L, coop_mul(L, acc, zc), zr_pow);
     if (have && which == 0) fq2_encode(z + inst * 96 + 16 * slot, r);
+}
+
+// Ragged batched verifier (ragged.cu): the GT updates of every round of every instance in ONE launch.  The verifier's challenges
+// depend only on A, B and the proof (verifier_native.rs:33-45), so once the transcript has been replayed every Z_L^x, Z_R^(1/x)
+// is an independent power and final_Z = Z * prod_r Z_L(r)^x_r Z_R(r)^(1/x_r) (:59-61 unrolled; exact in GT).  Power entry e
+// (launch.h RaggedGt): two groups in the same block as in k_gt_fold_batch, Z_L at proofs slot src and Z_R at src - 1, exponents
+// challenges[8 e ..] = x || x^-1; their product goes to factors[dst] un-encoded.  The blocks after the powers copy Z of every
+// instance (entries npow ..), decoded, to its factor slot, one thread per Fq2 coefficient.  A segmented product finishes.
+__global__ void __launch_bounds__(SIPP_ACCUM_THREADS) k_gt_fold_ragged(const uint32_t* __restrict__ proofs, const RaggedGt* __restrict__ ent, size_t npow,
+                                                                     size_t nz, const uint64_t* __restrict__ challenges, uint32_t* __restrict__ factors) {
+    __shared__ __align__(16) uint32_t xch[SIPP_ACCUM_GROUPS * 96];
+    const size_t pow_blocks = (2 * npow + SIPP_ACCUM_GROUPS - 1) / SIPP_ACCUM_GROUPS;
+    if (blockIdx.x >= pow_blocks) {  // block-uniform
+        const size_t t = (size_t)(blockIdx.x - pow_blocks) * blockDim.x + threadIdx.x;
+        if (t >= 6 * nz) return;
+        const RaggedGt z = ent[npow + t / 6];
+        const int k = (int)(t % 6), slot = (k & 1) * 3 + (k >> 1);
+        store_fq2_words(factors + (size_t)z.dst * 96 + k * 16, fq2_decode(proofs + z.src * 96 + 16 * slot));
+        return;
+    }
+    const Lane6 L = lane6_of_thread();
+    const int warp = threadIdx.x >> 5;
+    const bool active_lane = L.k < 6;
+    const int group = warp * SIPP_GROUPS_PER_WARP + (active_lane ? L.base / 6 : 0);
+    const int k = active_lane ? L.k : 0;
+    size_t g = (size_t)blockIdx.x * SIPP_ACCUM_GROUPS + group;
+    const bool have = active_lane && g < 2 * npow;
+    if (g >= 2 * npow) g = 2 * npow - 1;
+    const size_t e = g >> 1;
+    const int which = (int)(g & 1);
+    const int slot = (k & 1) * 3 + (k >> 1);
+    const RaggedGt en = ent[e];
+    const Fq2 base = fq2_decode(proofs + (en.src - (uint64_t)which) * 96 + 16 * slot);
+    Fq2 acc = lane_one(k);
+    coop_pow254(L, base, challenges + 8 * e + 4 * which, acc);
+    if (have && which == 1) store_fq2_words(xch + group * 96 + k * 16, acc);
+    __syncthreads();
+    const Fq2 zr_pow = load_fq2_words(xch + (which == 0 && group + 1 < SIPP_ACCUM_GROUPS ? group + 1 : group) * 96 + k * 16);
+    const Fq2 r = coop_mul(L, acc, zr_pow);
+    if (have && which == 0) store_fq2_words(factors + (size_t)en.dst * 96 + k * 16, r);
 }
 
 // ------------------------------------------------------------------------------------------------ test hook
@@ -401,6 +446,12 @@ int launch_gt_fold_batch(const uint32_t* proofs, size_t stride, int slot_l, int 
     size_t groups = 2 * count;
     k_gt_fold_batch<<<(unsigned)((groups + SIPP_ACCUM_GROUPS - 1) / SIPP_ACCUM_GROUPS), SIPP_ACCUM_THREADS, 0, s>>>(proofs, stride, slot_l, slot_r, challenges,
                                                                                                                    z, count);
+    return (int)cudaGetLastError();
+}
+int launch_gt_fold_ragged(const uint32_t* proofs, const RaggedGt* ent, size_t npow, size_t nz, const uint64_t* challenges, uint32_t* factors, cudaStream_t s) {
+    const size_t blocks = (2 * npow + SIPP_ACCUM_GROUPS - 1) / SIPP_ACCUM_GROUPS + (6 * nz + SIPP_ACCUM_THREADS - 1) / SIPP_ACCUM_THREADS;
+    if (blocks == 0) return 0;
+    k_gt_fold_ragged<<<(unsigned)blocks, SIPP_ACCUM_THREADS, 0, s>>>(proofs, ent, npow, nz, challenges, factors);
     return (int)cudaGetLastError();
 }
 int launch_qlines_batch(const uint32_t* B, size_t npoints, uint32_t* qlines, cudaStream_t s) {

@@ -6,6 +6,8 @@
 //   k_seg_product   one pass of the segmented product: every block multiplies a run of at most SIPP_PRODUCT_SPAN consecutive
 //                   Fq12 of one segment (2 per 6-lane group, then the block tree) into one.  The host chains passes until every
 //                   segment is one element, so the depth is logarithmic in the longest segment.  An empty run gives 1.
+//   k_ragged_gather / k_scatter_fq12   the per-round gather and the proof-slot scatter of the ragged batched prover
+//   k_gather_points  the final points of the ragged batched verifier
 #include "accum.cuh"
 #include "device_common.cuh"
 
@@ -129,6 +131,19 @@ __global__ void __launch_bounds__(256) k_scatter_fq12(const uint32_t* __restrict
     reinterpret_cast<uint4*>(proofs)[24 * dst[j] + q] = reinterpret_cast<const uint4*>(res)[24 * j + q];
 }
 
+// ragged batched verifier (ragged.cu): the final A, B of every instance -- its first point once every fold has run
+// (verifier_native.rs:74-75) -- side by side for the final pairings: gA[j] <- A[at[j]], gB[j] <- B[at[j]].  One thread per 16-byte
+// quarter of a Montgomery point: 4 of A, 8 of B per instance.
+__global__ void __launch_bounds__(256) k_gather_points(const uint32_t* __restrict__ A, const uint32_t* __restrict__ B, const uint64_t* __restrict__ at,
+                                                       size_t count, uint32_t* __restrict__ gA, uint32_t* __restrict__ gB) {
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= count * 12) return;
+    const size_t j = t / 12, src = at[j];
+    const int q = (int)(t % 12);
+    if (q < 4) reinterpret_cast<uint4*>(gA)[4 * j + q] = reinterpret_cast<const uint4*>(A)[4 * src + q];
+    else reinterpret_cast<uint4*>(gB)[8 * j + q - 4] = reinterpret_cast<const uint4*>(B)[8 * src + q - 4];
+}
+
 // ------------------------------------------------------------------------------------------------ launch wrappers
 int launch_ragged_gather(const uint32_t* A, const uint32_t* B, const RaggedInst* tab, unsigned act, size_t elems, uint32_t* gA, uint32_t* gB, cudaStream_t s) {
     const size_t threads = elems * SIPP_GATHER_QUADS;
@@ -137,6 +152,10 @@ int launch_ragged_gather(const uint32_t* A, const uint32_t* B, const RaggedInst*
 }
 int launch_scatter_fq12(const uint32_t* res, const uint64_t* dst, size_t count, uint32_t* proofs, cudaStream_t s) {
     k_scatter_fq12<<<(unsigned)((count * 24 + 255) / 256), 256, 0, s>>>(res, dst, count, proofs);
+    return (int)cudaGetLastError();
+}
+int launch_gather_points(const uint32_t* A, const uint32_t* B, const uint64_t* at, size_t count, uint32_t* gA, uint32_t* gB, cudaStream_t s) {
+    k_gather_points<<<(unsigned)((count * 12 + 255) / 256), 256, 0, s>>>(A, B, at, count, gA, gB);
     return (int)cudaGetLastError();
 }
 int launch_accum_plan(const uint32_t* lines, const ProductGroup* plan, size_t g0, size_t ngroups, size_t c0, int kpg, uint32_t* partials, cudaStream_t s) {

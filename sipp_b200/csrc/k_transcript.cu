@@ -239,10 +239,12 @@ __global__ void __launch_bounds__(SIPP_TR_THREADS) k_tr_round(uint64_t* __restri
 }
 
 // ragged batch, round `round` >= 1 of the active instances k < act: instance k's proof is pt[k] (its own np), its slots those of
-// batch.cu (Z at np - 1, absorbed in round 1 only; Z_L at np - 2 round, Z_R at np - 1 - 2 round)
+// batch.cu (Z at np - 1, absorbed in round 1 only; Z_L at np - 2 round, Z_R at np - 1 - 2 round).  challenges (or NULL: the prover)
+// receive x || x^-1 of every instance, for the verifier's GT updates.
 __global__ void __launch_bounds__(SIPP_TR_THREADS) k_tr_round_ragged(uint64_t* __restrict__ states, const uint32_t* __restrict__ proofs,
                                                                      const RaggedProof* __restrict__ pt, int round, int order, unsigned act,
-                                                                     FoldPlan* __restrict__ plans, int* __restrict__ flags) {
+                                                                     FoldPlan* __restrict__ plans, uint64_t* __restrict__ challenges,
+                                                                     int* __restrict__ flags) {
     __shared__ uint64_t rc[360];
     load_rc_shared(rc);
     const int l = threadIdx.x & 15;
@@ -251,7 +253,7 @@ __global__ void __launch_bounds__(SIPP_TR_THREADS) k_tr_round_ragged(uint64_t* _
     if (!have) inst = act - 1;
     const RaggedProof p = pt[inst];
     const int np = (int)p.np;
-    tr_round_lanes(states, proofs + p.first * 96, round == 1 ? np - 1 : -1, np - 2 * round, np - 1 - 2 * round, order, inst, have, l, rc, plans, nullptr,
+    tr_round_lanes(states, proofs + p.first * 96, round == 1 ? np - 1 : -1, np - 2 * round, np - 1 - 2 * round, order, inst, have, l, rc, plans, challenges,
                    flags);
 }
 
@@ -311,12 +313,12 @@ int launch_tr_absorb_pairs_ragged(const uint32_t* bytesA, const uint32_t* bytesB
     k_tr_absorb_pairs_ragged<<<(unsigned)(((size_t)act * 16 + SIPP_TR_THREADS - 1) / SIPP_TR_THREADS), SIPP_TR_THREADS, 0, s>>>(bytesA, bytesB, tab, act, states);
     return (int)cudaGetLastError();
 }
-int launch_tr_round_ragged(uint64_t* states, const uint32_t* proofs, const RaggedProof* pt, int round, int order, unsigned act, FoldPlan* plans, int* flags,
-                           cudaStream_t s) {
+int launch_tr_round_ragged(uint64_t* states, const uint32_t* proofs, const RaggedProof* pt, int round, int order, unsigned act, FoldPlan* plans,
+                           uint64_t* challenges, int* flags, cudaStream_t s) {
     int e = load_rc();
     if (e) return e;
     k_tr_round_ragged<<<(unsigned)(((size_t)act * 16 + SIPP_TR_THREADS - 1) / SIPP_TR_THREADS), SIPP_TR_THREADS, 0, s>>>(states, proofs, pt, round, order, act, plans,
-                                                                                                                        flags);
+                                                                                                                        challenges, flags);
     return (int)cudaGetLastError();
 }
 int launch_test_plan_build(const uint64_t* xs, const uint64_t* xinvs, size_t count, FoldPlan* plans, int* fails, cudaStream_t s) {

@@ -116,12 +116,25 @@ int launch_fold_wide_batch_ragged(uint32_t* A, uint32_t* B, const RaggedInst* ta
                                   cudaStream_t s);
 int launch_fold_straus_ragged(uint32_t* A, uint32_t* B, const RaggedInst* tab, unsigned act, size_t elems, const FoldPlan* plans, cudaStream_t s);
 int launch_tr_absorb_pairs_ragged(const uint32_t* bytesA, const uint32_t* bytesB, const RaggedInst* tab, unsigned act, uint64_t* states, cudaStream_t s);
-int launch_tr_round_ragged(uint64_t* states, const uint32_t* proofs, const RaggedProof* pt, int round, int order, unsigned act, FoldPlan* plans, int* flags,
-                           cudaStream_t s);
+// challenges: NULL, or act x 8 u64 (x || x^-1 of every active instance)
+int launch_tr_round_ragged(uint64_t* states, const uint32_t* proofs, const RaggedProof* pt, int round, int order, unsigned act, FoldPlan* plans,
+                           uint64_t* challenges, int* flags, cudaStream_t s);
 // gA / gB <- per active instance A_hi || A_lo and B_lo || B_hi at pairs [2 estart, 2 estart + 2h): Z_L and Z_R as two segments
 int launch_ragged_gather(const uint32_t* A, const uint32_t* B, const RaggedInst* tab, unsigned act, size_t elems, uint32_t* gA, uint32_t* gB, cudaStream_t s);
 // proofs[dst[j]] <- res[j] (Fq12 slots of 96 words)
 int launch_scatter_fq12(const uint32_t* res, const uint64_t* dst, size_t count, uint32_t* proofs, cudaStream_t s);
+
+// ragged batched verifier (host driver ragged.cu).  A GT entry: a power entry e reads Z_L at Fq12 slot `src` of the proofs and Z_R at
+// src - 1, with challenges[8 e .. 8 e + 8) = x || x^-1, and writes Z_L^x Z_R^(1/x) to factor slot `dst`; a Z entry copies the Fq12 at
+// `src` (decoded) to factor slot `dst`.  Factor slots are Fq12 of 96 words in the layout of k_seg_product.
+struct RaggedGt {
+    uint64_t src;
+    uint32_t dst, pad;
+};
+// entries [0, npow) are powers, [npow, npow + nz) Z copies
+int launch_gt_fold_ragged(const uint32_t* proofs, const RaggedGt* ent, size_t npow, size_t nz, const uint64_t* challenges, uint32_t* factors, cudaStream_t s);
+// gA[j] <- A[at[j]], gB[j] <- B[at[j]] (decoded points), j < count
+int launch_gather_points(const uint32_t* A, const uint32_t* B, const uint64_t* at, size_t count, uint32_t* gA, uint32_t* gB, cudaStream_t s);
 
 // BLS input producers (k_bls.cu): group 1 = G1 (16 words per point), 2 = G2 (32 words)
 size_t window_table_bytes(int group);
