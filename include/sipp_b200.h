@@ -239,6 +239,27 @@ int sipp_ctx_prove(sipp_ctx *ctx, const uint8_t *A, const uint8_t *B, uint8_t *p
  * final_A[64], final_B[128], final_Z[384] when non-NULL (A, B, Z are the caller's own inputs: statements.rs:80-88) */
 int sipp_verify_native(const uint8_t *A, size_t a_len, const uint8_t *B, size_t b_len, const uint8_t *proof, size_t proof_len,
                        uint8_t *final_A, uint8_t *final_B, uint8_t *final_Z);
+/* Proof and statement in one call: sipp_prove_native, plus the statement members that sipp_verify_native would write for
+ * (A, B, proof) -- final_A[64], final_B[128], final_Z[384], byte-identical -- without a verification pass.  The proof bytes are those
+ * of sipp_prove_native.  final_A / final_B are the points folded down to one (verifier_native.rs:74-75) and final_Z, which the
+ * verifier computes as Z prod Z_L^x Z_R^(1/x) (:59-61), is pairing(final_A, final_B) by bilinearity: the output satisfies
+ * pairing(final_A, final_B) == final_Z by construction, under either SIPP_OPT_FE_NORMALISATION, so the call returns SIPP_OK
+ * exactly where sipp_verify_native on its proof returns Ok(statement).  The statement's A, B and Z are the caller's inputs and the
+ * proof's last element.
+ *   - Each of final_A, final_B, final_Z may be NULL; that member is then not written (nor computed where skipping is free).
+ *   - Argument checks, their order and codes are those of sipp_prove_native, all before the device is touched; valid arguments
+ *     without a device give SIPP_ERR_CUDA.  A bad point (SIPP_ERR_ENCODING) or a zero challenge (SIPP_ERR_ZERO_CHALLENGE) fails the
+ *     call, and then nothing is written to `proof` or to any final buffer.
+ *   - Options: those of sipp_prove_native; every value gives the same bytes.  With a pairing-matrix tail stage (the defaults) the
+ *     tail keeps folding the points on the side stream and final_Z is its 1 x 1 matrix after the last round; without one
+ *     (SIPP_OPT_MATRIX_TAIL = 0, SIPP_OPT_PIPELINE = 0 or SIPP_OPT_FE_ENGINE = 0) final_Z is one pairing of the folded points.
+ *     n = 1: final_A = A, final_B = B, final_Z = Z.
+ *   - sipp_stats: miller_pairs and fold_points grow exactly as for sipp_prove_native, plus miller_pairs by 1 when n >= 2, final_Z
+ *     is non-NULL and no tail stage ran (the pairing of the folded points).  launches grows by more than for sipp_prove_native
+ *     (the tail's point folds, the last matrix fold and its encode, the encodes of final_A and final_B); that count is not part of
+ *     the contract. */
+int sipp_prove_native_statement(const uint8_t *A, size_t a_len, const uint8_t *B, size_t b_len, uint8_t *proof,
+                                uint8_t *final_A, uint8_t *final_B, uint8_t *final_Z);
 
 /* ---- witness hand-off to the untouched circuit side (host only, no GPU) --------------------------------------------------- */
 /* The u32 public-input vector of a SIPPStatement: what `SIPPStatement::from_vec` parses (statements.rs:133-170) and the verifier
@@ -268,6 +289,23 @@ int sipp_verify_native_batch(const uint8_t *A, const uint8_t *B, size_t n, size_
                              int *results, uint8_t *final_A, uint8_t *final_B, uint8_t *final_Z);
 /* same with DEVICE buffers in boundary format (inputs resident in HBM, proofs left in HBM) */
 int sipp_prove_native_batch_device(const void *dA, const void *dB, size_t n, size_t count, void *d_proofs);
+/* sipp_prove_native_batch plus every instance's statement members, as sipp_prove_native_statement gives them for one instance:
+ * final_A (count x 64 B), final_B (count x 128 B), final_Z (count x 384 B), byte-identical to sipp_verify_native on
+ * (A_j, B_j, proof_j), each may be NULL.  No verification is performed; pairing(final_A, final_B) == final_Z by construction.
+ *   - The proofs are those of sipp_prove_native_batch.  Argument checks and codes as for it (a NULL A, B or proofs, count == 0, n
+ *     not a non-zero power of two: SIPP_ERR_ARG), all before the device is touched, and valid arguments without a device give
+ *     SIPP_ERR_CUDA.  One difference: sipp_prove_native_batch initialises the device first, so without a device it returns
+ *     SIPP_ERR_CUDA for bad arguments too, where this call returns SIPP_ERR_ARG.  A bad point or a zero challenge fails the whole
+ *     call, and then nothing is written to the proofs or the finals.  Options: those of sipp_prove_native_batch.
+ *   - After the last round every instance's first point is its final point; final_Z is one batched one-pair product per instance
+ *     (the last step of sipp_verify_native_batch).  sipp_stats: miller_pairs and fold_points grow exactly as for
+ *     sipp_prove_native_batch, plus miller_pairs by count when final_Z is non-NULL; launches grows by more (not part of the
+ *     contract). */
+int sipp_prove_native_batch_statement(const uint8_t *A, const uint8_t *B, size_t n, size_t count, uint8_t *proofs,
+                                      uint8_t *final_A, uint8_t *final_B, uint8_t *final_Z);
+/* the same with A, B, proofs and the finals in DEVICE memory (boundary format) */
+int sipp_prove_native_batch_statement_device(const void *dA, const void *dB, size_t n, size_t count, void *d_proofs,
+                                             void *d_final_A, void *d_final_B, void *d_final_Z);
 
 /* ---- batched instances of different sizes: `count` independent proofs in lock-step, each with its own n ------------------- */
 /* count independent proofs of instances of different sizes, in lock-step.  Instance j = pairs [offsets[j], offsets[j+1]) of A and B;
@@ -294,6 +332,20 @@ int sipp_prove_native_batch_ragged(const uint8_t *A, size_t a_len, const uint8_t
                                    uint8_t *proofs);
 /* the same with A, B and proofs in DEVICE memory (boundary format); offsets stay on the host */
 int sipp_prove_native_batch_ragged_device(const void *dA, const void *dB, size_t n, const size_t *offsets, size_t count, void *d_proofs);
+/* sipp_prove_native_batch_ragged plus every instance's statement members, in the caller's instance order: final_A + 64 j,
+ * final_B + 128 j, final_Z + 384 j, byte-identical to sipp_verify_native on (A_j, B_j, proof_j), each may be NULL.  No verification
+ * is performed; pairing(final_A, final_B) == final_Z by construction.
+ *   - The proofs are those of sipp_prove_native_batch_ragged.  Argument checks, their order and codes as for it, all before the
+ *     device is touched (valid arguments without a device: SIPP_ERR_CUDA).  A bad point or a zero challenge fails the whole call,
+ *     and then nothing is written to the proofs or the finals.  Options: those of sipp_prove_native_batch_ragged.
+ *   - After the last round the final points are gathered and paired as sipp_verify_native_batch_ragged does: one batched one-pair
+ *     product per instance.  sipp_stats: miller_pairs and fold_points grow exactly as for sipp_prove_native_batch_ragged, plus
+ *     miller_pairs by count when final_Z is non-NULL; launches grows by more (not part of the contract). */
+int sipp_prove_native_batch_ragged_statement(const uint8_t *A, size_t a_len, const uint8_t *B, size_t b_len, const size_t *offsets,
+                                             size_t count, uint8_t *proofs, uint8_t *final_A, uint8_t *final_B, uint8_t *final_Z);
+/* the same with A, B, proofs and the finals in DEVICE memory (boundary format); offsets stay on the host */
+int sipp_prove_native_batch_ragged_statement_device(const void *dA, const void *dB, size_t n, const size_t *offsets, size_t count,
+                                                    void *d_proofs, void *d_final_A, void *d_final_B, void *d_final_Z);
 /* count independent verifications of instances of different sizes, in lock-step (verifier_native.rs:14-85 per instance).  A, B,
  * offsets: as for sipp_prove_native_batch_ragged, with the same checks in the same order.  proof_offsets: count + 1 HOST entries in
  * Fq12 units, proof_offsets[0] = 0, never decreasing: proof j is the Fq12 elements [proof_offsets[j], proof_offsets[j+1]) of

@@ -14,7 +14,7 @@ Values are arkworks canonical little-endian bytes (see include/sipp_b200.h): a G
 """
 import ctypes
 from dataclasses import dataclass
-from typing import List, Sequence, Union
+from typing import List, Sequence, Tuple, Union
 
 from . import _lib
 from ._lib import SippError
@@ -237,6 +237,95 @@ def sipp_prove_native_batch_ragged_device(dA: int, dB: int, n: int, lengths: Seq
     offs = _ragged_offsets(lengths, n)
     _lib.require_gpu_once()
     _lib.check(_lib.load().sipp_prove_native_batch_ragged_device(dA, dB, n, offs, len(offs) - 1, d_proofs))
+
+
+def _statements(a: bytes, b: bytes, offs: Sequence[int], proofs: List[List[bytes]], fa, fb, fz) -> List[Tuple[List[bytes], SIPPStatement]]:
+    """(proof, SIPPStatement) per instance j = pairs [offs[j], offs[j + 1]), the finals at index j of the C buffers"""
+    return [(p, SIPPStatement(A=_split(a[G1_BYTES * offs[j]:G1_BYTES * offs[j + 1]], G1_BYTES), B=_split(b[G2_BYTES * offs[j]:G2_BYTES * offs[j + 1]], G2_BYTES),
+                              Z=p[-1], final_A=fa.raw[G1_BYTES * j:G1_BYTES * (j + 1)], final_B=fb.raw[G2_BYTES * j:G2_BYTES * (j + 1)],
+                              final_Z=fz.raw[FQ12_BYTES * j:FQ12_BYTES * (j + 1)])) for j, p in enumerate(proofs)]
+
+
+def sipp_prove_native_statement(A: Points, B: Points) -> Tuple[List[bytes], SIPPStatement]:
+    """sipp_prove_native and, from the same call, the SIPPStatement sipp_verify_native returns for that proof (field for field, so
+    to_vec() gives the same circuit vector) without a verification pass (sipp_prove_native_statement)."""
+    a, b = _flat(A, G1_BYTES), _flat(B, G2_BYTES)
+    na, nb = len(a) // G1_BYTES, len(b) // G2_BYTES
+    assert na == nb, "assert_eq!(A.len(), B.len())"  # prover_native.rs:27
+    _lib.require_gpu_once()
+    lib = _lib.load()
+    plen = lib.sipp_proof_len(na)
+    if plen == 0:
+        raise SippError(_lib.ERR_ARG, "n must be a non-zero power of two")
+    proof = ctypes.create_string_buffer(FQ12_BYTES * plen)
+    fa, fb, fz = (ctypes.create_string_buffer(k) for k in (G1_BYTES, G2_BYTES, FQ12_BYTES))
+    _lib.check(lib.sipp_prove_native_statement(a, na, b, nb, proof, fa, fb, fz))
+    return _statements(a, b, [0, na], [_split(proof.raw, FQ12_BYTES)], fa, fb, fz)[0]
+
+
+def sipp_prove_native_batch_statement(A: Points, B: Points, n: int) -> List[Tuple[List[bytes], SIPPStatement]]:
+    """sipp_prove_native_batch with every instance's SIPPStatement, as sipp_verify_native returns it, from the same call
+    (sipp_prove_native_batch_statement): [(proof_j, statement_j)]"""
+    a, b = _flat(A, G1_BYTES), _flat(B, G2_BYTES)
+    na, nb = len(a) // G1_BYTES, len(b) // G2_BYTES
+    assert na == nb, "assert_eq!(A.len(), B.len())"  # prover_native.rs:27
+    if n <= 0 or na % n or na == 0:
+        raise ValueError("the number of pairs (%d) is not a non-zero multiple of the instance size %d" % (na, n))
+    count = na // n
+    _lib.require_gpu_once()
+    lib = _lib.load()
+    plen = lib.sipp_proof_len(n)
+    if plen == 0:
+        raise SippError(_lib.ERR_ARG, "n must be a non-zero power of two")
+    proofs = ctypes.create_string_buffer(FQ12_BYTES * plen * count)
+    fa, fb, fz = (ctypes.create_string_buffer(k * count) for k in (G1_BYTES, G2_BYTES, FQ12_BYTES))
+    _lib.check(lib.sipp_prove_native_batch_statement(a, b, n, count, proofs, fa, fb, fz))
+    raw = proofs.raw
+    ps = [_split(raw[j * plen * FQ12_BYTES:(j + 1) * plen * FQ12_BYTES], FQ12_BYTES) for j in range(count)]
+    return _statements(a, b, [n * j for j in range(count + 1)], ps, fa, fb, fz)
+
+
+def sipp_prove_native_batch_statement_device(dA: int, dB: int, n: int, count: int, d_proofs: int, d_final_A: int, d_final_B: int,
+                                             d_final_Z: int) -> None:
+    """sipp_prove_native_batch_statement on DEVICE buffers (integer pointers, e.g. tensor.data_ptr(); 0 for a final not wanted): dA
+    n count x 64 B, dB n count x 128 B, d_proofs count x (2 log2 n + 1) x 384 B, d_final_A / _B / _Z count x 64 / 128 / 384 B"""
+    _lib.require_gpu_once()
+    _lib.check(_lib.load().sipp_prove_native_batch_statement_device(dA, dB, n, count, d_proofs, d_final_A or None, d_final_B or None,
+                                                                    d_final_Z or None))
+
+
+def sipp_prove_native_batch_ragged_statement(A: Points, B: Points, lengths: Sequence[int]) -> List[Tuple[List[bytes], SIPPStatement]]:
+    """sipp_prove_native_batch_ragged with every instance's SIPPStatement, as sipp_verify_native returns it, from the same call
+    (sipp_prove_native_batch_ragged_statement): [(proof_j, statement_j)] in the caller's order.  A bad point or a zero challenge fails
+    the whole call (SippError)."""
+    a, b = _flat(A, G1_BYTES), _flat(B, G2_BYTES)
+    n = len(a) // G1_BYTES
+    assert n == len(b) // G2_BYTES, "assert_eq!(A.len(), B.len())"  # prover_native.rs:27
+    offs = _ragged_offsets(lengths, n)
+    count = len(offs) - 1
+    if count == 0:
+        raise ValueError("no instances")
+    _lib.require_gpu_once()
+    lib = _lib.load()
+    plens = [lib.sipp_proof_len(int(length)) for length in lengths]
+    proofs = ctypes.create_string_buffer(FQ12_BYTES * sum(plens))
+    fa, fb, fz = (ctypes.create_string_buffer(k * count) for k in (G1_BYTES, G2_BYTES, FQ12_BYTES))
+    _lib.check(lib.sipp_prove_native_batch_ragged_statement(a, n, b, n, offs, count, proofs, fa, fb, fz))
+    raw, ps, pos = proofs.raw, [], 0
+    for plen in plens:
+        ps.append(_split(raw[pos:pos + plen * FQ12_BYTES], FQ12_BYTES))
+        pos += plen * FQ12_BYTES
+    return _statements(a, b, list(offs), ps, fa, fb, fz)
+
+
+def sipp_prove_native_batch_ragged_statement_device(dA: int, dB: int, n: int, lengths: Sequence[int], d_proofs: int, d_final_A: int,
+                                                    d_final_B: int, d_final_Z: int) -> None:
+    """sipp_prove_native_batch_ragged_statement on DEVICE buffers (integer pointers; 0 for a final not wanted): dA, dB, d_proofs as
+    for sipp_prove_native_batch_ragged_device, d_final_A / _B / _Z len(lengths) x 64 / 128 / 384 B in the caller's order"""
+    offs = _ragged_offsets(lengths, n)
+    _lib.require_gpu_once()
+    _lib.check(_lib.load().sipp_prove_native_batch_ragged_statement_device(dA, dB, n, offs, len(offs) - 1, d_proofs, d_final_A or None,
+                                                                           d_final_B or None, d_final_Z or None))
 
 
 def sipp_verify_native_batch(A: Points, B: Points, n: int, proofs: Sequence[Sequence[bytes]]) -> List[Union[SIPPStatement, VerificationError]]:

@@ -300,6 +300,27 @@ int batch_check_flags(const BatchBuffers& b, cudaStream_t s) {
     return SIPP_OK;
 }
 
+// The statement members of every instance once its points are folded to one, A[0] and B[0] (verifier_native.rs:74-75): to `pair`
+// (when non-NULL) pairing(final_A, final_B) of every instance (:80; count x 384 B, encoded), to `fin` (when non-NULL) final_A
+// (count x 64 B) then final_B (count x 128 B), encoded.  Reuses b.bytesA / b.bytesB, which the rounds no longer read.
+int batch_finals(const BatchBuffers& b, size_t n, size_t count, uint32_t* pair, uint32_t* fin, cudaStream_t s) {
+    if (pair) {
+        int rc = lines_reserve(count * lines_bytes_per_pair());
+        if (rc) return rc;
+        rc = batch_products(b, n, count, 1, 0, pair, 1, 0, 0, lines_buffer(), count * lines_bytes_per_pair(), nullptr, s);
+        if (rc) return rc;
+    }
+    if (fin) {
+        CK(cudaMemcpy2DAsync(b.bytesA, 64, b.dA, n * 64, 64, count, cudaMemcpyDeviceToDevice, s));
+        CK(cudaMemcpy2DAsync(b.bytesB, 128, b.dB, n * 128, 128, count, cudaMemcpyDeviceToDevice, s));
+        int le = launch_codec_encode(b.bytesA, fin, count * 2, s);
+        if (!le) le = launch_codec_encode(b.bytesB, fin + count * 16, count * 4, s);
+        if (le) return cuda_fail((cudaError_t)le, "batch finals: encode");
+        g_stats.launches += 2;
+    }
+    return SIPP_OK;
+}
+
 int batch_args(const void* A, const void* B, size_t n, size_t count, const void* proofs) {
     if (!A || !B || !proofs || count == 0) return fail(SIPP_ERR_ARG, "null pointer or count == 0");
     if (!is_pow2(n)) return fail(SIPP_ERR_ARG, "n must be a non-zero power of two");
@@ -354,6 +375,55 @@ int sipp_prove_native_batch(const uint8_t* A, const uint8_t* B, size_t n, size_t
     else cudaStreamSynchronize(g_stream);
     b.release();
     return rc;
+}
+
+// sipp_prove_native_batch(_device) plus every instance's statement members (verifier_native.rs:74-75, :59-61): after the last round
+// the first point of every instance is its final point, and final_Z = pairing(final_A, final_B) by bilinearity.  Nothing is copied
+// to the caller before the flags passed.  in_kind / out_kind: the copies of the inputs and of every output.
+static int batch_prove_statement(const void* A, const void* B, size_t n, size_t count, void* proofs, void* final_A, void* final_B, void* final_Z,
+                                 cudaMemcpyKind in_kind, cudaMemcpyKind out_kind) {
+    int rc = batch_args(A, B, n, count, proofs);  // the checks of sipp_prove_native_batch, before the device is touched
+    if (rc) return rc;
+    rc = ensure_init();
+    if (rc) return rc;
+    const size_t np = sipp_proof_len(n);
+    BatchBuffers b;
+    rc = batch_alloc(b, n, count);
+    if (rc) return rc;
+    uint32_t *dpair = nullptr, *dfin = nullptr;
+    cudaError_t e = final_Z ? pool_alloc((void**)&dpair, count * 384) : cudaSuccess;
+    if (e == cudaSuccess && (final_A || final_B)) e = pool_alloc((void**)&dfin, count * 192);
+    auto run = [&]() -> int {
+        if (e != cudaSuccess) return cuda_fail(e, "cudaMalloc(batch statement)");
+        CK(cudaMemcpyAsync(b.bytesA, A, n * count * 64, in_kind, g_stream));
+        CK(cudaMemcpyAsync(b.bytesB, B, n * count * 128, in_kind, g_stream));
+        int rc2 = batch_prove_resident(b, n, count, g_stream);
+        if (!rc2) rc2 = batch_finals(b, n, count, dpair, dfin, g_stream);
+        if (!rc2) rc2 = batch_check_flags(b, g_stream);
+        if (rc2) return rc2;
+        CK(cudaMemcpyAsync(proofs, b.proofs, count * np * 384, out_kind, g_stream));
+        if (final_A) CK(cudaMemcpyAsync(final_A, dfin, count * 64, out_kind, g_stream));
+        if (final_B) CK(cudaMemcpyAsync(final_B, dfin + count * 16, count * 128, out_kind, g_stream));
+        if (final_Z) CK(cudaMemcpyAsync(final_Z, dpair, count * 384, out_kind, g_stream));
+        CK(cudaStreamSynchronize(g_stream));
+        return SIPP_OK;
+    };
+    rc = run();
+    if (rc) cudaStreamSynchronize(g_stream);
+    b.release();
+    pool_free(dpair);
+    pool_free(dfin);
+    return rc;
+}
+
+int sipp_prove_native_batch_statement(const uint8_t* A, const uint8_t* B, size_t n, size_t count, uint8_t* proofs, uint8_t* final_A,
+                                      uint8_t* final_B, uint8_t* final_Z) {
+    return batch_prove_statement(A, B, n, count, proofs, final_A, final_B, final_Z, cudaMemcpyHostToDevice, cudaMemcpyDeviceToHost);
+}
+
+int sipp_prove_native_batch_statement_device(const void* dA, const void* dB, size_t n, size_t count, void* d_proofs, void* d_final_A,
+                                             void* d_final_B, void* d_final_Z) {
+    return batch_prove_statement(dA, dB, n, count, d_proofs, d_final_A, d_final_B, d_final_Z, cudaMemcpyDeviceToDevice, cudaMemcpyDeviceToDevice);
 }
 
 // `count` independent verifications in lock-step (verifier_native.rs:14-85 per instance): the transcript replay, the folds and the
@@ -420,21 +490,10 @@ int sipp_verify_native_batch(const uint8_t* A, const uint8_t* B, size_t n, size_
             m /= 2;
             round++;
         }
-        // pairing(final_A, final_B) == final_Z   :80   (final_A = A[0], final_B = B[0] of every instance  :74-75)
-        int rc2 = lines_reserve(count * lines_bytes_per_pair());
+        int rc2 = batch_finals(b, n, count, dpair, (final_A || final_B) ? dfin : nullptr, s);   // :74-75, :80
         if (rc2) return rc2;
-        rc2 = batch_products(b, n, count, 1, 0, dpair, 1, 0, 0, lines_buffer(), count * lines_bytes_per_pair(), nullptr, s);
-        if (rc2) return rc2;
-        if (final_A || final_B) {
-            CK(cudaMemcpy2DAsync(b.bytesA, 64, b.dA, n * 64, 64, count, cudaMemcpyDeviceToDevice, s));
-            CK(cudaMemcpy2DAsync(b.bytesB, 128, b.dB, n * 128, 128, count, cudaMemcpyDeviceToDevice, s));
-            le = launch_codec_encode(b.bytesA, dfin, count * 2, s);
-            if (!le) le = launch_codec_encode(b.bytesB, dfin + count * 16, count * 4, s);
-            if (le) return cuda_fail((cudaError_t)le, "verify batch: encode");
-            g_stats.launches += 2;
-            if (final_A) CK(cudaMemcpyAsync(final_A, dfin, count * 64, cudaMemcpyDeviceToHost, s));
-            if (final_B) CK(cudaMemcpyAsync(final_B, dfin + count * 16, count * 128, cudaMemcpyDeviceToHost, s));
-        }
+        if (final_A) CK(cudaMemcpyAsync(final_A, dfin, count * 64, cudaMemcpyDeviceToHost, s));
+        if (final_B) CK(cudaMemcpyAsync(final_B, dfin + count * 16, count * 128, cudaMemcpyDeviceToHost, s));
         CK(cudaMemcpyAsync(hz.data(), dz, count * 384, cudaMemcpyDeviceToHost, s));
         CK(cudaMemcpyAsync(hp.data(), dpair, count * 384, cudaMemcpyDeviceToHost, s));
         return batch_check_flags(b, s);

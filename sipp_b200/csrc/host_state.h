@@ -41,6 +41,11 @@ struct sipp_ctx {
     size_t n = 0, cap = 0;
     bool stages = false;     // sipp_ctx_set_stages: products / folds may run on pairing-matrix stages
     bool stale = false;      // a tail stage ran: the points were not folded any more (sipp_ctx_read refuses)
+    // sipp_prove_native_statement only: a tail stage keeps folding the points (side stream) and its matrix diagonal, and its last
+    // round leaves the 1 x 1 matrix <final_A, final_B> in final_z (encoded)
+    bool keep_points = false;
+    bool has_final_z = false;
+    uint8_t final_z[384];
     bool pending_validation = false;  // the on-curve / subgroup check of these points is still running on the side stream
     cudaEvent_t validated = nullptr;
     sipp_host::MatTail mt;

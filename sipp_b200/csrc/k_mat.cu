@@ -79,19 +79,20 @@ int launch_mat_diag(const uint32_t* E, size_t n, int main_diagonal, uint32_t* pa
     return (int)cudaGetLastError();
 }
 
-// k_mat_fold: one block per entry (i, j), i != j, of the folded matrix; 8 machines = 2 exponents x 4 Frobenius components.
+// k_mat_fold: one block per entry (i, j), i != j (all entries with `diag`), of the folded matrix; 8 machines = 2 exponents x 4 Frobenius components.
 //   machine w < 4:  (frob^w E[i+h][j])^(k_w of x)        machine 4 + w:  (frob^w E[i][j+h])^(k_w of x^-1)
 // then machine 0 multiplies E[i][j] in, machine 4 E[i+h][j+h], and a tree product over the eight leaves the entry in machine 0.
-// The diagonal is never read by a later round (Z_L, Z_R use |i - j| = h / 2 and folds keep i - j modulo h), so it is skipped.
+// The diagonal is never read by a later round (Z_L, Z_R use |i - j| = h / 2 and folds keep i - j modulo h), so it is skipped, unless
+// `diag`: the statement prover reads the 1 x 1 matrix after the last round, <final_A, final_B>, which needs every diagonal before it.
 #define SIPP_MAT_MACHINES 8
 #define SIPP_MAT_REGS 4  // 0 accumulator, 1 base, 2 its conjugate, 3 exchange
 #define SIPP_MAT_SLOTS (SIPP_F12_GLOBAL_SLOTS + SIPP_F12_REG_SLOTS * SIPP_MAT_REGS)
-__global__ void __launch_bounds__(SIPP_MAT_MACHINES * 32) k_mat_fold(const uint32_t* __restrict__ E, size_t n, uint32_t* __restrict__ Eout, GtPlan plan_arg) {
+__global__ void __launch_bounds__(SIPP_MAT_MACHINES * 32) k_mat_fold(const uint32_t* __restrict__ E, size_t n, uint32_t* __restrict__ Eout, GtPlan plan_arg, int diag) {
     __shared__ __align__(16) uint32_t smem[SIPP_MAT_MACHINES * SIPP_MAT_SLOTS * 8];
     __shared__ GtPlan plan;
     const size_t h = n / 2;
     const size_t i = blockIdx.x / h, j = blockIdx.x % h;
-    if (i == j) return;
+    if (i == j && !diag) return;
     for (int t = threadIdx.x; t < (int)(sizeof(GtPlan) / 4); t += blockDim.x) ((uint32_t*)&plan)[t] = ((const uint32_t*)&plan_arg)[t];
     __syncthreads();
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -130,9 +131,9 @@ __global__ void __launch_bounds__(SIPP_MAT_MACHINES * 32) k_mat_fold(const uint3
         for (int w = lane; w < 96; w += 32) o[w] = slots[f12_reg_base(0) * 8 + w];
     }
 }
-int launch_mat_fold(const uint32_t* E, size_t n, uint32_t* Eout, const GtPlan& plan, cudaStream_t s) {
+int launch_mat_fold(const uint32_t* E, size_t n, uint32_t* Eout, const GtPlan& plan, bool diag, cudaStream_t s) {
     const size_t h = n / 2;
-    k_mat_fold<<<(unsigned)(h * h), SIPP_MAT_MACHINES * 32, 0, s>>>(E, n, Eout, plan);
+    k_mat_fold<<<(unsigned)(h * h), SIPP_MAT_MACHINES * 32, 0, s>>>(E, n, Eout, plan, diag ? 1 : 0);
     return (int)cudaGetLastError();
 }
 

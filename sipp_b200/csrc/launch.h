@@ -62,7 +62,8 @@ size_t lines_bytes_per_pair();
 int launch_mat_gather(const uint32_t* A, const uint32_t* B, size_t nr, size_t m, uint32_t* Aexp, uint32_t* Bexp, cudaStream_t s);
 int launch_mat_fe(const uint32_t* miller, size_t count, uint32_t* E, int ark_norm, cudaStream_t s);
 int launch_mat_diag(const uint32_t* E, size_t n, int main_diagonal, uint32_t* partials, cudaStream_t s);
-int launch_mat_fold(const uint32_t* E, size_t n, uint32_t* Eout, const GtPlan& plan, cudaStream_t s);
+// diag: also the diagonal entries, which no later round of a proof reads (the statement prover reads the last 1 x 1 matrix)
+int launch_mat_fold(const uint32_t* E, size_t n, uint32_t* Eout, const GtPlan& plan, bool diag, cudaStream_t s);
 
 // batched instances (k_coop.cu, k_fold.cu, k_transcript.cu)
 int launch_lines_batch(const uint32_t* A, const uint32_t* B, const BatchJob& job, size_t p0, size_t np, uint32_t* lines, cudaStream_t s);

@@ -1,5 +1,5 @@
 // ragged.cu -- batched proving and verification of independent instances of different sizes (C ABI: sipp_prove_native_batch_ragged,
-// sipp_prove_native_batch_ragged_device, sipp_verify_native_batch_ragged, test hook sipp_test_ragged_schedule).
+// sipp_prove_native_batch_ragged_device, their _statement forms, sipp_verify_native_batch_ragged, test hook sipp_test_ragged_schedule).
 //
 // Instance j is pairs [offsets[j], offsets[j + 1]) of A and B, n_j a power of two; its proof is exactly sipp_prove_native on those
 // pairs (prover_native.rs:26-80).  The instances run in lock-step rounds, as in batch.cu, but each with its own size:
@@ -185,9 +185,65 @@ int ragged_flags_status(const int fl[2]) {
     return SIPP_OK;
 }
 
+// The statement tail of a ragged batch, shared by the verifier and the statement prover (verifier_native.rs:74-75, :80): the final
+// point of every instance -- its first point once the points are folded -- gathered in the caller's order, paired through the
+// products path (one one-pair segment per instance) and encoded.
+struct RaggedFinals {
+    ProductPlan plan;
+    std::vector<uint64_t> at;
+    uint32_t *gA = nullptr, *gB = nullptr, *work = nullptr;
+    uint64_t* dat = nullptr;
+    ProductGroup* dgroups = nullptr;
+    ProductTask* dtasks = nullptr;
+    ~RaggedFinals() {  // recycled blocks: every caller synchronises its streams before it returns
+        pool_free(gA); pool_free(gB); pool_free(work); pool_free(dat); pool_free(dgroups); pool_free(dtasks);
+    }
+    // the host plan, the device blocks and the line table (before any launch: growing the table frees the old one); offsets checked
+    int prepare(const size_t* offsets, size_t count) {
+        at.assign(offsets, offsets + count);                                           // final_A = A[0], final_B = B[0]  :74-75
+        std::vector<size_t> ones(count + 1);
+        for (size_t j = 0; j <= count; j++) ones[j] = j;
+        int rc = product_plan(ones.data(), count, g_opt_batch_kpg_max, (size_t)g_opt_product_chunk, plan);
+        if (rc) return rc;
+        cudaError_t e = pool_alloc((void**)&gA, count * 64);
+        if (e == cudaSuccess) e = pool_alloc((void**)&gB, count * 128);
+        if (e == cudaSuccess) e = pool_alloc((void**)&work, plan.work_slots(count) * 384);
+        if (e == cudaSuccess) e = pool_alloc((void**)&dat, count * sizeof(uint64_t));
+        if (e == cudaSuccess) e = pool_alloc((void**)&dgroups, plan.groups.size() * sizeof(ProductGroup));
+        if (e == cudaSuccess) e = pool_alloc((void**)&dtasks, plan.tasks.size() * sizeof(ProductTask));
+        if (e != cudaSuccess) return cuda_fail(e, "cudaMalloc(ragged finals)");
+        return lines_reserve((count < plan.chunk_pairs ? count : plan.chunk_pairs) * lines_bytes_per_pair());
+    }
+    // enqueues on s, after the last fold of dA / dB: pair (when non-NULL) <- count pairings (384 B each, encoded); fin (when non-NULL)
+    // <- count x 64 B final_A, then count x 128 B final_B (encoded)
+    int run(const uint32_t* dA, const uint32_t* dB, size_t count, uint32_t* pair, uint32_t* fin, cudaStream_t s) {
+        if (!pair && !fin) return SIPP_OK;
+        CK(cudaMemcpyAsync(dat, at.data(), count * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+        int le = launch_gather_points(dA, dB, dat, count, gA, gB, s);
+        if (le) return cuda_fail((cudaError_t)le, "k_gather_points");
+        g_stats.launches++;
+        if (pair) {                                                                     // pairing(final_A, final_B)  :80
+            CK(cudaMemcpyAsync(dgroups, plan.groups.data(), plan.groups.size() * sizeof(ProductGroup), cudaMemcpyHostToDevice, s));
+            CK(cudaMemcpyAsync(dtasks, plan.tasks.data(), plan.tasks.size() * sizeof(ProductTask), cudaMemcpyHostToDevice, s));
+            le = products_launch(gA, gB, count, count, plan, dgroups, dtasks, work, pair, s);
+            if (le) return le;
+        }
+        if (fin) {
+            le = launch_codec_encode(gA, fin, count * 2, s);
+            if (!le) le = launch_codec_encode(gB, fin + count * 16, count * 4, s);
+            if (le) return cuda_fail((cudaError_t)le, "k_codec_encode");
+            g_stats.launches += 2;
+        }
+        return SIPP_OK;
+    }
+};
+
 // the whole call: bytesA / bytesB hold the boundary bytes (host staging copies or the caller's device buffers); the proofs are
-// copied to `out` (host or device memory, per out_kind) only when every point and every challenge passed its checks
-int ragged_run(const uint32_t* bytesA, const uint32_t* bytesB, size_t n, const size_t* offsets, size_t count, void* out, cudaMemcpyKind out_kind) {
+// copied to `out` (host or device memory, per out_kind) only when every point and every challenge passed its checks.  The statement
+// outputs (each may be NULL, then it is not computed): final_A / final_B / final_Z of every instance in the caller's order, copied
+// with the proofs.
+int ragged_run(const uint32_t* bytesA, const uint32_t* bytesB, size_t n, const size_t* offsets, size_t count, void* out, cudaMemcpyKind out_kind,
+               void* final_A, void* final_B, void* final_Z) {
     cudaStream_t s = g_stream;
     RaggedSchedule S;
     int rc = ragged_schedule(offsets, count, S);
@@ -223,6 +279,18 @@ int ragged_run(const uint32_t* bytesA, const uint32_t* bytesB, size_t n, const s
     if (e != cudaSuccess) return cuda_fail(e, "cudaMalloc(prove_native_batch_ragged)");
     rc = lines_reserve(S.lines_pairs * lines_bytes_per_pair());
     if (rc) return rc;
+    RaggedFinals fins;
+    uint32_t *pair = nullptr, *enc = nullptr;
+    const bool statement = final_A || final_B || final_Z;
+    if (statement) {
+        rc = fins.prepare(offsets, count);
+        if (rc) return rc;
+        e = final_Z ? pool_alloc((void**)&pair, count * 384) : cudaSuccess;
+        if (e == cudaSuccess && (final_A || final_B)) e = pool_alloc((void**)&enc, count * 192);
+        release.p.push_back(pair);
+        release.p.push_back(enc);
+        if (e != cudaSuccess) return cuda_fail(e, "cudaMalloc(prove_native_batch_ragged statement)");
+    }
     auto run = [&]() -> int {
         CK(cudaMemsetAsync(flags, 0, 2 * sizeof(int), s));
         CK(cudaMemcpyAsync(ddst, S.dst.data(), S.dst.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
@@ -267,12 +335,19 @@ int ragged_run(const uint32_t* bytesA, const uint32_t* bytesB, size_t n, const s
                 g_stats.fold_points += rd.elems;
             }
         }
+        if (statement) {
+            le = fins.run(dA, dB, count, pair, enc, s);
+            if (le) return le;
+        }
         int fl[2] = {0, 0};
         CK(cudaMemcpyAsync(fl, flags, sizeof fl, cudaMemcpyDeviceToHost, s));
         CK(cudaStreamSynchronize(s));
         const int st = ragged_flags_status(fl);
         if (st) return st;
         CK(cudaMemcpyAsync(out, proofs, S.proof_fq12 * 384, out_kind, s));
+        if (final_A) CK(cudaMemcpyAsync(final_A, enc, count * 64, out_kind, s));
+        if (final_B) CK(cudaMemcpyAsync(final_B, enc + count * 16, count * 128, out_kind, s));
+        if (final_Z) CK(cudaMemcpyAsync(final_Z, pair, count * 384, out_kind, s));
         CK(cudaStreamSynchronize(s));
         return SIPP_OK;
     };
@@ -312,7 +387,6 @@ int ragged_verify_run(const uint8_t* A, const uint8_t* B, size_t n, const size_t
     std::vector<RaggedGt> gt(npow + count);
     std::vector<ProductTask> ftasks(count);
     std::vector<size_t> fbase(count);
-    std::vector<uint64_t> at(count);
     size_t nfac = 0;
     for (size_t k = 0; k < count; k++) {
         const size_t j = S.order[k], nj = offsets[j + 1] - offsets[j], np = sipp_proof_len(nj);
@@ -326,22 +400,17 @@ int ragged_verify_run(const uint8_t* A, const uint8_t* B, size_t n, const size_t
     for (size_t r = 1; r <= R; r++)
         for (size_t k = 0; k < S.rounds[r].act; k++)                                   // Z_L at np - 2r, Z_R at np - 1 - 2r  :40, :42
             gt[S.rounds[r].tab0 + k] = RaggedGt{pt[k].first + pt[k].np - 2 * r, (uint32_t)(fbase[k] + r), 0};
-    for (size_t j = 0; j < count; j++) at[j] = offsets[j];                              // final_A = A[0], final_B = B[0]  :74-75
-    // the final pairings: one one-pair segment per instance
-    std::vector<size_t> ones(count + 1);
-    for (size_t j = 0; j <= count; j++) ones[j] = j;
-    ProductPlan plan;
-    int rc = product_plan(ones.data(), count, g_opt_batch_kpg_max, (size_t)g_opt_product_chunk, plan);
+    RaggedFinals fins;
+    int rc = fins.prepare(offsets, count);
     if (rc) return rc;
-    uint32_t *bA = nullptr, *bB = nullptr, *dA = nullptr, *dB = nullptr, *dproofs = nullptr, *fac = nullptr, *gA = nullptr, *gB = nullptr;
-    uint32_t *work = nullptr, *res = nullptr, *enc = nullptr;
-    uint64_t *states = nullptr, *chal = nullptr, *dat = nullptr;
+    uint32_t *bA = nullptr, *bB = nullptr, *dA = nullptr, *dB = nullptr, *dproofs = nullptr, *fac = nullptr;
+    uint32_t *res = nullptr, *enc = nullptr;
+    uint64_t *states = nullptr, *chal = nullptr;
     FoldPlan* plans = nullptr;
     RaggedInst* dtabs = nullptr;
     RaggedProof* dpt = nullptr;
     RaggedGt* dgt = nullptr;
-    ProductTask *dftasks = nullptr, *dtasks = nullptr;
-    ProductGroup* dgroups = nullptr;
+    ProductTask* dftasks = nullptr;
     int* flags = nullptr;  // [0] transcript / recoding, [1] encoding
     cudaError_t e = pool_alloc((void**)&bA, n * 64);
     if (e == cudaSuccess) e = pool_alloc((void**)&bB, n * 128);
@@ -349,29 +418,21 @@ int ragged_verify_run(const uint8_t* A, const uint8_t* B, size_t n, const size_t
     if (e == cudaSuccess) e = pool_alloc((void**)&dB, n * 128);
     if (e == cudaSuccess) e = pool_alloc((void**)&dproofs, ptotal * 384);
     if (e == cudaSuccess) e = pool_alloc((void**)&fac, (nfac + count) * 384);
-    if (e == cudaSuccess) e = pool_alloc((void**)&gA, count * 64);
-    if (e == cudaSuccess) e = pool_alloc((void**)&gB, count * 128);
-    if (e == cudaSuccess) e = pool_alloc((void**)&work, plan.work_slots(count) * 384);
     if (e == cudaSuccess) e = pool_alloc((void**)&res, 2 * count * 384);
     if (e == cudaSuccess) e = pool_alloc((void**)&enc, count * 192);
     if (e == cudaSuccess && act1) e = pool_alloc((void**)&states, act1 * 32);
     if (e == cudaSuccess && npow) e = pool_alloc((void**)&chal, npow * 64);
     if (e == cudaSuccess && npow) e = pool_alloc((void**)&plans, npow * sizeof(FoldPlan));
     if (e == cudaSuccess && npow) e = pool_alloc((void**)&dtabs, npow * sizeof(RaggedInst));
-    if (e == cudaSuccess) e = pool_alloc((void**)&dat, count * sizeof(uint64_t));
     if (e == cudaSuccess) e = pool_alloc((void**)&dpt, count * sizeof(RaggedProof));
     if (e == cudaSuccess) e = pool_alloc((void**)&dgt, gt.size() * sizeof(RaggedGt));
     if (e == cudaSuccess) e = pool_alloc((void**)&dftasks, count * sizeof(ProductTask));
-    if (e == cudaSuccess) e = pool_alloc((void**)&dgroups, plan.groups.size() * sizeof(ProductGroup));
-    if (e == cudaSuccess) e = pool_alloc((void**)&dtasks, plan.tasks.size() * sizeof(ProductTask));
     if (e == cudaSuccess) e = pool_alloc((void**)&flags, 2 * sizeof(int));
     struct Release {
         std::vector<void*> p;
         ~Release() { for (void* q : p) pool_free(q); }
-    } release{{bA, bB, dA, dB, dproofs, fac, gA, gB, work, res, enc, states, chal, plans, dtabs, dat, dpt, dgt, dftasks, dgroups, dtasks, flags}};
+    } release{{bA, bB, dA, dB, dproofs, fac, res, enc, states, chal, plans, dtabs, dpt, dgt, dftasks, flags}};
     if (e != cudaSuccess) return cuda_fail(e, "cudaMalloc(verify_native_batch_ragged)");
-    rc = lines_reserve((count < plan.chunk_pairs ? count : plan.chunk_pairs) * lines_bytes_per_pair());
-    if (rc) return rc;
     if (!g_fold_stream) CK(cudaStreamCreateWithFlags(&g_fold_stream, cudaStreamNonBlocking));
     cudaStream_t side = g_fold_stream;
     bool forked = false;
@@ -381,12 +442,9 @@ int ragged_verify_run(const uint8_t* A, const uint8_t* B, size_t n, const size_t
         CK(cudaMemcpyAsync(bB, B, n * 128, cudaMemcpyHostToDevice, s));
         CK(cudaMemcpyAsync(dproofs, proofs, ptotal * 384, cudaMemcpyHostToDevice, s));
         if (npow) CK(cudaMemcpyAsync(dtabs, S.tabs.data(), npow * sizeof(RaggedInst), cudaMemcpyHostToDevice, s));
-        CK(cudaMemcpyAsync(dat, at.data(), count * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
         CK(cudaMemcpyAsync(dpt, pt.data(), count * sizeof(RaggedProof), cudaMemcpyHostToDevice, s));
         CK(cudaMemcpyAsync(dgt, gt.data(), gt.size() * sizeof(RaggedGt), cudaMemcpyHostToDevice, s));
         CK(cudaMemcpyAsync(dftasks, ftasks.data(), count * sizeof(ProductTask), cudaMemcpyHostToDevice, s));
-        CK(cudaMemcpyAsync(dgroups, plan.groups.data(), plan.groups.size() * sizeof(ProductGroup), cudaMemcpyHostToDevice, s));
-        CK(cudaMemcpyAsync(dtasks, plan.tasks.data(), plan.tasks.size() * sizeof(ProductTask), cudaMemcpyHostToDevice, s));
         int le = ragged_decode_absorb(bA, bB, n, dA, dB, dtabs, act1, states, flags, s);  // round 1's table is the first
         if (le) return le;
         // the transcript replay: round r's fold plans and challenges x || x^-1 to its slices  :33 (first round), :40-46
@@ -423,16 +481,8 @@ int ragged_verify_run(const uint8_t* A, const uint8_t* B, size_t n, const size_t
             g_stats.launches++;
             g_stats.fold_points += rd.elems;
         }
-        // pairing(final_A, final_B)  :80
-        le = launch_gather_points(dA, dB, dat, count, gA, gB, s);
-        if (le) return cuda_fail((cudaError_t)le, "k_gather_points");
-        g_stats.launches++;
-        le = products_launch(gA, gB, count, count, plan, dgroups, dtasks, work, res + count * 96, s);
+        le = fins.run(dA, dB, count, res + count * 96, enc, s);                         // :74-75, :80
         if (le) return le;
-        le = launch_codec_encode(gA, enc, count * 2, s);
-        if (!le) le = launch_codec_encode(gB, enc + count * 16, count * 4, s);
-        if (le) return cuda_fail((cudaError_t)le, "k_codec_encode");
-        g_stats.launches += 2;
         CK(order_after(s, side));  // join
         int fl[2] = {0, 0};
         CK(cudaMemcpyAsync(fl, flags, sizeof fl, cudaMemcpyDeviceToHost, s));
@@ -454,7 +504,8 @@ int ragged_verify_run(const uint8_t* A, const uint8_t* B, size_t n, const size_t
 
 extern "C" {
 
-int sipp_prove_native_batch_ragged(const uint8_t* A, size_t a_len, const uint8_t* B, size_t b_len, const size_t* offsets, size_t count, uint8_t* proofs) {
+int sipp_prove_native_batch_ragged_statement(const uint8_t* A, size_t a_len, const uint8_t* B, size_t b_len, const size_t* offsets, size_t count,
+                                             uint8_t* proofs, uint8_t* final_A, uint8_t* final_B, uint8_t* final_Z) {
     int rc = ragged_args(A, a_len, B, b_len, offsets, count, proofs);
     if (rc) return rc;
     rc = ensure_init();
@@ -469,15 +520,24 @@ int sipp_prove_native_batch_ragged(const uint8_t* A, size_t a_len, const uint8_t
     if (e != cudaSuccess) return cuda_fail(e, "cudaMalloc(prove_native_batch_ragged)");
     CK(cudaMemcpyAsync(tA, A, a_len * 64, cudaMemcpyHostToDevice, g_stream));
     CK(cudaMemcpyAsync(tB, B, a_len * 128, cudaMemcpyHostToDevice, g_stream));
-    return ragged_run(tA, tB, a_len, offsets, count, proofs, cudaMemcpyDeviceToHost);  // synchronises: the staging blocks are idle on return
+    return ragged_run(tA, tB, a_len, offsets, count, proofs, cudaMemcpyDeviceToHost, final_A, final_B, final_Z);  // synchronises
 }
 
-int sipp_prove_native_batch_ragged_device(const void* dA, const void* dB, size_t n, const size_t* offsets, size_t count, void* d_proofs) {
+int sipp_prove_native_batch_ragged_statement_device(const void* dA, const void* dB, size_t n, const size_t* offsets, size_t count, void* d_proofs,
+                                                    void* d_final_A, void* d_final_B, void* d_final_Z) {
     int rc = ragged_args(dA, n, dB, n, offsets, count, d_proofs);
     if (rc) return rc;
     rc = ensure_init();
     if (rc) return rc;
-    return ragged_run((const uint32_t*)dA, (const uint32_t*)dB, n, offsets, count, d_proofs, cudaMemcpyDeviceToDevice);
+    return ragged_run((const uint32_t*)dA, (const uint32_t*)dB, n, offsets, count, d_proofs, cudaMemcpyDeviceToDevice, d_final_A, d_final_B, d_final_Z);
+}
+
+int sipp_prove_native_batch_ragged(const uint8_t* A, size_t a_len, const uint8_t* B, size_t b_len, const size_t* offsets, size_t count, uint8_t* proofs) {
+    return sipp_prove_native_batch_ragged_statement(A, a_len, B, b_len, offsets, count, proofs, nullptr, nullptr, nullptr);
+}
+
+int sipp_prove_native_batch_ragged_device(const void* dA, const void* dB, size_t n, const size_t* offsets, size_t count, void* d_proofs) {
+    return sipp_prove_native_batch_ragged_statement_device(dA, dB, n, offsets, count, d_proofs, nullptr, nullptr, nullptr);
 }
 
 int sipp_verify_native_batch_ragged(const uint8_t* A, size_t a_len, const uint8_t* B, size_t b_len, const size_t* offsets, size_t count,

@@ -530,18 +530,22 @@ int mat_products(MatTail& mt, uint8_t* zl, uint8_t* zr) {
 
 // E'[i][j] = E[i][j] E[i+h][j+h] E[i+h][j]^x E[i][j+h]^(x^-1)   (prover_native.rs:60-69 in GT); c->n halves.  A look-ahead stage
 // (m > 1) also folds the points themselves, on the side stream; when the matrix is used up the library stream waits for them.
+// c->keep_points (the statement prover): the tail stage folds its points the same way and keeps the diagonal, so that the 1 x 1
+// matrix after its last round is <final_A, final_B> = final_Z (verifier_native.rs:59-61, :80 by bilinearity).
 int mat_fold(sipp_ctx* c, MatTail& mt, const uint8_t x[32], const uint8_t xinv[32]) {
-    if (mt.n > 2) {  // the 1 x 1 matrix after the last round of a stage is never read
+    const bool keep = c->keep_points && mt.m == 1;
+    if (mt.n > 2 || keep) {  // the 1 x 1 matrix after the last round of a stage is never read by the proof
         GtPlan plan;
         if (gt_plan_build(x, xinv, &plan)) return fail(SIPP_ERR_ENCODING, "fold scalar out of range (must be < r)");
         Span sp(2, g_stream);
-        int le = launch_mat_fold(mt.E[mt.cur], mt.n, mt.E[mt.cur ^ 1], plan, g_stream);
+        int le = launch_mat_fold(mt.E[mt.cur], mt.n, mt.E[mt.cur ^ 1], plan, keep, g_stream);
         if (le) return cuda_fail((cudaError_t)le, "k_mat_fold");
         g_stats.launches++;
         mt.cur ^= 1;
     }
     const size_t h = c->n / 2;
-    if (mt.fold_points) {
+    const bool fold_points = mt.fold_points || keep;
+    if (fold_points) {
         FoldPlan fp;
         if (fold_plan_build(x, xinv, &fp)) return fail(SIPP_ERR_ENCODING, "fold scalar out of range (must be < r)");
         if (!g_fold_stream) CK(cudaStreamCreateWithFlags(&g_fold_stream, cudaStreamNonBlocking));
@@ -551,12 +555,24 @@ int mat_fold(sipp_ctx* c, MatTail& mt, const uint8_t x[32], const uint8_t xinv[3
         if (le) return cuda_fail((cudaError_t)le, "k_fold (look-ahead stage)");
         g_stats.launches++;
     }
-    if (!mt.fold_points) c->stale = true;  // the tail: the points are not folded any more
+    if (!fold_points) c->stale = true;  // the tail: the points are not folded any more
     g_stats.fold_points += h;
     c->n = h;
     mt.n /= 2;
     if (mt.n == 1) {  // stage over
-        if (mt.fold_points) CK(order_after(g_stream, g_fold_stream));
+        if (keep) {  // the 1 x 1 matrix, encoded as mat_products encodes Z_L, Z_R
+            {
+                Span sp(1, g_stream);
+                int le = launch_reduce_fe_eng(mt.E[mt.cur], 1, 1, g_scr.out, 2, g_opt_fe_norm, g_stream);
+                if (le) return cuda_fail((cudaError_t)le, "final_Z (matrix)");
+            }
+            g_stats.launches++;
+            CK(cudaMemcpyAsync(g_scr.h_out, g_scr.out, 384, cudaMemcpyDeviceToHost, g_stream));
+            CK(cudaStreamSynchronize(g_stream));
+            memcpy(c->final_z, g_scr.h_out, 384);
+            c->has_final_z = true;
+        }
+        if (fold_points) CK(order_after(g_stream, g_fold_stream));
         mt.reset();
     }
     return SIPP_OK;
@@ -1058,6 +1074,46 @@ int sipp_prove_native(const uint8_t* A, size_t a_len, const uint8_t* B, size_t b
     const int vrc = ctx_finish_validation(c);
     sipp_ctx_destroy(c);
     return vrc ? vrc : rc;
+}
+
+// sipp_prove_native plus the statement members sipp_verify_native would compute from its proof (verifier_native.rs:74-75, :59-61):
+// the points are folded to one (a tail stage keeps folding them, c->keep_points) and final_Z = <final_A, final_B>, read from the
+// tail's last matrix or, without a tail stage, paired as the verifier pairs them (:80).  Nothing reaches the caller unless every
+// point and challenge passed.
+int sipp_prove_native_statement(const uint8_t* A, size_t a_len, const uint8_t* B, size_t b_len, uint8_t* proof, uint8_t* final_A,
+                                uint8_t* final_B, uint8_t* final_Z) {
+    if (a_len != b_len) return fail(SIPP_ERR_LENGTH, "assert_eq!(A.len(), B.len()) failed");  // prover_native.rs:27
+    if (!is_pow2(a_len)) return fail(SIPP_ERR_ARG, "n must be a non-zero power of two");
+    if (!A || !B || !proof) return fail(SIPP_ERR_ARG, "null argument");
+    int rc = ensure_init();
+    if (rc) return rc;
+    AbsorbJob job;
+    job.start(A, B, a_len);
+    sipp_ctx* c;
+    rc = ctx_create_ex(A, B, a_len, &c, true);
+    if (rc) return rc;
+    c->keep_points = true;
+    std::vector<uint8_t> pf(sipp_proof_len(a_len) * 384);
+    uint8_t fa[64], fb[128], fz[384];
+    rc = prove_core(c, job, pf.data());
+    if (!rc && a_len == 1) {  // no round: the inputs and Z
+        memcpy(fa, A, 64);
+        memcpy(fb, B, 128);
+        memcpy(fz, pf.data(), 384);
+    } else if (!rc) {
+        rc = sipp_ctx_read(c, final_A ? fa : nullptr, final_B ? fb : nullptr);  // A[0], B[0]  :74-75
+        if (!rc && c->has_final_z) memcpy(fz, c->final_z, 384);
+        else if (!rc && final_Z) rc = sipp_ctx_inner_product(c, fz);             // pairing(final_A, final_B)  :80
+    }
+    const int vrc = ctx_finish_validation(c);
+    sipp_ctx_destroy(c);
+    if (vrc) return vrc;
+    if (rc) return rc;
+    memcpy(proof, pf.data(), pf.size());
+    if (final_A) memcpy(final_A, fa, 64);
+    if (final_B) memcpy(final_B, fb, 128);
+    if (final_Z) memcpy(final_Z, fz, 384);
+    return SIPP_OK;
 }
 
 int sipp_verify_native(const uint8_t* A, size_t a_len, const uint8_t* B, size_t b_len, const uint8_t* proof, size_t proof_len, uint8_t* final_A,
