@@ -287,6 +287,20 @@ int sipp_prove_native_batch(const uint8_t *A, const uint8_t *B, size_t n, size_t
  * the computed statement members when non-NULL.  The return value reports whether the batch ran, not whether proofs verified. */
 int sipp_verify_native_batch(const uint8_t *A, const uint8_t *B, size_t n, size_t count, const uint8_t *proofs, size_t proof_len,
                              int *results, uint8_t *final_A, uint8_t *final_B, uint8_t *final_Z);
+/* sipp_verify_native_batch with every buffer in DEVICE memory (boundary format, 4-byte aligned): dA, dB, d_proofs as for the host form,
+ * d_results count x int32, d_final_A / _B / _Z count x 64 / 128 / 384 B, each final may be NULL.  results[j] and every final are
+ * byte-identical to the host form's on the same bytes and options: the finals are written for every instance, SIPP_ERR_ENCODING ones
+ * included.  A, B and the proofs are only read, in place; no input crosses PCIe.
+ *   - Argument checks, all before the device is touched: a NULL dA, dB or d_proofs, count == 0, n not a non-zero power of two, then
+ *     a NULL d_results: SIPP_ERR_ARG; then proof_len < sipp_proof_len(n): SIPP_ERR_SHORT_PROOF.  Valid arguments without a device give
+ *     SIPP_ERR_CUDA.  One difference: sipp_verify_native_batch initialises the device first, so without a device it returns
+ *     SIPP_ERR_CUDA for bad arguments too, where this call returns their own codes.
+ *   - A bad point or a zero challenge fails the whole call, and then nothing is written to d_results or the finals.
+ *   - The library stream waits for the work already enqueued on the legacy default stream (torch's current stream unless the caller
+ *     switched streams) before it reads an input; the call returns when the results and finals are complete.
+ *   - Options and sipp_stats.fold_points / miller_pairs as for the host form; launches grows by more (not part of the contract). */
+int sipp_verify_native_batch_device(const void *dA, const void *dB, size_t n, size_t count, const void *d_proofs, size_t proof_len,
+                                    int *d_results, void *d_final_A, void *d_final_B, void *d_final_Z);
 /* same with DEVICE buffers in boundary format (inputs resident in HBM, proofs left in HBM) */
 int sipp_prove_native_batch_device(const void *dA, const void *dB, size_t n, size_t count, void *d_proofs);
 /* sipp_prove_native_batch plus every instance's statement members, as sipp_prove_native_statement gives them for one instance:
@@ -375,6 +389,16 @@ int sipp_prove_native_batch_ragged_statement_device(const void *dA, const void *
 int sipp_verify_native_batch_ragged(const uint8_t *A, size_t a_len, const uint8_t *B, size_t b_len, const size_t *offsets, size_t count,
                                     const uint8_t *proofs, const size_t *proof_offsets, int *results, uint8_t *final_A, uint8_t *final_B,
                                     uint8_t *final_Z);
+/* sipp_verify_native_batch_ragged with A, B, the proofs, d_results (count x int32) and the finals in DEVICE memory (boundary format,
+ * 4-byte aligned; n pairs); offsets and proof_offsets stay on the host.  results[j] and every final are byte-identical to the host
+ * form's on the same bytes and options: the finals of an instance are written only when its result is SIPP_OK or SIPP_ERR_VERIFY,
+ * and its slots are left untouched for SIPP_ERR_ENCODING.  A, B and the proofs are only read, in place.  Argument checks, their order
+ * and codes as for the host form, all before the device is touched (valid arguments without a device: SIPP_ERR_CUDA).  A bad point or
+ * a zero challenge fails the whole call and writes nothing to d_results or the finals.  Stream order, options and sipp_stats as for
+ * sipp_verify_native_batch_device. */
+int sipp_verify_native_batch_ragged_device(const void *dA, const void *dB, size_t n, const size_t *offsets, size_t count,
+                                           const void *d_proofs, const size_t *proof_offsets, int *d_results, void *d_final_A,
+                                           void *d_final_B, void *d_final_Z);
 
 /* ---- input producers of the BLS-aggregation demo (bin/bls_aggregation.rs:95-117; SURVEY 8f row 3) ---------------------------- */
 /* Scalars are 32-byte little-endian integers < r.  The `_device` forms take DEVICE pointers in the same formats.

@@ -9,6 +9,6 @@ from .api import (ProverContext, SIPPStatement, Transcript, VerificationError, c
                   pairing, pairing_batch, seeded_inputs, set_option, sipp_prove_native, sipp_prove_native_batch,
                   sipp_prove_native_batch_ragged, sipp_prove_native_batch_ragged_device, sipp_prove_native_batch_ragged_statement,
                   sipp_prove_native_batch_ragged_statement_device, sipp_prove_native_batch_statement, sipp_prove_native_batch_statement_device,
-                  sipp_prove_native_statement, sipp_verify_native, sipp_verify_native_batch,
-                  sipp_verify_native_batch_ragged, stats)
+                  sipp_prove_native_statement, sipp_verify_native, sipp_verify_native_batch, sipp_verify_native_batch_device,
+                  sipp_verify_native_batch_ragged, sipp_verify_native_batch_ragged_device, stats)
 from ._lib import SippError  # noqa: F401

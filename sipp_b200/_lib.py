@@ -122,6 +122,8 @@ def load():
     lib.sipp_prove_native_batch_ragged_statement_device.argtypes = [vp, vp, sz, szp, sz, vp, vp, vp, vp]
     lib.sipp_verify_native_batch.argtypes = [u8p, u8p, sz, sz, u8p, sz, ctypes.POINTER(ctypes.c_int), u8p, u8p, u8p]
     lib.sipp_verify_native_batch_ragged.argtypes = [u8p, sz, u8p, sz, szp, sz, u8p, szp, ctypes.POINTER(ctypes.c_int), u8p, u8p, u8p]
+    lib.sipp_verify_native_batch_device.argtypes = [vp, vp, sz, sz, vp, sz, vp, vp, vp, vp]
+    lib.sipp_verify_native_batch_ragged_device.argtypes = [vp, vp, sz, szp, sz, vp, szp, vp, vp, vp, vp]
     lib.sipp_test_poseidon_device.argtypes = [ctypes.POINTER(ctypes.c_uint64), sz]
     lib.sipp_test_transcript_round_device.argtypes = [ctypes.POINTER(ctypes.c_uint64), u8p, i, sz, u8p, ctypes.POINTER(ctypes.c_uint32)]
     lib.sipp_test_fold_plan.argtypes = [u8p, u8p, ctypes.POINTER(ctypes.c_uint32), sz]

@@ -401,6 +401,33 @@ def sipp_verify_native_batch_ragged(A: Points, B: Points, lengths: Sequence[int]
     return out
 
 
+def sipp_verify_native_batch_device(dA: int, dB: int, n: int, count: int, d_proofs: int, proof_len: int, d_results: int, d_final_A: int = 0,
+                                    d_final_B: int = 0, d_final_Z: int = 0) -> None:
+    """sipp_verify_native_batch on DEVICE buffers (integer pointers, e.g. tensor.data_ptr(); 0 for a final not wanted): dA n count x 64 B,
+    dB n count x 128 B, d_proofs count x proof_len x 384 B, d_results count x int32 (SIPP_OK / ERR_VERIFY / ERR_ENCODING per instance),
+    d_final_A / _B / _Z count x 64 / 128 / 384 B.  Inputs written on torch's default stream need no synchronisation first."""
+    _lib.require_gpu_once()
+    _lib.check(_lib.load().sipp_verify_native_batch_device(dA, dB, n, count, d_proofs, proof_len, d_results, d_final_A or None, d_final_B or None,
+                                                           d_final_Z or None))
+
+
+def sipp_verify_native_batch_ragged_device(dA: int, dB: int, n: int, lengths: Sequence[int], d_proofs: int, proof_lengths: Sequence[int],
+                                           d_results: int, d_final_A: int = 0, d_final_B: int = 0, d_final_Z: int = 0) -> None:
+    """sipp_verify_native_batch_ragged on DEVICE buffers (integer pointers; 0 for a final not wanted): instance j is the next lengths[j]
+    of the n pairs of dA / dB, its proof the next proof_lengths[j] Fq12 of d_proofs (read from its end); d_results len(lengths) x int32,
+    d_final_A / _B / _Z len(lengths) x 64 / 128 / 384 B in the caller's order, written for the instances that are not ERR_ENCODING"""
+    offs = _ragged_offsets(lengths, n)
+    count = len(offs) - 1
+    if count == 0:
+        raise ValueError("no instances")
+    if len(proof_lengths) != count:
+        raise ValueError("%d instances but %d proof lengths" % (count, len(proof_lengths)))
+    poffs = _offsets(proof_lengths, sum(int(x) for x in proof_lengths))
+    _lib.require_gpu_once()
+    _lib.check(_lib.load().sipp_verify_native_batch_ragged_device(dA, dB, n, offs, count, d_proofs, poffs, d_results, d_final_A or None,
+                                                                  d_final_B or None, d_final_Z or None))
+
+
 def sipp_verify_native(A: Points, B: Points, proof: Sequence[bytes]) -> SIPPStatement:
     """verifier_native.rs:14-85; returns the SIPPStatement or raises VerificationError."""
     a, b = _flat(A, G1_BYTES), _flat(B, G2_BYTES)

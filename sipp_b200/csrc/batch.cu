@@ -327,6 +327,70 @@ int batch_args(const void* A, const void* B, size_t n, size_t count, const void*
     return SIPP_OK;
 }
 
+// The device blocks of a batched verification.  staging: the host form uploads A, B and the proofs to b.bytesA, b.bytesB and
+// dproofs; otherwise b.bytesA / b.bytesB are only the scratch of batch_finals (count points each) and there is no dproofs.
+struct VerifyBuffers {
+    BatchBuffers b;
+    uint32_t *dproofs = nullptr, *dz = nullptr, *dpair = nullptr, *dfin = nullptr;
+    uint64_t* dchal = nullptr;
+    int alloc(size_t n, size_t count, size_t proof_len, bool staging) {
+        const size_t pts = staging ? n * count : count, total = n * count;
+        cudaError_t e = pool_alloc((void**)&b.bytesA, pts * 64);
+        if (e == cudaSuccess) e = pool_alloc((void**)&b.bytesB, pts * 128);
+        if (e == cudaSuccess) e = pool_alloc((void**)&b.dA, total * 64);
+        if (e == cudaSuccess) e = pool_alloc((void**)&b.dB, total * 128);
+        if (e == cudaSuccess) e = pool_alloc((void**)&b.partials, count * 384);
+        if (e == cudaSuccess) e = pool_alloc((void**)&b.states, count * 32);
+        if (e == cudaSuccess) e = pool_alloc((void**)&b.plans, count * sizeof(FoldPlan));
+        if (e == cudaSuccess) e = pool_alloc((void**)&b.flags, 2 * sizeof(int));
+        if (e == cudaSuccess && staging) e = pool_alloc((void**)&dproofs, count * proof_len * 384);
+        if (e == cudaSuccess) e = pool_alloc((void**)&dz, count * 384);
+        if (e == cudaSuccess) e = pool_alloc((void**)&dpair, count * 384);
+        if (e == cudaSuccess) e = pool_alloc((void**)&dfin, count * 192);
+        if (e == cudaSuccess) e = pool_alloc((void**)&dchal, count * 64);
+        return e == cudaSuccess ? SIPP_OK : cuda_fail(e, "cudaMalloc(verify batch)");
+    }
+    ~VerifyBuffers() {  // recycled blocks: every caller synchronises the stream before it returns
+        b.release();
+        pool_free(dproofs); pool_free(dz); pool_free(dpair); pool_free(dfin); pool_free(dchal);
+    }
+};
+
+// `count` independent verifications in lock-step (verifier_native.rs:14-80 per instance) on boundary bytes in device memory, which are
+// only read: bytesA / bytesB (count x n points), proofs (count x proof_len Fq12).  The transcript replay, the folds and the GT update
+// Z_L^x Z Z_R^(x^-1) of every instance run in the same launches; the final pairing check (:80) is one batched product of one pair per
+// instance.  Enqueues on s: final_Z to v.dz, the pairings to v.dpair and, when fin, final_A then final_B to v.dfin (encoded).
+int batch_verify_enqueue(VerifyBuffers& v, const uint32_t* bytesA, const uint32_t* bytesB, const uint32_t* proofs, size_t n, size_t count,
+                         size_t proof_len, bool fin, cudaStream_t s) {
+    BatchBuffers& b = v.b;
+    const size_t total = n * count, top = proof_len;  // the verifier pops from the end: Z = proof[top - 1]
+    CK(cudaMemsetAsync(b.flags, 0, 2 * sizeof(int), s));
+    int le = launch_codec_decode(bytesA, b.dA, total * 2, b.flags + 1, s);
+    if (!le) le = launch_codec_decode(bytesB, b.dB, total * 4, b.flags + 1, s);
+    if (!le && g_opt_validate) { le = launch_validate_points(b.dA, b.dB, total, b.flags + 1, s); g_stats.launches++; }
+    if (!le) le = launch_tr_absorb_pairs(bytesA, bytesB, n, count, b.states, s);                       // :25-28
+    if (le) return cuda_fail((cudaError_t)le, "verify batch: decode / absorb");
+    g_stats.launches += 3;
+    // let original_Z = proof.pop().unwrap();  :31   (Z of instance j = its last Fq12)
+    CK(cudaMemcpy2DAsync(v.dz, 384, (const uint8_t*)proofs + (top - 1) * 384, proof_len * 384, 384, count, cudaMemcpyDeviceToDevice, s));
+    size_t m = n;
+    int round = 1;
+    while (m > 1) {                                                                                     // :35
+        const int slot_l = (int)top - 2 * round, slot_r = (int)top - 1 - 2 * round;                     // :40, :42
+        le = launch_tr_round(b.states, proofs, proof_len, round == 1 ? (int)top - 1 : -1, slot_l, slot_r, g_opt_fq12_order, count, b.plans,
+                             v.dchal, b.flags, s);                                                       // :33 (first round), :41-46
+        if (!le) le = (g_opt_fold_straus && count * (m / 2) >= 16384) ? launch_fold_straus(b.dA, b.dB, m / 2, n, count, b.plans, s)
+                                                                         : launch_fold_batch(b.dA, b.dB, m / 2, n, count, b.plans, s);  // :48-57
+        if (!le) le = launch_gt_fold_batch(proofs, proof_len, slot_l, slot_r, v.dchal, v.dz, count, s);  // :59-61
+        if (le) return cuda_fail((cudaError_t)le, "verify batch: round");
+        g_stats.launches += 3;
+        g_stats.fold_points += count * (m / 2);
+        m /= 2;
+        round++;
+    }
+    return batch_finals(b, n, count, v.dpair, fin ? v.dfin : nullptr, s);                              // :74-75, :80
+}
+
 }  // namespace
 
 extern "C" {
@@ -426,9 +490,8 @@ int sipp_prove_native_batch_statement_device(const void* dA, const void* dB, siz
     return batch_prove_statement(dA, dB, n, count, d_proofs, d_final_A, d_final_B, d_final_Z, cudaMemcpyDeviceToDevice, cudaMemcpyDeviceToDevice);
 }
 
-// `count` independent verifications in lock-step (verifier_native.rs:14-85 per instance): the transcript replay, the folds and the
-// GT update Z_L^x Z Z_R^(x^-1) of every instance run in the same launches; the final pairing check (:80) is one batched
-// product of one pair per instance.  results[j] = SIPP_OK / SIPP_ERR_VERIFY.
+// `count` independent verifications in lock-step (verifier_native.rs:14-85 per instance, batch_verify_enqueue).
+// results[j] = SIPP_OK / SIPP_ERR_VERIFY / SIPP_ERR_ENCODING.
 int sipp_verify_native_batch(const uint8_t* A, const uint8_t* B, size_t n, size_t count, const uint8_t* proofs, size_t proof_len, int* results,
                              uint8_t* final_A, uint8_t* final_B, uint8_t* final_Z) {
     int rc = ensure_init();
@@ -438,69 +501,28 @@ int sipp_verify_native_batch(const uint8_t* A, const uint8_t* B, size_t n, size_
     if (rc) return rc;
     const size_t np = sipp_proof_len(n);
     if (proof_len < np) return fail(SIPP_ERR_SHORT_PROOF, "proof.pop().unwrap() on an empty proof");  // verifier_native.rs:31,40,42
-    const size_t total = n * count, top = proof_len;  // the verifier pops from the end: Z = proof[top - 1]
+    const size_t total = n * count;
     cudaStream_t s = g_stream;
-    BatchBuffers b;
-    uint32_t *dproofs = nullptr, *dz = nullptr, *dpair = nullptr, *dfin = nullptr;
-    uint64_t* dchal = nullptr;
-    cudaError_t e = pool_alloc((void**)&b.bytesA, total * 64);
-    if (e == cudaSuccess) e = pool_alloc((void**)&b.bytesB, total * 128);
-    if (e == cudaSuccess) e = pool_alloc((void**)&b.dA, total * 64);
-    if (e == cudaSuccess) e = pool_alloc((void**)&b.dB, total * 128);
-    if (e == cudaSuccess) e = pool_alloc((void**)&b.partials, count * 384);
-    if (e == cudaSuccess) e = pool_alloc((void**)&b.states, count * 32);
-    if (e == cudaSuccess) e = pool_alloc((void**)&b.plans, count * sizeof(FoldPlan));
-    if (e == cudaSuccess) e = pool_alloc((void**)&b.flags, 2 * sizeof(int));
-    if (e == cudaSuccess) e = pool_alloc((void**)&dproofs, count * proof_len * 384);
-    if (e == cudaSuccess) e = pool_alloc((void**)&dz, count * 384);
-    if (e == cudaSuccess) e = pool_alloc((void**)&dpair, count * 384);
-    if (e == cudaSuccess) e = pool_alloc((void**)&dfin, count * 192);
-    if (e == cudaSuccess) e = pool_alloc((void**)&dchal, count * 64);
-    auto release = [&]() {
-        b.release();
-        pool_free(dproofs); pool_free(dz); pool_free(dpair); pool_free(dfin); pool_free(dchal);
-    };
-    if (e != cudaSuccess) { release(); return cuda_fail(e, "cudaMalloc(verify batch)"); }
     std::vector<uint8_t> hz(count * 384), hp(count * 384);
-    auto run = [&]() -> int {
-        CK(cudaMemcpyAsync(b.bytesA, A, total * 64, cudaMemcpyHostToDevice, s));
-        CK(cudaMemcpyAsync(b.bytesB, B, total * 128, cudaMemcpyHostToDevice, s));
-        CK(cudaMemcpyAsync(dproofs, proofs, count * proof_len * 384, cudaMemcpyHostToDevice, s));
-        CK(cudaMemsetAsync(b.flags, 0, 2 * sizeof(int), s));
-        int le = launch_codec_decode(b.bytesA, b.dA, total * 2, b.flags + 1, s);
-        if (!le) le = launch_codec_decode(b.bytesB, b.dB, total * 4, b.flags + 1, s);
-        if (!le && g_opt_validate) { le = launch_validate_points(b.dA, b.dB, total, b.flags + 1, s); g_stats.launches++; }
-        if (!le) le = launch_tr_absorb_pairs(b.bytesA, b.bytesB, n, count, b.states, s);                 // :25-28
-        if (le) return cuda_fail((cudaError_t)le, "verify batch: decode / absorb");
-        g_stats.launches += 3;
-        // let original_Z = proof.pop().unwrap();  :31   (Z of instance j = its last Fq12)
-        CK(cudaMemcpy2DAsync(dz, 384, (const uint8_t*)dproofs + (top - 1) * 384, proof_len * 384, 384, count, cudaMemcpyDeviceToDevice, s));
-        size_t m = n;
-        int round = 1;
-        while (m > 1) {                                                                                     // :35
-            const int slot_l = (int)top - 2 * round, slot_r = (int)top - 1 - 2 * round;                     // :40, :42
-            le = launch_tr_round(b.states, dproofs, proof_len, round == 1 ? (int)top - 1 : -1, slot_l, slot_r, g_opt_fq12_order, count, b.plans,
-                                 dchal, b.flags, s);                                                         // :33 (first round), :41-46
-            if (!le) le = (g_opt_fold_straus && count * (m / 2) >= 16384) ? launch_fold_straus(b.dA, b.dB, m / 2, n, count, b.plans, s)
-                                                                             : launch_fold_batch(b.dA, b.dB, m / 2, n, count, b.plans, s);  // :48-57
-            if (!le) le = launch_gt_fold_batch(dproofs, proof_len, slot_l, slot_r, dchal, dz, count, s);  // :59-61
-            if (le) return cuda_fail((cudaError_t)le, "verify batch: round");
-            g_stats.launches += 3;
-            g_stats.fold_points += count * (m / 2);
-            m /= 2;
-            round++;
-        }
-        int rc2 = batch_finals(b, n, count, dpair, (final_A || final_B) ? dfin : nullptr, s);   // :74-75, :80
-        if (rc2) return rc2;
-        if (final_A) CK(cudaMemcpyAsync(final_A, dfin, count * 64, cudaMemcpyDeviceToHost, s));
-        if (final_B) CK(cudaMemcpyAsync(final_B, dfin + count * 16, count * 128, cudaMemcpyDeviceToHost, s));
-        CK(cudaMemcpyAsync(hz.data(), dz, count * 384, cudaMemcpyDeviceToHost, s));
-        CK(cudaMemcpyAsync(hp.data(), dpair, count * 384, cudaMemcpyDeviceToHost, s));
-        return batch_check_flags(b, s);
-    };
-    rc = run();
-    if (rc) cudaStreamSynchronize(s);
-    release();
+    {
+        VerifyBuffers v;
+        rc = v.alloc(n, count, proof_len, true);
+        if (rc) return rc;
+        auto run = [&]() -> int {
+            CK(cudaMemcpyAsync(v.b.bytesA, A, total * 64, cudaMemcpyHostToDevice, s));
+            CK(cudaMemcpyAsync(v.b.bytesB, B, total * 128, cudaMemcpyHostToDevice, s));
+            CK(cudaMemcpyAsync(v.dproofs, proofs, count * proof_len * 384, cudaMemcpyHostToDevice, s));
+            int rc2 = batch_verify_enqueue(v, v.b.bytesA, v.b.bytesB, v.dproofs, n, count, proof_len, final_A || final_B, s);
+            if (rc2) return rc2;
+            if (final_A) CK(cudaMemcpyAsync(final_A, v.dfin, count * 64, cudaMemcpyDeviceToHost, s));
+            if (final_B) CK(cudaMemcpyAsync(final_B, v.dfin + count * 16, count * 128, cudaMemcpyDeviceToHost, s));
+            CK(cudaMemcpyAsync(hz.data(), v.dz, count * 384, cudaMemcpyDeviceToHost, s));
+            CK(cudaMemcpyAsync(hp.data(), v.dpair, count * 384, cudaMemcpyDeviceToHost, s));
+            return batch_check_flags(v.b, s);
+        };
+        rc = run();
+        if (rc) cudaStreamSynchronize(s);
+    }
     if (rc) return rc;
     for (size_t j = 0; j < count; j++) {
         // a proof with a coordinate >= p is one the reference could not have deserialised: refused on its own, like a bad A or B
@@ -510,6 +532,46 @@ int sipp_verify_native_batch(const uint8_t* A, const uint8_t* B, size_t n, size_
     }
     if (final_Z) memcpy(final_Z, hz.data(), count * 384);
     return SIPP_OK;
+}
+
+// sipp_verify_native_batch on the caller's device buffers, read in place; the outcome of every instance (k_verify_outcome) goes to
+// d_results and the finals only once the flags of the call were found clean.
+int sipp_verify_native_batch_device(const void* dA, const void* dB, size_t n, size_t count, const void* d_proofs, size_t proof_len, int* d_results,
+                                    void* d_final_A, void* d_final_B, void* d_final_Z) {
+    int rc = batch_args(dA, dB, n, count, d_proofs);  // every argument check before the device is touched
+    if (rc) return rc;
+    if (!d_results) return fail(SIPP_ERR_ARG, "null results");
+    const size_t np = sipp_proof_len(n);
+    if (proof_len < np) return fail(SIPP_ERR_SHORT_PROOF, "proof.pop().unwrap() on an empty proof");  // verifier_native.rs:31,40,42
+    rc = ensure_init();
+    if (rc) return rc;
+    cudaStream_t s = g_stream;
+    std::vector<RaggedProof> pt(count);  // the elements read of proof j: its last np
+    for (size_t j = 0; j < count; j++) pt[j] = RaggedProof{j * proof_len + proof_len - np, (uint32_t)np, 0};
+    VerifyBuffers v;
+    rc = v.alloc(n, count, proof_len, false);
+    if (rc) return rc;
+    RaggedProof* dpt = nullptr;
+    cudaError_t e = pool_alloc((void**)&dpt, count * sizeof(RaggedProof));
+    struct Release { RaggedProof* p; ~Release() { pool_free(p); } } release{dpt};
+    if (e != cudaSuccess) return cuda_fail(e, "cudaMalloc(verify batch)");
+    const uint32_t* proofs = (const uint32_t*)d_proofs;
+    auto run = [&]() -> int {
+        CK(order_after(s, cudaStreamLegacy));  // inputs just written on the legacy default stream (torch's, unless switched)
+        CK(cudaMemcpyAsync(dpt, pt.data(), count * sizeof(RaggedProof), cudaMemcpyHostToDevice, s));
+        int rc2 = batch_verify_enqueue(v, (const uint32_t*)dA, (const uint32_t*)dB, proofs, n, count, proof_len, d_final_A || d_final_B, s);
+        if (!rc2) rc2 = batch_check_flags(v.b, s);  // synchronises
+        if (rc2) return rc2;
+        int le = launch_verify_outcome(proofs, dpt, count, v.dz, v.dpair, v.dfin, true, d_results, (uint32_t*)d_final_A, (uint32_t*)d_final_B,
+                                       (uint32_t*)d_final_Z, s);
+        if (le) return cuda_fail((cudaError_t)le, "k_verify_outcome");
+        g_stats.launches++;
+        CK(cudaStreamSynchronize(s));
+        return SIPP_OK;
+    };
+    rc = run();
+    if (rc) cudaStreamSynchronize(s);
+    return rc;
 }
 
 // `count` independent Poseidon permutations on the device (test hook for k_transcript.cu)

@@ -1,5 +1,6 @@
 // k_misc.cu -- see kernels overview in device_common.cuh
 #include "device_common.cuh"
+#include "../../include/sipp_b200.h"
 
 namespace sipp {
 
@@ -27,6 +28,42 @@ __global__ void k_codec_encode(const uint32_t* __restrict__ in, uint32_t* __rest
     Fq c = fq_from_mont(m);
 #pragma unroll
     for (int k = 0; k < 8; k++) out[8 * i + k] = c.l[k];
+}
+
+// ------------------------------------------------------------------------------------------------ batched verifier outcome
+// The per-instance outcome of the _device batched verifiers (batch.cu, ragged.cu), launched once the flags of the call were found
+// clean.  One warp per instance j: the 12 np coordinates of its proof elements read, Fq12 [pt[j].first, pt[j].first + pt[j].np) of
+// `proofs`, must all be < p (the host forms' fq_bytes_canonical) -- the lanes stride over the coordinates, one 32-byte little-endian
+// integer each, and vote.  results[j] = SIPP_ERR_ENCODING when one is not, else SIPP_OK when z[j] == pair[j] (verifier_native.rs:81-84),
+// else SIPP_ERR_VERIFY.  Then the finals that are non-NULL, unless the proof was not canonical and !enc_finals: final_Z[j] <- z[j],
+// final_A[j] <- fin + 16 j, final_B[j] <- fin + 16 count + 32 j (words).
+__global__ void __launch_bounds__(128) k_verify_outcome(const uint32_t* __restrict__ proofs, const RaggedProof* __restrict__ pt, size_t count,
+                                                        const uint32_t* __restrict__ z, const uint32_t* __restrict__ pair,
+                                                        const uint32_t* __restrict__ fin, int enc_finals, int* __restrict__ results,
+                                                        uint32_t* __restrict__ final_A, uint32_t* __restrict__ final_B, uint32_t* __restrict__ final_Z) {
+    const size_t j = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) / 32;
+    const int lane = threadIdx.x & 31;
+    if (j >= count) return;  // whole warps
+    const RaggedProof t = pt[j];
+    const uint32_t* e = proofs + 96 * t.first;
+    const uint32_t P[8] = {SIPP_P0, SIPP_P1, SIPP_P2, SIPP_P3, SIPP_P4, SIPP_P5, SIPP_P6, SIPP_P7};
+    bool ok = true;
+    for (size_t c = lane; c < 12 * (size_t)t.np; c += 32) {
+        uint32_t w[8], d[8];
+#pragma unroll
+        for (int k = 0; k < 8; k++) w[k] = e[8 * c + k];
+        ok &= sub8(d, w, P) != 0;  // a borrow: w < p
+    }
+    const bool canonical = __all_sync(0xffffffffu, ok);
+    bool same = true;
+    for (int k = lane; k < 96; k += 32) same &= z[96 * j + k] == pair[96 * j + k];
+    same = __all_sync(0xffffffffu, same);
+    if (lane == 0) results[j] = !canonical ? SIPP_ERR_ENCODING : same ? SIPP_OK : SIPP_ERR_VERIFY;
+    if (!canonical && !enc_finals) return;
+    if (final_Z)
+        for (int k = lane; k < 96; k += 32) final_Z[96 * j + k] = z[96 * j + k];
+    if (final_A && lane < 16) final_A[16 * j + lane] = fin[16 * j + lane];
+    if (final_B) final_B[32 * j + lane] = fin[16 * count + 32 * j + lane];
 }
 
 // ------------------------------------------------------------------------------------------------ test hooks
@@ -146,6 +183,12 @@ int launch_codec_decode(const uint32_t* in, uint32_t* out, size_t n_fq, int* fla
 }
 int launch_codec_encode(const uint32_t* in, uint32_t* out, size_t n_fq, cudaStream_t s) {
     k_codec_encode<<<(unsigned)((n_fq + 255) / 256), 256, 0, s>>>(in, out, n_fq);
+    return (int)cudaGetLastError();
+}
+int launch_verify_outcome(const uint32_t* proofs, const RaggedProof* pt, size_t count, const uint32_t* z, const uint32_t* pair, const uint32_t* fin,
+                          bool enc_finals, int* results, uint32_t* final_A, uint32_t* final_B, uint32_t* final_Z, cudaStream_t s) {
+    k_verify_outcome<<<(unsigned)((count * 32 + 127) / 128), 128, 0, s>>>(proofs, pt, count, z, pair, fin, enc_finals ? 1 : 0, results, final_A,
+                                                                          final_B, final_Z);
     return (int)cudaGetLastError();
 }
 int launch_test_fq_op(int op, const uint32_t* a, const uint32_t* b, uint32_t* out, size_t count, cudaStream_t s) {

@@ -136,6 +136,12 @@ struct RaggedGt {
 int launch_gt_fold_ragged(const uint32_t* proofs, const RaggedGt* ent, size_t npow, size_t nz, const uint64_t* challenges, uint32_t* factors, cudaStream_t s);
 // gA[j] <- A[at[j]], gB[j] <- B[at[j]] (decoded points), j < count
 int launch_gather_points(const uint32_t* A, const uint32_t* B, const uint64_t* at, size_t count, uint32_t* gA, uint32_t* gB, cudaStream_t s);
+// outcome of the _device batched verifiers (k_misc.cu), instance j < count in the caller's order: results[j] = SIPP_ERR_ENCODING when a
+// coordinate of its proof elements read (pt[j]: Fq12 slots of `proofs`, boundary format) is >= p, else SIPP_OK / SIPP_ERR_VERIFY as
+// z[j] == pair[j] or not (Fq12 slots, encoded); then final_Z[j] <- z[j], final_A[j] / final_B[j] <- fin (count x 16 words of final_A,
+// then count x 32 of final_B), each when non-NULL, for every instance when enc_finals and otherwise for the canonical ones only
+int launch_verify_outcome(const uint32_t* proofs, const RaggedProof* pt, size_t count, const uint32_t* z, const uint32_t* pair, const uint32_t* fin,
+                          bool enc_finals, int* results, uint32_t* final_A, uint32_t* final_B, uint32_t* final_Z, cudaStream_t s);
 
 // BLS input producers (k_bls.cu): group 1 = G1 (16 words per point), 2 = G2 (32 words)
 size_t window_table_bytes(int group);

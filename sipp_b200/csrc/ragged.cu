@@ -368,19 +368,27 @@ int ragged_verify_args(const size_t* offsets, size_t count, const size_t* proof_
     return SIPP_OK;
 }
 
+// where sipp_verify_native_batch_ragged_device wants the outcome: device buffers in the caller's instance order (finals may be NULL)
+struct DeviceOutcome {
+    int* results;
+    uint32_t *final_A, *final_B, *final_Z;
+};
+
 // The whole verification on the device (verifier_native.rs:14-85 per instance, every instance in lock-step).  The challenges depend
 // only on A, B and the proofs (:33-45), so the transcript is replayed first, round by round over the active instances, and then:
 //   main stream  the folds of every round back to back (the prover's fold tables and kernels), the final points gathered in the
 //                caller's order and their pairings (:80) through the products path, one one-pair segment per instance;
 //   side stream  every GT update in one launch (k_gt_fold_ragged: 1 + log2 n_j factors per instance), one k_seg_product pass
 //                (1 + log2 n_j <= 32 <= SIPP_PRODUCT_SPAN factors per instance) and the encode: final_Z of every instance.
-// out: count x 384 B final_Z then count x 384 B pairings; fin: count x 64 B final_A then count x 128 B final_B (boundary bytes).
-int ragged_verify_run(const uint8_t* A, const uint8_t* B, size_t n, const size_t* offsets, size_t count, const uint8_t* proofs,
-                      const size_t* proof_offsets, uint8_t* out, uint8_t* fin) {
+// bytesA / bytesB / proofs: boundary bytes in device memory, only read.  Host outcome (dev NULL): out <- count x 384 B final_Z then
+// count x 384 B pairings, fin <- count x 64 B final_A then count x 128 B final_B (boundary bytes), copied with the flags.  Device
+// outcome: once the flags are clean, k_verify_outcome writes dev's results and finals (of the instances whose proof is canonical).
+int ragged_verify_run(const uint32_t* bytesA, const uint32_t* bytesB, size_t n, const size_t* offsets, size_t count, const uint32_t* proofs,
+                      const size_t* proof_offsets, uint8_t* out, uint8_t* fin, const DeviceOutcome* dev) {
     cudaStream_t s = g_stream;
     RaggedSchedule S;
     ragged_folds(offsets, count, S);
-    const size_t R = S.rounds.size() - 1, act1 = R ? S.rounds[1].act : 0, npow = S.tabs.size(), ptotal = proof_offsets[count];
+    const size_t R = S.rounds.size() - 1, act1 = R ? S.rounds[1].act : 0, npow = S.tabs.size();
     // per position k of the order: its proof (the last np_k elements of its slice), its factor slots [fbase[k], fbase[k] + 1 + log2 n_k)
     // -- Z, then the update of round r at fbase[k] + r -- and the task multiplying them into the slot nfac + (caller index)
     std::vector<RaggedProof> pt(count);
@@ -400,23 +408,22 @@ int ragged_verify_run(const uint8_t* A, const uint8_t* B, size_t n, const size_t
     for (size_t r = 1; r <= R; r++)
         for (size_t k = 0; k < S.rounds[r].act; k++)                                   // Z_L at np - 2r, Z_R at np - 1 - 2r  :40, :42
             gt[S.rounds[r].tab0 + k] = RaggedGt{pt[k].first + pt[k].np - 2 * r, (uint32_t)(fbase[k] + r), 0};
+    std::vector<RaggedProof> ot(dev ? count : 0);                                     // the device outcome's table: pt in the caller's order
+    for (size_t k = 0; k < ot.size(); k++) ot[S.order[k]] = pt[k];
     RaggedFinals fins;
     int rc = fins.prepare(offsets, count);
     if (rc) return rc;
-    uint32_t *bA = nullptr, *bB = nullptr, *dA = nullptr, *dB = nullptr, *dproofs = nullptr, *fac = nullptr;
+    uint32_t *dA = nullptr, *dB = nullptr, *fac = nullptr;
     uint32_t *res = nullptr, *enc = nullptr;
     uint64_t *states = nullptr, *chal = nullptr;
     FoldPlan* plans = nullptr;
     RaggedInst* dtabs = nullptr;
-    RaggedProof* dpt = nullptr;
+    RaggedProof *dpt = nullptr, *dot = nullptr;
     RaggedGt* dgt = nullptr;
     ProductTask* dftasks = nullptr;
     int* flags = nullptr;  // [0] transcript / recoding, [1] encoding
-    cudaError_t e = pool_alloc((void**)&bA, n * 64);
-    if (e == cudaSuccess) e = pool_alloc((void**)&bB, n * 128);
-    if (e == cudaSuccess) e = pool_alloc((void**)&dA, n * 64);
+    cudaError_t e = pool_alloc((void**)&dA, n * 64);
     if (e == cudaSuccess) e = pool_alloc((void**)&dB, n * 128);
-    if (e == cudaSuccess) e = pool_alloc((void**)&dproofs, ptotal * 384);
     if (e == cudaSuccess) e = pool_alloc((void**)&fac, (nfac + count) * 384);
     if (e == cudaSuccess) e = pool_alloc((void**)&res, 2 * count * 384);
     if (e == cudaSuccess) e = pool_alloc((void**)&enc, count * 192);
@@ -428,30 +435,29 @@ int ragged_verify_run(const uint8_t* A, const uint8_t* B, size_t n, const size_t
     if (e == cudaSuccess) e = pool_alloc((void**)&dgt, gt.size() * sizeof(RaggedGt));
     if (e == cudaSuccess) e = pool_alloc((void**)&dftasks, count * sizeof(ProductTask));
     if (e == cudaSuccess) e = pool_alloc((void**)&flags, 2 * sizeof(int));
+    if (e == cudaSuccess && dev) e = pool_alloc((void**)&dot, count * sizeof(RaggedProof));
     struct Release {
         std::vector<void*> p;
         ~Release() { for (void* q : p) pool_free(q); }
-    } release{{bA, bB, dA, dB, dproofs, fac, res, enc, states, chal, plans, dtabs, dpt, dgt, dftasks, flags}};
+    } release{{dA, dB, fac, res, enc, states, chal, plans, dtabs, dpt, dgt, dftasks, flags, dot}};
     if (e != cudaSuccess) return cuda_fail(e, "cudaMalloc(verify_native_batch_ragged)");
     if (!g_fold_stream) CK(cudaStreamCreateWithFlags(&g_fold_stream, cudaStreamNonBlocking));
     cudaStream_t side = g_fold_stream;
     bool forked = false;
     auto run = [&]() -> int {
         CK(cudaMemsetAsync(flags, 0, 2 * sizeof(int), s));
-        CK(cudaMemcpyAsync(bA, A, n * 64, cudaMemcpyHostToDevice, s));
-        CK(cudaMemcpyAsync(bB, B, n * 128, cudaMemcpyHostToDevice, s));
-        CK(cudaMemcpyAsync(dproofs, proofs, ptotal * 384, cudaMemcpyHostToDevice, s));
         if (npow) CK(cudaMemcpyAsync(dtabs, S.tabs.data(), npow * sizeof(RaggedInst), cudaMemcpyHostToDevice, s));
         CK(cudaMemcpyAsync(dpt, pt.data(), count * sizeof(RaggedProof), cudaMemcpyHostToDevice, s));
         CK(cudaMemcpyAsync(dgt, gt.data(), gt.size() * sizeof(RaggedGt), cudaMemcpyHostToDevice, s));
         CK(cudaMemcpyAsync(dftasks, ftasks.data(), count * sizeof(ProductTask), cudaMemcpyHostToDevice, s));
-        int le = ragged_decode_absorb(bA, bB, n, dA, dB, dtabs, act1, states, flags, s);  // round 1's table is the first
+        if (dev) CK(cudaMemcpyAsync(dot, ot.data(), count * sizeof(RaggedProof), cudaMemcpyHostToDevice, s));
+        int le = ragged_decode_absorb(bytesA, bytesB, n, dA, dB, dtabs, act1, states, flags, s);  // round 1's table is the first
         if (le) return le;
         // the transcript replay: round r's fold plans and challenges x || x^-1 to its slices  :33 (first round), :40-46
         for (size_t r = 1; r <= R; r++) {
             const RaggedRound& rd = S.rounds[r];
             Span sp(3, s);
-            le = launch_tr_round_ragged(states, dproofs, dpt, (int)r, g_opt_fq12_order, (unsigned)rd.act, plans + rd.tab0, chal + 8 * rd.tab0, flags, s);
+            le = launch_tr_round_ragged(states, proofs, dpt, (int)r, g_opt_fq12_order, (unsigned)rd.act, plans + rd.tab0, chal + 8 * rd.tab0, flags, s);
             if (le) return cuda_fail((cudaError_t)le, "k_tr_round_ragged");
             g_stats.launches++;
         }
@@ -460,7 +466,7 @@ int ragged_verify_run(const uint8_t* A, const uint8_t* B, size_t n, const size_t
         forked = true;
         {
             Span sp(1, side);
-            le = launch_gt_fold_ragged(dproofs, dgt, npow, count, chal, fac, side);
+            le = launch_gt_fold_ragged(proofs, dgt, npow, count, chal, fac, side);
             if (le) return cuda_fail((cudaError_t)le, "k_gt_fold_ragged");
             le = launch_seg_product(dftasks, count, fac, side);
             if (le) return cuda_fail((cudaError_t)le, "k_seg_product");
@@ -486,10 +492,18 @@ int ragged_verify_run(const uint8_t* A, const uint8_t* B, size_t n, const size_t
         CK(order_after(s, side));  // join
         int fl[2] = {0, 0};
         CK(cudaMemcpyAsync(fl, flags, sizeof fl, cudaMemcpyDeviceToHost, s));
-        CK(cudaMemcpyAsync(out, res, 2 * count * 384, cudaMemcpyDeviceToHost, s));
-        CK(cudaMemcpyAsync(fin, enc, count * 192, cudaMemcpyDeviceToHost, s));
+        if (!dev) {
+            CK(cudaMemcpyAsync(out, res, 2 * count * 384, cudaMemcpyDeviceToHost, s));
+            CK(cudaMemcpyAsync(fin, enc, count * 192, cudaMemcpyDeviceToHost, s));
+        }
         CK(cudaStreamSynchronize(s));
-        return ragged_flags_status(fl);
+        const int st = ragged_flags_status(fl);
+        if (st || !dev) return st;
+        le = launch_verify_outcome(proofs, dot, count, res, res + count * 96, enc, false, dev->results, dev->final_A, dev->final_B, dev->final_Z, s);
+        if (le) return cuda_fail((cudaError_t)le, "k_verify_outcome");
+        g_stats.launches++;
+        CK(cudaStreamSynchronize(s));
+        return SIPP_OK;
     };
     rc = run();
     if (rc) {  // neither stream may still use a block when the pool recycles it
@@ -550,7 +564,22 @@ int sipp_verify_native_batch_ragged(const uint8_t* A, size_t a_len, const uint8_
     rc = ensure_init();
     if (rc) return rc;
     std::vector<uint8_t> out(2 * count * 384), fin(count * 192);
-    rc = ragged_verify_run(A, B, a_len, offsets, count, proofs, proof_offsets, out.data(), fin.data());
+    {
+        const size_t ptotal = proof_offsets[count];
+        uint32_t *bA = nullptr, *bB = nullptr, *dproofs = nullptr;
+        cudaError_t e = pool_alloc((void**)&bA, a_len * 64);
+        if (e == cudaSuccess) e = pool_alloc((void**)&bB, a_len * 128);
+        if (e == cudaSuccess) e = pool_alloc((void**)&dproofs, ptotal * 384);
+        struct Release {
+            uint32_t *a, *b, *p;
+            ~Release() { pool_free(a); pool_free(b); pool_free(p); }
+        } release{bA, bB, dproofs};  // recycled: later work on g_stream only
+        if (e != cudaSuccess) return cuda_fail(e, "cudaMalloc(verify_native_batch_ragged)");
+        CK(cudaMemcpyAsync(bA, A, a_len * 64, cudaMemcpyHostToDevice, g_stream));
+        CK(cudaMemcpyAsync(bB, B, a_len * 128, cudaMemcpyHostToDevice, g_stream));
+        CK(cudaMemcpyAsync(dproofs, proofs, ptotal * 384, cudaMemcpyHostToDevice, g_stream));
+        rc = ragged_verify_run(bA, bB, a_len, offsets, count, dproofs, proof_offsets, out.data(), fin.data(), nullptr);
+    }
     if (rc) return rc;
     for (size_t j = 0; j < count; j++) {
         // a proof with a coordinate >= p is one the reference could not have deserialised: refused on its own, like a bad A or B
@@ -565,6 +594,20 @@ int sipp_verify_native_batch_ragged(const uint8_t* A, size_t a_len, const uint8_
         if (final_Z) memcpy(final_Z + 384 * j, &out[384 * j], 384);
     }
     return SIPP_OK;
+}
+
+int sipp_verify_native_batch_ragged_device(const void* dA, const void* dB, size_t n, const size_t* offsets, size_t count, const void* d_proofs,
+                                           const size_t* proof_offsets, int* d_results, void* d_final_A, void* d_final_B, void* d_final_Z) {
+    int rc = ragged_args(dA, n, dB, n, offsets, count, d_proofs);
+    if (rc) return rc;
+    rc = ragged_verify_args(offsets, count, proof_offsets, d_results);
+    if (rc) return rc;
+    rc = ensure_init();
+    if (rc) return rc;
+    CK(order_after(g_stream, cudaStreamLegacy));  // inputs just written on the legacy default stream (torch's, unless switched)
+    const DeviceOutcome dev{d_results, (uint32_t*)d_final_A, (uint32_t*)d_final_B, (uint32_t*)d_final_Z};
+    return ragged_verify_run((const uint32_t*)dA, (const uint32_t*)dB, n, offsets, count, (const uint32_t*)d_proofs, proof_offsets, nullptr, nullptr,
+                             &dev);
 }
 
 // host-only schedule of a ragged batch (no GPU needed) under the current options: 5 words per round r = 0 .. log2 max n_j -- active
