@@ -212,6 +212,40 @@ int sipp_inner_product_batch_device(const void *dA, const void *dB, size_t n, co
 /* out[j] = pairing(a_j, b_j)  (verifier_native.rs:80) for j < count: the batch above with one pair per segment */
 int sipp_pairing_batch(const uint8_t *a, const uint8_t *b, size_t count, uint8_t *out);
 
+/* ---- batched multi-scalar multiplications: many independent MSMs of unequal lengths in G1 and G2 in one call ----------------- */
+/* count independent MSMs, CSR segments: out[j] = sum_{offsets[j] <= i < offsets[j+1]} [k_i] P_i.
+ *   - Formats: points in the boundary format (G1 64 B, G2 128 B; the identity is all-zero bytes), scalars 32 B little-endian integers,
+ *     one per point.  out: count x 64 B (G1) or count x 128 B (G2) canonical affine points; an empty segment, or a sum that is the
+ *     identity, gives all-zero bytes.  The results are canonical group elements: every out[j] is byte-identical to the sum of the
+ *     [k_i] P_i of its segment computed any other way.
+ *   - offsets: count + 1 HOST entries, offsets[0] = 0, non-decreasing, offsets[count] = n (as sipp_inner_product_batch).
+ *     count == 0 with n == 0 returns what sipp_init(0) would (SIPP_ERR_CUDA without a device) and writes nothing.
+ *   - SIPP_ERR_ARG: a NULL pointer (count > 0), bad offsets, count == 0 with n > 0, or n > 2^32 - 1; all before the device is touched.
+ *     Valid arguments without a device give SIPP_ERR_CUDA.
+ *   - Host forms: a scalar >= r, then a coordinate >= p, is refused on the host with SIPP_ERR_ENCODING before the device is touched.
+ *     Device forms: the same checks run on the device; a failure fails the whole call with SIPP_ERR_ENCODING and nothing is written
+ *     to d_out.  Both forms report the first failure in this order: a scalar >= r, a coordinate >= p, a point off the curve, a G2
+ *     point outside the subgroup (sipp_last_error names it).  With SIPP_OPT_VALIDATE_POINTS = 1 (default) a point off the curve, or a G2 point outside the order-r subgroup, is
+ *     refused the same way; with 0 the caller guarantees the points, and results for points outside the r-torsion are unspecified
+ *     (the kernels use the GLV / GLS endomorphisms, which act as scalars only there).
+ *   - Path per segment, chosen from its length alone (sipp_test_msm_plan shows it): fewer than 13 (G1) or 8 (G2) points, Straus (one thread per
+ *     segment, doublings shared by the 2 (G1) or 4 (G2) GLV / GLS sub-scalars of all its points); from there on, Pippenger with
+ *     signed c-bit windows, c from 5 to 16 growing with the length.
+ *   - Device scratch, returned to the library's pool on return, per point: NC W sort entries of 16 B (keys and values, double-buffered
+ *     for the sort) with their chunk partials (12 B per entry in G1, 24 B in G2), NC terms (64 B G1, 128 B G2) and, when its segment
+ *     takes the Straus path, NC x 44 B of NAF digits; NC = 2 (G1) or 4 (G2), W = 128 / c + 1 (G1) or 66 / c + 1 (G2) windows, at most
+ *     26 / 14 -- about 2.1 KB per G1 point and 3.4 KB per G2 point at most -- plus W 2^(c-1) Jacobian buckets (96 B G1, 192 B G2) per
+ *     Pippenger segment and the sort's own scratch.  More than 2^31 terms, sort entries or buckets, or more than 2^32 - 1 segments,
+ *     give SIPP_ERR_CUDA; calls of 2^20 points per group are supported.
+ *   - The device forms: points, scalars and d_out in DEVICE memory (4-byte aligned); offsets stay on the host.  Before reading any
+ *     input the library stream waits for the legacy default stream, so inputs just written there need no synchronisation; the call
+ *     returns once d_out is complete.  No option other than SIPP_OPT_VALIDATE_POINTS is read; sipp_stats.launches grows, no other
+ *     counter changes. */
+int sipp_g1_msm_batch(const uint8_t *points, const uint8_t *scalars, size_t n, const size_t *offsets, size_t count, uint8_t *out);
+int sipp_g2_msm_batch(const uint8_t *points, const uint8_t *scalars, size_t n, const size_t *offsets, size_t count, uint8_t *out);
+int sipp_g1_msm_batch_device(const void *d_points, const void *d_scalars, size_t n, const size_t *offsets, size_t count, void *d_out);
+int sipp_g2_msm_batch_device(const void *d_points, const void *d_scalars, size_t n, const size_t *offsets, size_t count, void *d_out);
+
 /* ---- Fiat-Shamir transcript (host; Poseidon over Goldilocks)  transcript_native.rs:14-66 ---------------- */
 typedef struct { uint64_t state[4]; } sipp_transcript;
 void sipp_transcript_new(sipp_transcript *t);                                          /* :19-23 */
@@ -485,6 +519,15 @@ long sipp_test_product_plan(const size_t *offsets, size_t count, int kpg_max, si
  * in their ragged forms) and line-table chunks -- to `out` when out_cap >= 5 x rounds; returns the number of rounds or a negative
  * sipp_status (the argument checks of sipp_prove_native_batch_ragged) */
 long sipp_test_ragged_schedule(const size_t *offsets, size_t count, long long *out, size_t out_cap);
+/* the plan of sipp_g1_msm_batch / sipp_g2_msm_batch (host logic only): 4 words per segment -- G1 path (0 Straus, 1 Pippenger), G1 window
+ * bits (0 for Straus), G2 path, G2 window bits -- to `out` when out_cap >= 4 x count; returns count or a negative sipp_status (the
+ * offsets checks of the entry points) */
+long sipp_test_msm_plan(const size_t *offsets, size_t count, int *out, size_t out_cap);
+/* sipp_g1_msm_batch_device (group 1) / sipp_g2_msm_batch_device (group 2) with every non-empty segment forced onto one path: c = 0 Straus,
+ * 5 <= c <= 16 Pippenger with c-bit windows (another c or group: SIPP_ERR_ARG).  The outputs are the same bytes; for timing both paths
+ * at one segment length (tools/msm_time.py). */
+int sipp_test_msm_batch_device(int group, int c, const void *d_points, const void *d_scalars, size_t n, const size_t *offsets, size_t count,
+                               void *d_out);
 long sipp_test_poseidon_chain(uint64_t seed, long count);
 int sipp_test_poseidon_scalar(int which, const uint64_t *in, uint64_t *out);
 /* the derived tables of the host Poseidon (sipp::PoseidonFastTables, poseidon_fast.h), for tools/probe/poseidon_lab.cc */

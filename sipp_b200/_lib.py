@@ -141,6 +141,13 @@ def load():
     lib.sipp_g2_sum.argtypes = [u8p, sz, u8p]
     lib.sipp_g2_sum_device.argtypes = [vp, sz, vp]
     lib.sipp_g1_neg_generator.argtypes = [u8p]
+    for name in ("sipp_g1_msm_batch", "sipp_g2_msm_batch"):
+        getattr(lib, name).argtypes = [u8p, u8p, sz, szp, sz, u8p]
+    for name in ("sipp_g1_msm_batch_device", "sipp_g2_msm_batch_device"):
+        getattr(lib, name).argtypes = [vp, vp, sz, szp, sz, vp]
+    lib.sipp_test_msm_plan.argtypes = [szp, sz, ctypes.POINTER(ctypes.c_int), sz]
+    lib.sipp_test_msm_plan.restype = ctypes.c_long
+    lib.sipp_test_msm_batch_device.argtypes = [i, i, vp, vp, sz, szp, sz, vp]
     lib.sipp_comm_get_unique_id.argtypes = [u8p]
     lib.sipp_comm_init.argtypes = [u8p, i, i]
     lib.sipp_comm_init_host.argtypes = [i, i, ALLGATHER_FN, BROADCAST_FN, vp]

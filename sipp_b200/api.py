@@ -588,6 +588,47 @@ def g1_neg_generator() -> bytes:
     return out.raw
 
 
+# ---- batched multi-scalar multiplications -----------------------------------------------------------------------------------
+def _msm_batch(group: int, points: Points, scalars: Points, lengths: Sequence[int]) -> List[bytes]:
+    size = G1_BYTES if group == 1 else G2_BYTES
+    p, k = _flat(points, size), _flat(scalars, FR_BYTES)
+    n = len(p) // size
+    if len(k) // FR_BYTES != n:
+        raise ValueError("%d points but %d scalars" % (n, len(k) // FR_BYTES))
+    offs = _offsets(lengths, n)
+    count = len(offs) - 1
+    _lib.require_gpu_once()
+    out = ctypes.create_string_buffer(max(1, size * count))
+    fn = _lib.load().sipp_g1_msm_batch if group == 1 else _lib.load().sipp_g2_msm_batch
+    _lib.check(fn(p, k, n, offs, count, out))
+    return _split(out.raw[:size * count], size)
+
+
+def g1_msm_batch(points: Points, scalars: Points, lengths: Sequence[int]) -> List[bytes]:
+    """[sum of [k_i] P_i over segment j for j < len(lengths)] in G1 in one call (sipp_g1_msm_batch): segment j holds the next
+    lengths[j] (point, scalar) pairs, an empty segment gives the identity (all-zero bytes)"""
+    return _msm_batch(1, points, scalars, lengths)
+
+
+def g2_msm_batch(points: Points, scalars: Points, lengths: Sequence[int]) -> List[bytes]:
+    """g1_msm_batch in G2 (sipp_g2_msm_batch)"""
+    return _msm_batch(2, points, scalars, lengths)
+
+
+def g1_msm_batch_device(d_points: int, d_scalars: int, n: int, lengths: Sequence[int], d_out: int) -> None:
+    """g1_msm_batch on DEVICE buffers (integer pointers): d_points n x 64 B, d_scalars n x 32 B, d_out len(lengths) x 64 B"""
+    offs = _offsets(lengths, n)
+    _lib.require_gpu_once()
+    _lib.check(_lib.load().sipp_g1_msm_batch_device(d_points, d_scalars, n, offs, len(offs) - 1, d_out))
+
+
+def g2_msm_batch_device(d_points: int, d_scalars: int, n: int, lengths: Sequence[int], d_out: int) -> None:
+    """g2_msm_batch on DEVICE buffers: d_points n x 128 B, d_scalars n x 32 B, d_out len(lengths) x 128 B"""
+    offs = _offsets(lengths, n)
+    _lib.require_gpu_once()
+    _lib.check(_lib.load().sipp_g2_msm_batch_device(d_points, d_scalars, n, offs, len(offs) - 1, d_out))
+
+
 def seeded_inputs(seed: int, n: int):
     """A_i = [a_i]G1, B_i = [b_i]G2 with the documented SplitMix64 scalar stream, generated on the GPU."""
     _lib.require_gpu_once()

@@ -322,9 +322,10 @@ __device__ bool jac_equal(const Jac<Fq2>& p, const Jac<Fq2>& q) {
     if (!fq2_eq(f_mul(p.x, z2), f_mul(q.x, z1))) return false;
     return fq2_eq(f_mul(p.y, f_mul(z2, q.z)), f_mul(q.y, f_mul(z1, p.z)));
 }
-__global__ void __launch_bounds__(64) k_validate_points(const uint32_t* __restrict__ dA, const uint32_t* __restrict__ dB, size_t n, int* __restrict__ flags) {
+__global__ void __launch_bounds__(64) k_validate_points(const uint32_t* __restrict__ dA, size_t n, const uint32_t* __restrict__ dB, size_t nb,
+                                                         int* __restrict__ flags) {
     const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= 2 * n) return;
+    if (t >= n + nb) return;
     if (t < n) {
         const G1A p{load_fq_words(dA + 16 * t), load_fq_words(dA + 16 * t + 8)};
         if (affine_is_identity(p)) return;
@@ -346,7 +347,10 @@ __global__ void __launch_bounds__(64) k_validate_points(const uint32_t* __restri
     if (!jac_equal(lhs, rhs)) atomicOr(flags, 4);
 }
 int launch_validate_points(const uint32_t* dA, const uint32_t* dB, size_t n, int* flags, cudaStream_t s) {
-    k_validate_points<<<(unsigned)((2 * n + 63) / 64), 64, 0, s>>>(dA, dB, n, flags);
+    return launch_validate_points_groups(dA, n, dB, n, flags, s);
+}
+int launch_validate_points_groups(const uint32_t* dA, size_t na, const uint32_t* dB, size_t nb, int* flags, cudaStream_t s) {
+    k_validate_points<<<(unsigned)((na + nb + 63) / 64), 64, 0, s>>>(dA, na, dB, nb, flags);
     return (int)cudaGetLastError();
 }
 

@@ -41,6 +41,8 @@ int launch_fold(uint32_t* A, uint32_t* B, size_t h, const FoldPlan& plan, cudaSt
 int launch_fold_wide(uint32_t* A, uint32_t* B, size_t h, const FoldPlan& plan, cudaStream_t s);
 // on-curve + G2 subgroup check of decoded points: flags |= 2 (off the curve), |= 4 (outside the prime-order subgroup)
 int launch_validate_points(const uint32_t* dA, const uint32_t* dB, size_t n, int* flags, cudaStream_t s);
+// the same check of na G1 points dA and nb G2 points dB (either may be 0)
+int launch_validate_points_groups(const uint32_t* dA, size_t na, const uint32_t* dB, size_t nb, int* flags, cudaStream_t s);
 int launch_test_fq_op(int op, const uint32_t* a, const uint32_t* b, uint32_t* out, size_t count, cudaStream_t s);
 int launch_test_fq12_op(int op, const uint32_t* a, const uint32_t* b, uint32_t* out, size_t count, cudaStream_t s);
 int launch_microbench(int which, int blocks, int threads, void* out, int iters, uint32_t seed, double* ops_per_thread, cudaStream_t s);
@@ -152,5 +154,36 @@ int g2_sum_blocks(size_t count, int sm_count);
 int launch_g2_sum(const uint32_t* points, size_t count, uint32_t* partials, int blocks, uint32_t* out, cudaStream_t s);
 int launch_seeded_scalars(uint64_t seed, size_t n, uint32_t* sa, uint32_t* sb, cudaStream_t s);
 int launch_generators(uint32_t* gens, cudaStream_t s);
+
+// batched multi-scalar multiplications (k_msm.cu, host driver msm.cu, algorithm msm.cuh); group 1 = G1, 2 = G2.  A segment is
+// points [first, first + len); c = 0 runs it on the Straus path, c > 0 on the Pippenger path with c-bit windows: its sort entries
+// start at ebase (W = msm::windows(bits, c) per term), its buckets at bbase (2^(c-1) per window), the partial sums of its windows at
+// wbase (`parts` per window, window-major).
+struct MsmSeg {
+    uint32_t first, len, c, ebase, bbase, wbase, parts, pad;
+};
+// one block of k_msm_windows: buckets [lo, lo + count) of the window whose first bucket is bucket0 (weights lo + 1 ...)
+struct MsmWin {
+    uint32_t bucket0, lo, count, pad;
+};
+size_t msm_term_bytes(int group);  // one affine term
+size_t msm_jac_bytes(int group);   // one Jacobian bucket / partial
+int launch_msm_recode(int group, const uint32_t* points, const uint32_t* scalars, uint32_t n, const MsmSeg* segs, uint32_t count, void* terms,
+                      FoldComp* naf, uint32_t* keys, uint32_t* vals, uint32_t nbuckets, int* flags, cudaStream_t s);
+int msm_sort(void* temp, size_t* temp_bytes, const uint32_t* keys_in, uint32_t* keys_out, const uint32_t* vals_in, uint32_t* vals_out, uint32_t entries,
+             int key_bits, cudaStream_t s);
+#define SIPP_MSM_CHUNK 16      // sorted entries per thread of k_msm_chunks
+#define SIPP_MSM_LONG_SPAN 64   // a bucket over more chunks than this is summed by blocks (k_msm_long_buckets), not by one thread
+#define SIPP_MSM_LONG_PARTS 64  // blocks per such bucket
+// buckets (nbuckets Jacobian points, zeroed by the caller: empty buckets stay the identity) from the sorted entries; first / last: 2 x
+// ceil(entries / SIPP_MSM_CHUNK) Jacobian partials of scratch; long_list: msm_long_list_words(entries) words of scratch; long_parts:
+// (msm_long_list_words(entries) - 1) x SIPP_MSM_LONG_PARTS Jacobian points of scratch
+size_t msm_long_list_words(uint32_t entries);
+int launch_msm_buckets(int group, const uint32_t* keys, const uint32_t* vals, uint32_t entries, uint32_t nbuckets, const void* terms, void* buckets,
+                       void* first, void* last, uint32_t* long_list, void* long_parts, cudaStream_t s);
+int launch_msm_windows(int group, const void* buckets, const MsmWin* wins, uint32_t nwins, void* parts, cudaStream_t s);
+int launch_msm_finish(int group, const void* parts, const MsmSeg* segs, const uint32_t* idx, uint32_t nseg, uint32_t* out, cudaStream_t s);
+int launch_msm_straus(int group, const void* terms, const FoldComp* naf, const MsmSeg* segs, const uint32_t* idx, uint32_t nseg, uint32_t* out,
+                      cudaStream_t s);
 
 }  // namespace sipp
