@@ -246,6 +246,37 @@ int sipp_g2_msm_batch(const uint8_t *points, const uint8_t *scalars, size_t n, c
 int sipp_g1_msm_batch_device(const void *d_points, const void *d_scalars, size_t n, const size_t *offsets, size_t count, void *d_out);
 int sipp_g2_msm_batch_device(const void *d_points, const void *d_scalars, size_t n, const size_t *offsets, size_t count, void *d_out);
 
+/* ---- batched multi-exponentiations in GT (Fq12): many independent products of powers of unequal lengths in one call --------------- */
+/* count independent multi-exponentiations, CSR segments: out[j] = prod_{offsets[j] <= i < offsets[j+1]} g_i^(k_i), computed in Fq12 as a
+ * field, exactly as the reference's `Z_L.pow(x)` (square-and-multiply over the bits of the integer) followed by products.  Products in
+ * Fq12 are exact, so every out[j] is byte-identical to that computation for EVERY Fq12 input: elements outside GT, non-units and zero
+ * (0^0 = 1, 0^k = 0 for k >= 1) included.  No GT membership is assumed or checked.
+ *   - Formats: elements in the boundary format (Fq12, 384 B, arkworks nested order), scalars 32 B little-endian integers, one per element.
+ *     out: count x 384 B; an empty segment gives Fq12::one().
+ *   - offsets: count + 1 HOST entries, offsets[0] = 0, non-decreasing, offsets[count] = n (as sipp_inner_product_batch).
+ *     count == 0 with n == 0 returns what sipp_init(0) would (SIPP_ERR_CUDA without a device) and writes nothing.
+ *   - SIPP_ERR_ARG: a NULL pointer (count > 0), bad offsets, count == 0 with n > 0, or n > 2^32 - 1; all before the device is touched.
+ *     Valid arguments without a device give SIPP_ERR_CUDA.
+ *   - Host form: a scalar >= r, then a coordinate >= p, is refused on the host with SIPP_ERR_ENCODING before the device is touched.
+ *     Device form: the same checks run on the device; a failure fails the whole call with SIPP_ERR_ENCODING and nothing is written to
+ *     d_out.  Both forms report the first failure in this order: a scalar >= r, then a coordinate >= p (sipp_last_error names it).
+ *   - Path per segment, chosen from its length alone (sipp_test_gt_msm_plan shows it): fewer than 512 elements, one generic power per
+ *     element (6 lanes each) and a segmented product; from there on, Pippenger with unsigned c-bit windows (ceil(254 / c) windows of
+ *     2^c - 1 buckets), c from 2 to 16 growing with the length.  No Frobenius split, cyclotomic squaring or inverse is used.
+ *   - Device scratch, returned to the library's pool on return, per element: 384 B (decoded table) and, on the short path, 32 B; on the
+ *     Pippenger path W sort entries of 16 B (keys and values, double-buffered for the sort) with 48 B of chunk partials each, W =
+ *     ceil(254 / c) (at most 127; 16 at 2^20 elements); per Pippenger segment W (2^c - 1) buckets and W ceil((2^c - 1) / 512) window
+ *     partials of 384 B (about 400 MB for one segment of 2^20 elements); plus the sort's own scratch.  More than 2^31 - 1 elements, sort
+ *     entries or buckets, more than 2^32 - 1 segments, or scratch the device cannot hold, give SIPP_ERR_CUDA with a message and write
+ *     nothing; calls of 2^20 elements are supported.
+ *   - The device form: elements, scalars and d_out in DEVICE memory (4-byte aligned; inputs are read one word at a time); offsets stay on
+ *     the host.  Before reading any input the library stream waits for the legacy default stream, so inputs just written there need no
+ *     synchronisation; the call returns once d_out is complete; copies use cudaMemcpyAsync.
+ *   - No option is read (SIPP_OPT_VALIDATE_POINTS included: there are no points, and the encoding checks always run; no pairing or
+ *     transcript is involved, so the H1 / H2 switches do not apply).  sipp_stats.launches grows, no other counter changes. */
+int sipp_gt_msm_batch(const uint8_t *elems, const uint8_t *scalars, size_t n, const size_t *offsets, size_t count, uint8_t *out);
+int sipp_gt_msm_batch_device(const void *d_elems, const void *d_scalars, size_t n, const size_t *offsets, size_t count, void *d_out);
+
 /* ---- Fiat-Shamir transcript (host; Poseidon over Goldilocks)  transcript_native.rs:14-66 ---------------- */
 typedef struct { uint64_t state[4]; } sipp_transcript;
 void sipp_transcript_new(sipp_transcript *t);                                          /* :19-23 */
@@ -528,6 +559,12 @@ long sipp_test_msm_plan(const size_t *offsets, size_t count, int *out, size_t ou
  * at one segment length (tools/msm_time.py). */
 int sipp_test_msm_batch_device(int group, int c, const void *d_points, const void *d_scalars, size_t n, const size_t *offsets, size_t count,
                                void *d_out);
+/* the plan of sipp_gt_msm_batch (host logic only): 2 words per segment -- path (0 short, 1 Pippenger), window bits (0 for the short
+ * path) -- to `out` when out_cap >= 2 x count; returns count or a negative sipp_status (the offsets checks of the entry points) */
+long sipp_test_gt_msm_plan(const size_t *offsets, size_t count, int *out, size_t out_cap);
+/* sipp_gt_msm_batch_device with every non-empty segment forced onto one path: c = 0 the short path, 2 <= c <= 16 Pippenger with c-bit
+ * windows (another c: SIPP_ERR_ARG).  The outputs are the same bytes; for timing both paths at one segment length (tools/gt_msm_time.py). */
+int sipp_test_gt_msm_batch_device(int c, const void *d_elems, const void *d_scalars, size_t n, const size_t *offsets, size_t count, void *d_out);
 long sipp_test_poseidon_chain(uint64_t seed, long count);
 int sipp_test_poseidon_scalar(int which, const uint64_t *in, uint64_t *out);
 /* the derived tables of the host Poseidon (sipp::PoseidonFastTables, poseidon_fast.h), for tools/probe/poseidon_lab.cc */

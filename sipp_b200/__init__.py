@@ -5,7 +5,7 @@ mirror of the reference interface used by the tests and bench.py.  Nothing here 
 Poseidon transcript, which the reference also keeps on the host.
 """
 from .api import (ProverContext, SIPPStatement, Transcript, VerificationError, combine_partials, fr_inverse,  # noqa: F401
-                  g1_generator_mul_batch, g1_msm_batch, g1_msm_batch_device, g1_neg_generator, g2_msm_batch, g2_msm_batch_device, g2_mul_batch, g2_sum, inner_product, inner_product_batch, inner_product_batch_device,
+                  g1_generator_mul_batch, g1_msm_batch, g1_msm_batch_device, g1_neg_generator, g2_msm_batch, g2_msm_batch_device, g2_mul_batch, g2_sum, gt_msm_batch, gt_msm_batch_device, inner_product, inner_product_batch, inner_product_batch_device,
                   pairing, pairing_batch, seeded_inputs, set_option, sipp_prove_native, sipp_prove_native_batch,
                   sipp_prove_native_batch_ragged, sipp_prove_native_batch_ragged_device, sipp_prove_native_batch_ragged_statement,
                   sipp_prove_native_batch_ragged_statement_device, sipp_prove_native_batch_statement, sipp_prove_native_batch_statement_device,

@@ -148,6 +148,11 @@ def load():
     lib.sipp_test_msm_plan.argtypes = [szp, sz, ctypes.POINTER(ctypes.c_int), sz]
     lib.sipp_test_msm_plan.restype = ctypes.c_long
     lib.sipp_test_msm_batch_device.argtypes = [i, i, vp, vp, sz, szp, sz, vp]
+    lib.sipp_gt_msm_batch.argtypes = [u8p, u8p, sz, szp, sz, u8p]
+    lib.sipp_gt_msm_batch_device.argtypes = [vp, vp, sz, szp, sz, vp]
+    lib.sipp_test_gt_msm_plan.argtypes = [szp, sz, ctypes.POINTER(ctypes.c_int), sz]
+    lib.sipp_test_gt_msm_plan.restype = ctypes.c_long
+    lib.sipp_test_gt_msm_batch_device.argtypes = [i, vp, vp, sz, szp, sz, vp]
     lib.sipp_comm_get_unique_id.argtypes = [u8p]
     lib.sipp_comm_init.argtypes = [u8p, i, i]
     lib.sipp_comm_init_host.argtypes = [i, i, ALLGATHER_FN, BROADCAST_FN, vp]

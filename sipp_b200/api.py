@@ -629,6 +629,29 @@ def g2_msm_batch_device(d_points: int, d_scalars: int, n: int, lengths: Sequence
     _lib.check(_lib.load().sipp_g2_msm_batch_device(d_points, d_scalars, n, offs, len(offs) - 1, d_out))
 
 
+# ---- batched multi-exponentiations in GT (Fq12) ------------------------------------------------------------------------------
+def gt_msm_batch(elems: Points, scalars: Points, lengths: Sequence[int]) -> List[bytes]:
+    """[product of g_i^(k_i) over segment j for j < len(lengths)] in Fq12 in one call (sipp_gt_msm_batch): segment j holds the next
+    lengths[j] (element, scalar) pairs, an empty segment gives Fq12::one().  Generic Fq12 arithmetic: any Fq12 is a valid element."""
+    g, k = _flat(elems, FQ12_BYTES), _flat(scalars, FR_BYTES)
+    n = len(g) // FQ12_BYTES
+    if len(k) // FR_BYTES != n:
+        raise ValueError("%d elements but %d scalars" % (n, len(k) // FR_BYTES))
+    offs = _offsets(lengths, n)
+    count = len(offs) - 1
+    _lib.require_gpu_once()
+    out = ctypes.create_string_buffer(max(1, FQ12_BYTES * count))
+    _lib.check(_lib.load().sipp_gt_msm_batch(g, k, n, offs, count, out))
+    return _split(out.raw[:FQ12_BYTES * count], FQ12_BYTES)
+
+
+def gt_msm_batch_device(d_elems: int, d_scalars: int, n: int, lengths: Sequence[int], d_out: int) -> None:
+    """gt_msm_batch on DEVICE buffers (integer pointers): d_elems n x 384 B, d_scalars n x 32 B, d_out len(lengths) x 384 B"""
+    offs = _offsets(lengths, n)
+    _lib.require_gpu_once()
+    _lib.check(_lib.load().sipp_gt_msm_batch_device(d_elems, d_scalars, n, offs, len(offs) - 1, d_out))
+
+
 def seeded_inputs(seed: int, n: int):
     """A_i = [a_i]G1, B_i = [b_i]G2 with the documented SplitMix64 scalar stream, generated on the GPU."""
     _lib.require_gpu_once()

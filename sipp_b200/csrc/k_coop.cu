@@ -372,6 +372,25 @@ __global__ void __launch_bounds__(SIPP_ACCUM_THREADS) k_gt_fold_ragged(const uin
     if (have && which == 0) store_fq2_words(factors + (size_t)en.dst * 96 + k * 16, r);
 }
 
+// GT multi-exponentiation, short path (msm.cu, sipp_gt_msm_batch): table[i] <- table[i]^k_i in place for i = idx[g], one 6-lane group
+// per element (coop_pow254: generic square-and-multiply, so every Fq12 is a valid base).  table: Fq12 slots of 96 words in the layout of
+// k_seg_product; sc: the scalars, 4 u64 per element.
+__global__ void __launch_bounds__(SIPP_ACCUM_THREADS) k_gt_msm_pow(uint32_t* __restrict__ table, const uint64_t* __restrict__ sc,
+                                                                 const uint32_t* __restrict__ idx, size_t count) {
+    const Lane6 L = lane6_of_thread();
+    const int warp = threadIdx.x >> 5;
+    const bool active_lane = L.k < 6;
+    const int k = active_lane ? L.k : 0;
+    size_t g = (size_t)blockIdx.x * SIPP_ACCUM_GROUPS + warp * SIPP_GROUPS_PER_WARP + (active_lane ? L.base / 6 : 0);
+    const bool have = active_lane && g < count;
+    if (g >= count) g = count - 1;
+    const size_t i = idx[g];
+    const Fq2 base = load_fq2_words(table + i * 96 + k * 16);
+    Fq2 acc = lane_one(k);
+    coop_pow254(L, base, sc + 4 * i, acc);
+    if (have) store_fq2_words(table + i * 96 + k * 16, acc);
+}
+
 // ------------------------------------------------------------------------------------------------ test hook
 // op: 0 mul, 1 sqr (via mul), 2 inv, 3..5 frobenius, 6 conj, 7 cyclotomic sqr, 8 cyclotomic ^x, 9 final exponentiation
 __global__ void __launch_bounds__(32) k_test_coop_op(int op, const uint32_t* __restrict__ a, const uint32_t* __restrict__ b, uint32_t* __restrict__ out,
@@ -452,6 +471,10 @@ int launch_gt_fold_ragged(const uint32_t* proofs, const RaggedGt* ent, size_t np
     const size_t blocks = (2 * npow + SIPP_ACCUM_GROUPS - 1) / SIPP_ACCUM_GROUPS + (6 * nz + SIPP_ACCUM_THREADS - 1) / SIPP_ACCUM_THREADS;
     if (blocks == 0) return 0;
     k_gt_fold_ragged<<<(unsigned)blocks, SIPP_ACCUM_THREADS, 0, s>>>(proofs, ent, npow, nz, challenges, factors);
+    return (int)cudaGetLastError();
+}
+int launch_gt_msm_pow(uint32_t* table, const uint64_t* sc, const uint32_t* idx, size_t count, cudaStream_t s) {
+    k_gt_msm_pow<<<(unsigned)((count + SIPP_ACCUM_GROUPS - 1) / SIPP_ACCUM_GROUPS), SIPP_ACCUM_THREADS, 0, s>>>(table, sc, idx, count);
     return (int)cudaGetLastError();
 }
 int launch_qlines_batch(const uint32_t* B, size_t npoints, uint32_t* qlines, cudaStream_t s) {

@@ -43,17 +43,6 @@ __device__ __forceinline__ void store_point<Fq>(uint32_t* p, size_t i, const G1A
 template <>
 __device__ __forceinline__ void store_point<Fq2>(uint32_t* p, size_t i, const G2A& v) { store_g2(p, i, v); }
 
-// the segment of point i: the last segment whose first point is <= i (empty segments share their first with the next one)
-__device__ __forceinline__ uint32_t segment_of(const MsmSeg* segs, uint32_t count, uint32_t i) {
-    uint32_t lo = 0, hi = count;  // invariant: segs[lo].first <= i, answer in [lo, hi)
-    while (hi - lo > 1) {
-        const uint32_t mid = (lo + hi) >> 1;
-        if (segs[mid].first <= i) lo = mid;
-        else hi = mid;
-    }
-    return lo;
-}
-
 }  // namespace
 
 template <class F>
@@ -64,7 +53,7 @@ __global__ void __launch_bounds__(128) k_msm_recode(const uint32_t* __restrict__
     constexpr int NC = msm::Group<F>::NC, BITS = msm::Group<F>::BITS;
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const MsmSeg sg = segs[segment_of(segs, count, i)];
+    const MsmSeg sg = segs[msm::segment_of(segs, count, i)];
     uint32_t k[8];  // word by word: the caller's scalars need only be 4-byte aligned (as in k_bls.cu)
 #pragma unroll
     for (int w = 0; w < 8; w++) k[w] = scalars[8 * (size_t)i + w];

@@ -186,4 +186,21 @@ int launch_msm_finish(int group, const void* parts, const MsmSeg* segs, const ui
 int launch_msm_straus(int group, const void* terms, const FoldComp* naf, const MsmSeg* segs, const uint32_t* idx, uint32_t nseg, uint32_t* out,
                       cudaStream_t s);
 
+// batched multi-exponentiations in Fq12 (k_gt_msm.cu, short path k_coop.cu; host driver msm.cu).  Segments are MsmSeg with c = 0 (short
+// path) or c > 0 (Pippenger, unsigned c-bit digits: msm::gt_windows(c) windows of 2^c - 1 buckets).  table: n + more Fq12 slots of 96
+// words (w-basis Montgomery, the layout of k_seg_product); element i is decoded to slot i, a Pippenger segment's result goes to the
+// slot of its first element.  sc: 8 words per element (scalars of the short-path elements).  buckets / first / last / long_parts /
+// parts are Fq12 (96 words each) with the counts of launch_msm_buckets and launch_msm_windows.
+int launch_gt_msm_decode(const uint32_t* elems, const uint32_t* scalars, uint32_t n, const MsmSeg* segs, uint32_t count, uint32_t* table, uint32_t* sc,
+                         uint32_t* keys, uint32_t* vals, uint32_t nbuckets, int* flags, cudaStream_t s);
+int launch_gt_msm_buckets(const uint32_t* keys, const uint32_t* vals, uint32_t entries, uint32_t nbuckets, const uint32_t* table, uint32_t* buckets,
+                          uint32_t* first, uint32_t* last, uint32_t* long_list, uint32_t* long_parts, cudaStream_t s);
+// window partials, then per Pippenger segment idx[q] (q < nseg) its result to its table slot
+int launch_gt_msm_windows(const uint32_t* buckets, const MsmWin* wins, uint32_t nwins, uint32_t* parts, uint32_t nseg, const MsmSeg* segs,
+                          const uint32_t* idx, uint32_t* table, cudaStream_t s);
+// table[idx[g]] <- table[idx[g]]^sc[idx[g]], g < count
+int launch_gt_msm_pow(uint32_t* table, const uint64_t* sc, const uint32_t* idx, size_t count, cudaStream_t s);
+// out[j] (boundary bytes) <- work[j] (table slots), j < count
+int launch_gt_msm_encode(const uint32_t* work, size_t count, uint32_t* out, cudaStream_t s);
+
 }  // namespace sipp

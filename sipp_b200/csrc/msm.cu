@@ -1,5 +1,6 @@
 // msm.cu -- batched multi-scalar multiplications (C ABI: sipp_g1_msm_batch, sipp_g2_msm_batch and their _device forms; test hook
-// sipp_test_msm_plan).  Kernels: k_msm.cu; recoding and bucket arithmetic: msm.cuh.
+// sipp_test_msm_plan) and batched multi-exponentiations in Fq12 (sipp_gt_msm_batch and its _device form; test hook
+// sipp_test_gt_msm_plan).  Kernels: k_msm.cu, k_gt_msm.cu; recoding and bucket arithmetic: msm.cuh.
 //
 // `count` independent MSMs of unequal lengths in one call: out[j] = sum_{offsets[j] <= i < offsets[j+1]} [k_i] P_i.  Every segment is
 // planned on the host from its length alone:
@@ -7,11 +8,16 @@
 //   Pippenger  (from there on): signed c-bit windows, c from the cost model msm_window_bits; the buckets of all
 //              Pippenger segments are filled by one sort of (bucket, term) entries
 // Empty segments take the Straus path with no terms and give the identity.
+//
+// The GT multi-exponentiation (group 3 below) is planned the same way: out[j] = prod g_i^(k_i) in Fq12, each segment either on the short
+// path (len < SIPP_GT_MSM_SHORT_BELOW: one generic power per element, k_gt_msm_pow, then k_seg_product) or on Pippenger with unsigned
+// c-bit windows (k_gt_msm.cu), whose results join the segmented product as one factor each.
 #include <string.h>
 
 #include <vector>
 
 #include "host_state.h"
+#include "products.h"
 
 using namespace sipp;
 using namespace sipp_host;
@@ -23,25 +29,37 @@ using namespace sipp_host;
 #define SIPP_MSM_MIN_C 5
 #define SIPP_MSM_MAX_C 16
 #define SIPP_MSM_BUCKETS_PER_THREAD 8  // k_msm_windows: running sums of at most 8 buckets per thread, 64 threads per block
+// GT segments shorter than this take the short path: where the two paths, both forced (sipp_test_gt_msm_batch_device), cross for batches
+// of many segments on one B200 (tools/gt_msm_time.py, DESIGN §7: 4,096 x 256 elements, short path faster; 2,048 x 512, Pippenger
+// faster).  One segment alone crosses later, between 2^12 and 2^14 elements.
+#define SIPP_GT_MSM_SHORT_BELOW 512
+#define SIPP_GT_MSM_MIN_C 2
 
 namespace {
 
+// group 1 = G1, 2 = G2, 3 = GT (the multi-exponentiation in Fq12)
 struct GroupInfo {
-    int nc, bits, words;  // sub-scalars per scalar, bound of a sub-scalar, u32 words of an affine point
+    int nc, bits, words;  // sub-scalars per scalar, bound of a sub-scalar, u32 words of an input element
+    bool gt;              // unsigned digits: ceil(bits / c) windows of 2^c - 1 buckets (signed: bits / c + 1 windows of 2^(c-1))
 };
-GroupInfo group_info(int group) { return group == 1 ? GroupInfo{2, 128, 16} : GroupInfo{4, 66, 32}; }
+GroupInfo group_info(int group) { return group == 1 ? GroupInfo{2, 128, 16, false} : group == 2 ? GroupInfo{4, 66, 32, false} : GroupInfo{1, 254, 96, true}; }
 
-int windows_of(int bits, int c) { return bits / c + 1; }
+int windows_of(const GroupInfo& g, int c) { return g.gt ? (g.bits + c - 1) / c : g.bits / c + 1; }
+size_t buckets_of(const GroupInfo& g, int c) { return g.gt ? ((size_t)1 << c) - 1 : (size_t)1 << (c - 1); }
 
-// the window size of a Pippenger segment: the c minimising W (NC len + 3 2^(c-1)) -- one mixed addition per term and window to fill
-// the buckets, two Jacobian additions (about 1.5 mixed ones each) per bucket to reduce them
+// the window size of a Pippenger segment.  G1 / G2: the c minimising W (NC len + 3 2^(c-1)) -- one mixed addition per term and window
+// to fill the buckets, two Jacobian additions (about 1.5 mixed ones each) per bucket to reduce them.  GT: W (len + 2 2^c) + c W Fq12
+// products -- one per element and window, two per bucket, c squarings per window.
 int msm_window_bits(int group, size_t len) {
     const GroupInfo g = group_info(group);
-    int best = SIPP_MSM_MIN_C;
+    const int lo = g.gt ? SIPP_GT_MSM_MIN_C : SIPP_MSM_MIN_C;
+    int best = lo;
     double best_cost = 0;
-    for (int c = SIPP_MSM_MIN_C; c <= SIPP_MSM_MAX_C; c++) {
-        const double cost = windows_of(g.bits, c) * ((double)g.nc * (double)len + 3.0 * (double)(1u << (c - 1)));
-        if (c == SIPP_MSM_MIN_C || cost < best_cost) {
+    for (int c = lo; c <= SIPP_MSM_MAX_C; c++) {
+        const double W = windows_of(g, c);
+        const double cost = g.gt ? W * ((double)len + 2.0 * (double)(1u << c)) + c * W
+                                 : W * ((double)g.nc * (double)len + 3.0 * (double)(1u << (c - 1)));
+        if (c == lo || cost < best_cost) {
             best_cost = cost;
             best = c;
         }
@@ -49,9 +67,9 @@ int msm_window_bits(int group, size_t len) {
     return best;
 }
 
-// 0: Straus, else the window bits of the Pippenger path
+// 0: Straus (the short path in GT), else the window bits of the Pippenger path
 int msm_segment_c(int group, size_t len) {
-    const size_t below = group == 1 ? SIPP_MSM_STRAUS_BELOW_G1 : SIPP_MSM_STRAUS_BELOW_G2;
+    const size_t below = group == 1 ? SIPP_MSM_STRAUS_BELOW_G1 : group == 2 ? SIPP_MSM_STRAUS_BELOW_G2 : SIPP_GT_MSM_SHORT_BELOW;
     return len < below ? 0 : msm_window_bits(group, len);
 }
 
@@ -84,7 +102,7 @@ int msm_plan(int group, const size_t* offsets, size_t count, MsmPlan& p, int for
             continue;
         }
         pipp.push_back((uint32_t)j);
-        const size_t W = (size_t)windows_of(g.bits, (int)s.c), nb = (size_t)1 << (s.c - 1);
+        const size_t W = (size_t)windows_of(g, (int)s.c), nb = buckets_of(g, (int)s.c);
         const size_t span = (size_t)64 * SIPP_MSM_BUCKETS_PER_THREAD;
         s.parts = (uint32_t)((nb + span - 1) / span);
         s.ebase = (uint32_t)p.entries;
@@ -280,6 +298,156 @@ int msm_device(int group, const void* d_points, const void* d_scalars, size_t n,
     return msm_run(group, (const uint32_t*)d_points, (const uint32_t*)d_scalars, n, offsets, count, d_out, cudaMemcpyDeviceToDevice, force_c);
 }
 
+// the GT multi-exponentiation on the device: elems / scalars hold the boundary bytes (the caller's buffers or staging copies); the
+// results (boundary bytes) are copied to `out` (host or device memory, per out_kind) only when every input passed its checks
+int gt_msm_run(const uint32_t* elems, const uint32_t* scalars, size_t n, const size_t* offsets, size_t count, void* out, cudaMemcpyKind out_kind,
+               int force_c = -1) {
+    cudaStream_t s = g_stream;
+    MsmPlan plan;
+    int rc = msm_plan(3, offsets, count, plan, force_c);
+    if (rc) return rc;
+    // the segmented product over the table slots: a short-path segment multiplies its powered elements, a Pippenger segment its one
+    // result (k_gt_msm_finish writes it to the slot of its first element), an empty segment gives 1
+    std::vector<size_t> start(count), len(count);
+    std::vector<uint32_t> pow_idx;
+    pow_idx.reserve(plan.straus_terms);
+    for (size_t j = 0; j < count; j++) {
+        const MsmSeg& sg = plan.segs[j];
+        start[j] = sg.first;
+        len[j] = sg.c ? 1 : sg.len;
+        if (sg.c == 0)
+            for (uint32_t i = 0; i < sg.len; i++) pow_idx.push_back(sg.first + i);
+    }
+    std::vector<ProductTask> tasks;
+    std::vector<size_t> pass_first;
+    const size_t seg0 = seg_product_tasks(start, len, n, tasks, pass_first);
+    const size_t entries = plan.entries, npipp = count - plan.nstraus, fq12 = 384;
+    size_t sort_bytes = 0;
+    if (entries) {
+        const int le = msm_sort(nullptr, &sort_bytes, nullptr, nullptr, nullptr, nullptr, (uint32_t)entries, plan.key_bits, s);
+        if (le) return cuda_fail((cudaError_t)le, "gt_msm_batch: sort scratch");
+    }
+    std::vector<void*> blocks;
+    struct Release {
+        std::vector<void*>& p;
+        ~Release() { for (void* q : p) pool_free(q); }  // recycled blocks: later work on the same stream only
+    } release{blocks};
+    cudaError_t e = cudaSuccess;
+    auto get = [&](void** ptr, size_t bytes) {
+        *ptr = nullptr;
+        if (e == cudaSuccess && bytes) {
+            e = pool_alloc(ptr, bytes);
+            if (e == cudaSuccess) blocks.push_back(*ptr);
+        }
+    };
+    const size_t chunks = (entries + SIPP_MSM_CHUNK - 1) / SIPP_MSM_CHUNK, lwords = entries ? msm_long_list_words((uint32_t)entries) : 0;
+    uint32_t *table, *sc, *keys, *vals, *keys2, *vals2, *buckets, *first, *last, *long_list, *long_parts, *parts, *enc, *idx, *dpow;
+    void* temp;
+    MsmSeg* dsegs;
+    MsmWin* dwins;
+    ProductTask* dtasks;
+    int* flags;
+    get((void**)&table, (seg0 + count) * fq12);
+    get((void**)&sc, pow_idx.size() ? n * 32 : 0);
+    get((void**)&keys, entries * 4);
+    get((void**)&vals, entries * 4);
+    get((void**)&keys2, entries * 4);
+    get((void**)&vals2, entries * 4);
+    get(&temp, sort_bytes);
+    get((void**)&buckets, plan.nbuckets * fq12);
+    get((void**)&first, chunks * fq12);
+    get((void**)&last, chunks * fq12);
+    get((void**)&long_list, lwords * 4);
+    get((void**)&long_parts, lwords ? (lwords - 1) * SIPP_MSM_LONG_PARTS * fq12 : 0);
+    get((void**)&parts, plan.wins.size() * fq12);
+    get((void**)&enc, count * fq12);
+    get((void**)&dsegs, count * sizeof(MsmSeg));
+    get((void**)&dwins, plan.wins.size() * sizeof(MsmWin));
+    get((void**)&idx, count * sizeof(uint32_t));
+    get((void**)&dpow, pow_idx.size() * sizeof(uint32_t));
+    get((void**)&dtasks, tasks.size() * sizeof(ProductTask));
+    get((void**)&flags, sizeof(int));
+    if (e != cudaSuccess) return cuda_fail(e, "cudaMalloc(gt_msm_batch)");
+    auto run = [&]() -> int {
+        CK(cudaMemsetAsync(flags, 0, sizeof(int), s));
+        CK(cudaMemcpyAsync(dsegs, plan.segs.data(), count * sizeof(MsmSeg), cudaMemcpyHostToDevice, s));
+        CK(cudaMemcpyAsync(idx, plan.idx.data(), count * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
+        CK(cudaMemcpyAsync(dtasks, tasks.data(), tasks.size() * sizeof(ProductTask), cudaMemcpyHostToDevice, s));
+        if (!plan.wins.empty()) CK(cudaMemcpyAsync(dwins, plan.wins.data(), plan.wins.size() * sizeof(MsmWin), cudaMemcpyHostToDevice, s));
+        if (!pow_idx.empty()) CK(cudaMemcpyAsync(dpow, pow_idx.data(), pow_idx.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
+        int le = 0;
+        if (n) {
+            le = launch_gt_msm_decode(elems, scalars, (uint32_t)n, dsegs, (uint32_t)count, table, sc, keys, vals, (uint32_t)plan.nbuckets, flags, s);
+            if (le) return cuda_fail((cudaError_t)le, "k_gt_msm_decode");
+            g_stats.launches++;
+        }
+        if (entries) {
+            le = msm_sort(temp, &sort_bytes, keys, keys2, vals, vals2, (uint32_t)entries, plan.key_bits, s);
+            if (le) return cuda_fail((cudaError_t)le, "gt_msm_batch: sort");
+            le = launch_gt_msm_buckets(keys2, vals2, (uint32_t)entries, (uint32_t)plan.nbuckets, table, buckets, first, last, long_list, long_parts, s);
+            if (!le) le = launch_gt_msm_windows(buckets, dwins, (uint32_t)plan.wins.size(), parts, (uint32_t)npipp, dsegs, idx + plan.nstraus, table, s);
+            if (le) return cuda_fail((cudaError_t)le, "k_gt_msm_buckets / k_gt_msm_windows / k_gt_msm_finish");
+            g_stats.launches += 8;
+        }
+        if (!pow_idx.empty()) {
+            le = launch_gt_msm_pow(table, (const uint64_t*)sc, dpow, pow_idx.size(), s);
+            if (le) return cuda_fail((cudaError_t)le, "k_gt_msm_pow");
+            g_stats.launches++;
+        }
+        for (size_t k = 0; k + 1 < pass_first.size(); k++) {
+            le = launch_seg_product(dtasks + pass_first[k], pass_first[k + 1] - pass_first[k], table, s);
+            if (le) return cuda_fail((cudaError_t)le, "k_seg_product");
+            g_stats.launches++;
+        }
+        int flag = 0;
+        CK(cudaMemcpyAsync(&flag, flags, sizeof(int), cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        // the precedence of the host forms: a scalar >= r first, then a coordinate >= p
+        if (flag & 8) return fail(SIPP_ERR_ENCODING, "scalar >= r");
+        if (flag & 1) return fail(SIPP_ERR_ENCODING, "input coordinate >= p");
+        le = launch_gt_msm_encode(table + seg0 * 96, count, enc, s);
+        if (le) return cuda_fail((cudaError_t)le, "k_gt_msm_encode");
+        g_stats.launches++;
+        CK(cudaMemcpyAsync(out, enc, count * fq12, out_kind, s));
+        CK(cudaStreamSynchronize(s));
+        return SIPP_OK;
+    };
+    rc = run();
+    if (rc) cudaStreamSynchronize(s);
+    return rc;
+}
+
+int gt_msm_host(const uint8_t* elems, const uint8_t* scalars, size_t n, const size_t* offsets, size_t count, uint8_t* out) {
+    int rc = msm_args(elems, scalars, n, offsets, count, out);
+    if (rc || count == 0) return rc ? rc : ensure_init();
+    if (!scalars_canonical(scalars, n)) return fail(SIPP_ERR_ENCODING, "scalar >= r");
+    if (!fq_bytes_canonical(elems, n * 12)) return fail(SIPP_ERR_ENCODING, "input coordinate >= p");
+    rc = ensure_init();
+    if (rc) return rc;
+    uint8_t *te = nullptr, *tk = nullptr;
+    cudaError_t e = pool_alloc((void**)&te, n ? n * 384 : 1);
+    if (e == cudaSuccess) e = pool_alloc((void**)&tk, n ? n * 32 : 1);
+    struct Release {
+        uint8_t *a, *b;
+        ~Release() { pool_free(a); pool_free(b); }
+    } release{te, tk};
+    if (e != cudaSuccess) return cuda_fail(e, "cudaMalloc(gt_msm_batch)");
+    if (n) {
+        CK(cudaMemcpyAsync(te, elems, n * 384, cudaMemcpyHostToDevice, g_stream));
+        CK(cudaMemcpyAsync(tk, scalars, n * 32, cudaMemcpyHostToDevice, g_stream));
+    }
+    return gt_msm_run((const uint32_t*)te, (const uint32_t*)tk, n, offsets, count, out, cudaMemcpyDeviceToHost);  // synchronises
+}
+
+int gt_msm_device(const void* d_elems, const void* d_scalars, size_t n, const size_t* offsets, size_t count, void* d_out, int force_c = -1) {
+    int rc = msm_args(d_elems, d_scalars, n, offsets, count, d_out);
+    if (rc || count == 0) return rc ? rc : ensure_init();
+    rc = ensure_init();
+    if (rc) return rc;
+    CK(order_after(g_stream, cudaStreamLegacy));  // inputs just written on the legacy default stream (torch's, unless switched)
+    return gt_msm_run((const uint32_t*)d_elems, (const uint32_t*)d_scalars, n, offsets, count, d_out, cudaMemcpyDeviceToDevice, force_c);
+}
+
 }  // namespace
 
 extern "C" {
@@ -326,6 +494,38 @@ int sipp_test_msm_batch_device(int group, int c, const void* d_points, const voi
     if (group != 1 && group != 2) return fail(SIPP_ERR_ARG, "group must be 1 or 2");
     if (c != 0 && (c < SIPP_MSM_MIN_C || c > SIPP_MSM_MAX_C)) return fail(SIPP_ERR_ARG, "c must be 0 or 5 .. 16");
     return msm_device(group, d_points, d_scalars, n, offsets, count, d_out, c);
+}
+
+int sipp_gt_msm_batch(const uint8_t* elems, const uint8_t* scalars, size_t n, const size_t* offsets, size_t count, uint8_t* out) {
+    return gt_msm_host(elems, scalars, n, offsets, count, out);
+}
+int sipp_gt_msm_batch_device(const void* d_elems, const void* d_scalars, size_t n, const size_t* offsets, size_t count, void* d_out) {
+    return gt_msm_device(d_elems, d_scalars, n, offsets, count, d_out);
+}
+
+// host-only plan of a GT batch (no GPU needed): 2 words per segment -- path (0 short, 1 Pippenger), window bits (0 for the short path) --
+// to `out` when out_cap >= 2 x count; returns count or a negative status (the offsets checks of the entry points)
+long sipp_test_gt_msm_plan(const size_t* offsets, size_t count, int* out, size_t out_cap) {
+    if (!offsets) return fail(SIPP_ERR_ARG, "null offsets");
+    if (count == 0) return 0;
+    int rc = msm_offsets_args(offsets[count], offsets, count);
+    if (rc) return rc;
+    if (out && out_cap >= 2 * count) {
+        for (size_t j = 0; j < count; j++) {
+            const int c = msm_segment_c(3, offsets[j + 1] - offsets[j]);
+            out[2 * j] = c ? 1 : 0;
+            out[2 * j + 1] = c;
+        }
+    }
+    return (long)count;
+}
+
+// sipp_gt_msm_batch_device with every non-empty segment forced onto one path: c = 0 the short path, SIPP_GT_MSM_MIN_C <= c <=
+// SIPP_MSM_MAX_C Pippenger with c-bit windows (any other c: SIPP_ERR_ARG, before the checks of the device form).  Same outputs as the
+// plan's path; for timing both paths at the same segment length.
+int sipp_test_gt_msm_batch_device(int c, const void* d_elems, const void* d_scalars, size_t n, const size_t* offsets, size_t count, void* d_out) {
+    if (c != 0 && (c < SIPP_GT_MSM_MIN_C || c > SIPP_MSM_MAX_C)) return fail(SIPP_ERR_ARG, "c must be 0 or 2 .. 16");
+    return gt_msm_device(d_elems, d_scalars, n, offsets, count, d_out, c);
 }
 
 }  // extern "C"

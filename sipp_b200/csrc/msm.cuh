@@ -83,6 +83,17 @@ SIPP_HD void signed_digits(const uint64_t mag[3], int bits, int c, Emit emit) {
     }
 }
 
+// GT (k_gt_msm.cu): unsigned c-bit digits of a scalar < r < 2^254, no split -- ceil(254 / c) windows of 2^c - 1 buckets (digit d > 0 in
+// bucket d - 1).  Fq12 has no cheap inverse, and the multi-exponentiation is defined for every Fq12, not only for GT.
+SIPP_HD int gt_windows(int c) { return (254 + c - 1) / c; }
+// bits [pos, pos + c) of a 256-bit little-endian scalar (c <= 16)
+SIPP_HD uint32_t scalar_digit(const uint32_t k[8], int pos, int c) {
+    const int w = pos >> 5, s = pos & 31;
+    uint64_t v = k[w] >> s;
+    if (w + 1 < 8) v |= (uint64_t)k[w + 1] << (32 - s);
+    return (uint32_t)(v & ((1ull << c) - 1));
+}
+
 // the term table entry of sub-scalar j: (-1)^neg endo^j(P)
 template <class F>
 SIPP_HD Affine<F> term_point(const Affine<F>& p, int j, int neg) {
@@ -114,46 +125,16 @@ SIPP_HD uint32_t lower_bound(const uint32_t* keys, uint32_t n, uint32_t key) {
     return lo;
 }
 
-// Bucket sums from the sorted entries in chunks of `ch` entries, so that no thread walks a whole bucket (the buckets of a window
-// are far from even: the top window of a short sub-scalar uses few of them).  Chunk k sums every run of equal keys inside
-// [k ch, (k + 1) ch): a run that is a whole bucket goes to buckets[key]; otherwise its first run goes to first[k] and its last run to
-// last[k] (one run spanning the chunk is both).  Keys >= nbuckets (zero digits) are skipped.
-template <class F>
-SIPP_HD void chunk_sums(const uint32_t* keys, const uint32_t* vals, uint32_t entries, uint32_t nbuckets, uint32_t k, uint32_t ch,
-                        const Affine<F>* terms, Jac<F>* buckets, Jac<F>* first, Jac<F>* last) {
-    const uint32_t s = k * ch, e = s + ch < entries ? s + ch : entries;
-    uint32_t r = s;
-    while (r < e) {
-        const uint32_t key = keys[r];
-        uint32_t q = r;
-        while (q < e && keys[q] == key) q++;
-        if (key >= nbuckets) break;  // the zero-digit entries sort last
-        const Jac<F> acc = bucket_sum(terms, vals + r, q - r);
-        const bool whole = (r == 0 || keys[r - 1] != key) && (q == entries || keys[q] != key);
-        if (whole) {
-            buckets[key] = acc;
-        } else {
-            if (r == s) first[k] = acc;
-            if (q == e) last[k] = acc;
-        }
-        r = q;
+// the segment of item i: the last segment whose first item is <= i (empty segments share their first with the next one)
+template <class Seg>
+SIPP_HD uint32_t segment_of(const Seg* segs, uint32_t count, uint32_t i) {
+    uint32_t lo = 0, hi = count;  // invariant: segs[lo].first <= i, answer in [lo, hi)
+    while (hi - lo > 1) {
+        const uint32_t mid = (lo + hi) >> 1;
+        if (segs[mid].first <= i) lo = mid;
+        else hi = mid;
     }
-}
-
-// bucket b when its run [lo, hi) crosses chunks: the last run of its first chunk, the whole chunks between, the first run of its last
-// chunk (buckets inside one chunk were written by chunk_sums, empty ones stay the identity).  Returns false, writing nothing, when the
-// run crosses more than max_span chunks: the caller sums those partials in parallel (k_msm_long_buckets), in any order.
-template <class F>
-SIPP_HD bool bucket_combine(const uint32_t* keys, uint32_t entries, uint32_t b, uint32_t ch, uint32_t max_span, const Jac<F>* first,
-                            const Jac<F>* last, Jac<F>* buckets) {
-    const uint32_t lo = lower_bound(keys, entries, b), hi = lower_bound(keys, entries, b + 1);
-    if (hi == lo || lo / ch == (hi - 1) / ch) return true;
-    const uint32_t kl = lo / ch, kh = (hi - 1) / ch;
-    if (kh - kl > max_span) return false;
-    Jac<F> acc = last[kl];
-    for (uint32_t k = kl + 1; k <= kh; k++) acc = jac_add(acc, first[k]);
-    buckets[b] = acc;
-    return true;
+    return lo;
 }
 
 // [v] P for a small non-negative integer v (Jacobian P), MSB first
@@ -167,15 +148,84 @@ SIPP_HD Jac<F> jac_mul_small(const Jac<F>& p, uint32_t v) {
     return acc;
 }
 
+// The bucket runs and window sums below are written once over a group in an Ops type: T (a bucket or partial), In (a table entry),
+// identity(), add(a, b), run(terms, vals, count) (the sum of a run of >= 1 sorted entries) and mul_small(p, v) ([v] p).  JacOps is G1 /
+// G2 in Jacobian coordinates; the GT multi-exponentiation (k_gt_msm.cu) writes the same logic multiplicatively over Fq12.
+template <class F>
+struct JacOps {
+    using T = Jac<F>;
+    using In = Affine<F>;
+    static SIPP_HD T identity() { return jac_identity<F>(); }
+    static SIPP_HD T add(const T& a, const T& b) { return jac_add(a, b); }
+    static SIPP_HD T run(const In* terms, const uint32_t* vals, size_t count) { return bucket_sum(terms, vals, count); }
+    static SIPP_HD T mul_small(const T& p, uint32_t v) { return jac_mul_small(p, v); }
+};
+
+// Bucket sums from the sorted entries in chunks of `ch` entries, so that no thread walks a whole bucket (the buckets of a window
+// are far from even: the top window of a short sub-scalar uses few of them).  Chunk k sums every run of equal keys inside
+// [k ch, (k + 1) ch): a run that is a whole bucket goes to buckets[key]; otherwise its first run goes to first[k] and its last run to
+// last[k] (one run spanning the chunk is both).  Keys >= nbuckets (zero digits) are skipped.
+template <class Ops>
+SIPP_HD void chunk_sums_of(const uint32_t* keys, const uint32_t* vals, uint32_t entries, uint32_t nbuckets, uint32_t k, uint32_t ch,
+                           const typename Ops::In* terms, typename Ops::T* buckets, typename Ops::T* first, typename Ops::T* last) {
+    const uint32_t s = k * ch, e = s + ch < entries ? s + ch : entries;
+    uint32_t r = s;
+    while (r < e) {
+        const uint32_t key = keys[r];
+        uint32_t q = r;
+        while (q < e && keys[q] == key) q++;
+        if (key >= nbuckets) break;  // the zero-digit entries sort last
+        const typename Ops::T acc = Ops::run(terms, vals + r, q - r);
+        const bool whole = (r == 0 || keys[r - 1] != key) && (q == entries || keys[q] != key);
+        if (whole) {
+            buckets[key] = acc;
+        } else {
+            if (r == s) first[k] = acc;
+            if (q == e) last[k] = acc;
+        }
+        r = q;
+    }
+}
+template <class F>
+SIPP_HD void chunk_sums(const uint32_t* keys, const uint32_t* vals, uint32_t entries, uint32_t nbuckets, uint32_t k, uint32_t ch,
+                        const Affine<F>* terms, Jac<F>* buckets, Jac<F>* first, Jac<F>* last) {
+    chunk_sums_of<JacOps<F>>(keys, vals, entries, nbuckets, k, ch, terms, buckets, first, last);
+}
+
+// bucket b when its run [lo, hi) crosses chunks: the last run of its first chunk, the whole chunks between, the first run of its last
+// chunk (buckets inside one chunk were written by chunk_sums, empty ones stay the identity).  Returns false, writing nothing, when the
+// run crosses more than max_span chunks: the caller sums those partials in parallel (k_msm_long_buckets), in any order.
+template <class Ops>
+SIPP_HD bool bucket_combine_of(const uint32_t* keys, uint32_t entries, uint32_t b, uint32_t ch, uint32_t max_span, const typename Ops::T* first,
+                               const typename Ops::T* last, typename Ops::T* buckets) {
+    const uint32_t lo = lower_bound(keys, entries, b), hi = lower_bound(keys, entries, b + 1);
+    if (hi == lo || lo / ch == (hi - 1) / ch) return true;
+    const uint32_t kl = lo / ch, kh = (hi - 1) / ch;
+    if (kh - kl > max_span) return false;
+    typename Ops::T acc = last[kl];
+    for (uint32_t k = kl + 1; k <= kh; k++) acc = Ops::add(acc, first[k]);
+    buckets[b] = acc;
+    return true;
+}
+template <class F>
+SIPP_HD bool bucket_combine(const uint32_t* keys, uint32_t entries, uint32_t b, uint32_t ch, uint32_t max_span, const Jac<F>* first,
+                            const Jac<F>* last, Jac<F>* buckets) {
+    return bucket_combine_of<JacOps<F>>(keys, entries, b, ch, max_span, first, last, buckets);
+}
+
 // sum_{lo <= b < hi} (b + 1) S_b of one window's buckets (running sums from the top, then lo times the plain sum)
+template <class Ops>
+SIPP_HD typename Ops::T window_part_of(const typename Ops::T* buckets, uint32_t lo, uint32_t hi) {
+    typename Ops::T run = Ops::identity(), acc = Ops::identity();
+    for (uint32_t b = hi; b > lo; b--) {
+        run = Ops::add(run, buckets[b - 1]);
+        acc = Ops::add(acc, run);
+    }
+    return lo ? Ops::add(acc, Ops::mul_small(run, lo)) : acc;
+}
 template <class F>
 SIPP_HD Jac<F> window_part(const Jac<F>* buckets, uint32_t lo, uint32_t hi) {
-    Jac<F> run = jac_identity<F>(), acc = jac_identity<F>();
-    for (uint32_t b = hi; b > lo; b--) {
-        run = jac_add(run, buckets[b - 1]);
-        acc = jac_add(acc, run);
-    }
-    return lo ? jac_add(acc, jac_mul_small(run, lo)) : acc;
+    return window_part_of<JacOps<F>>(buckets, lo, hi);
 }
 
 // sum_w 2^(c w) wins[w], Horner from the top window

@@ -108,23 +108,12 @@ int products_launch(const uint32_t* dA, const uint32_t* dB, size_t n, size_t cou
     return SIPP_OK;
 }
 
-}  // namespace sipp_host
-
-namespace {
-
-// passes of k_seg_product over the work array [group partials | intermediate runs | one product per segment]; p.seg0 = the slot
-// of segment 0's product (the `count` products are consecutive)
-void product_tasks(ProductPlan& p, size_t count) {
-    std::vector<ProductTask>& tasks = p.tasks;
-    std::vector<size_t>& pass_first = p.pass_first;
-    std::vector<size_t> start(count), len(count);
+size_t seg_product_tasks(std::vector<size_t> start, std::vector<size_t> len, size_t next, std::vector<ProductTask>& tasks,
+                         std::vector<size_t>& pass_first) {
+    const size_t count = start.size();
     size_t longest = 0;
-    for (size_t j = 0; j < count; j++) {
-        start[j] = p.seg_first_group[j];
-        len[j] = p.seg_first_group[j + 1] - start[j];
+    for (size_t j = 0; j < count; j++)
         if (len[j] > longest) longest = len[j];
-    }
-    size_t next = p.groups.size();
     tasks.clear();
     pass_first.clear();
     // segments longer than one task shrink SIPP_PRODUCT_SPAN-fold per pass; the others wait where they are
@@ -148,7 +137,22 @@ void product_tasks(ProductPlan& p, size_t count) {
     pass_first.push_back(tasks.size());
     for (size_t j = 0; j < count; j++) tasks.push_back(ProductTask{(uint32_t)start[j], (uint32_t)len[j], (uint32_t)(next + j), 0});
     pass_first.push_back(tasks.size());
-    p.seg0 = next;
+    return next;
+}
+
+}  // namespace sipp_host
+
+namespace {
+
+// passes of k_seg_product over the work array [group partials | intermediate runs | one product per segment]; p.seg0 = the slot
+// of segment 0's product (the `count` products are consecutive)
+void product_tasks(ProductPlan& p, size_t count) {
+    std::vector<size_t> start(count), len(count);
+    for (size_t j = 0; j < count; j++) {
+        start[j] = p.seg_first_group[j];
+        len[j] = p.seg_first_group[j + 1] - start[j];
+    }
+    p.seg0 = seg_product_tasks(start, len, p.groups.size(), p.tasks, p.pass_first);
 }
 
 int products_args(const void* A, size_t a_len, const void* B, size_t b_len, const size_t* offsets, size_t count, const void* out) {

@@ -33,5 +33,9 @@ int product_plan(const size_t* offsets, size_t count, int kpg_max, size_t chunk_
 // Fq12; the line table must already hold min(n, plan.chunk_pairs) pairs.  Enqueues on s.
 int products_launch(const uint32_t* dA, const uint32_t* dB, size_t n, size_t count, const ProductPlan& plan, const sipp::ProductGroup* dgroups,
                     const sipp::ProductTask* dtasks, uint32_t* work, uint32_t* res, cudaStream_t s);
+// k_seg_product passes multiplying segment j = work slots [start[j], start[j] + len[j]) into slot seg0 + j (returned), an empty one
+// into 1; intermediate runs take the slots from `next` on (the products follow them).  Pass k is tasks [pass_first[k], pass_first[k + 1]).
+size_t seg_product_tasks(std::vector<size_t> start, std::vector<size_t> len, size_t next, std::vector<sipp::ProductTask>& tasks,
+                         std::vector<size_t>& pass_first);
 
 }  // namespace sipp_host
